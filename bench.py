@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the B200 migration/filtering hot path (contract: task prompt, SURVEY.md 8d).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference] [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  Default workload = the north-star target (BASELINE.json): Kirchhoff migration of ONE
 65536-trace x 8192-sample radargram (configs[4]), output-trace ranges sharded over the N ranks with the aperture-halo
@@ -20,6 +20,10 @@ radargram.
   cpu_baseline  the reference's own loop (baseline/_ref, kind "reference"; the oracle's reference-cost port when
              baseline/_ref is absent) on a bounded sample, 1 host core
   --impl reference   the reference's CPU implementation on all usable host cores, no GPU involved
+  --dump-outputs DIR after the timed steps, rank 0 writes the output its last timed step returned as DIR/<record>.npy
+             (headline: DIR/<workload>.npy; sub-records under their `records` key), at most DUMP_BYTES in all: an
+             output that does not fit its share is sampled to every row of a fixed, seeded set of output traces
+             (output_sample).  The inputs are seeded, so two builds run with the same arguments compare file by file.
 """
 import argparse
 import json
@@ -36,6 +40,26 @@ sys.path.insert(0, ROOT)
 
 VEL_K = 1.69e8
 VEL_S = 1.68e8
+DUMP_BYTES = 60 * 1000 * 1000     # --dump-outputs: all arrays together, .npy headers included, stay below 64 MB
+
+
+def output_sample(t, budget, seed=0):
+    """float32 / float64 host copy of the output tensor `t` (..., T) in at most `budget` bytes of data: the whole
+    tensor when it fits, else every row at a seeded, sorted choice of the T output traces (the same columns for the
+    same shape and budget in every run)."""
+    import torch
+    if t.dtype not in (torch.float32, torch.float64):
+        t = t.float()
+    T = t.shape[-1]
+    col_bytes = t.numel() // T * t.element_size()
+    if col_bytes * T > budget:
+        k = budget // col_bytes
+        if k < 1:
+            raise ValueError("one output trace of a %s tensor is larger than the %d-byte dump budget"
+                             % (tuple(t.shape), budget))
+        cols = np.sort(np.random.default_rng(seed).choice(T, k, replace=False))
+        t = t.index_select(-1, torch.as_tensor(cols, device=t.device))
+    return t.detach().cpu().numpy()
 
 
 def load_peaks():
@@ -192,6 +216,10 @@ class Workload(object):
 
     def parity(self):
         return None
+
+    def output(self):
+        """The device tensor the last step() returned to its caller (--dump-outputs)."""
+        return self.out
 
     def teardown(self):
         """Drop every tensor so that the next record starts from an empty device."""
@@ -434,6 +462,9 @@ class KirchhoffC5(KirchhoffC2):
             self.x, self.tt, self.dist, VEL_K, False, rank=self.rank, world=self.world,
             gather=True if self.exchange == "broadcast" else 'src', exchange=self.exchange, **kw)
 
+    def output(self):
+        return self.result
+
     def e2e_step(self):
         if self.world == 1:
             return KirchhoffC2.e2e_step(self)
@@ -520,7 +551,10 @@ class StoltC5(Workload):
 
     def step(self):
         from impdar_b200 import migrationlib as ml
-        ml.stolt_device(self.x, 1e-8, 5.0, VEL_S, 10, 10, out=self.out)
+        self.result = ml.stolt_device(self.x, 1e-8, 5.0, VEL_S, 10, 10, out=self.out)
+
+    def output(self):
+        return self.result                             # (2 * (snum // 2), tnum) for a 2-D radargram
 
     def e2e_step(self):
         import impdar_b200
@@ -815,8 +849,9 @@ def usable_processes(bytes_per_process):
 
 def run_reference(args, rank, world):
     """The reference's CPU implementation of the path on the host cores, no GPU involved.  Kirchhoff workloads: the
-    UNMODIFIED reference's migrationKirchhoffLoop from baseline/_ref (`pip install --target` of /root/reference; the
-    module is loaded standalone from there), one process per usable core because the loop is single-threaded numpy.
+    UNMODIFIED reference's migrationKirchhoffLoop from baseline/_ref (`pip install --target` of an ImpDAR checkout by
+    build(); the module is loaded standalone from there), one process per usable core because the loop is
+    single-threaded numpy.
     Each step = every process computes `ref_n` output samples (the loop bounds tnum=1, snum=ref_n the reference itself
     accepts) against an (snum x ref_T_used) float64 input."""
     if rank != 0:
@@ -877,9 +912,10 @@ class Ctx(object):
     pass
 
 
-def measure(wl, ctx, steps, warmup, with_e2e=True, with_cpu=False, with_parity=True, n_e2e=None):
-    """Warm up, time `steps` steps with CUDA events (barrier + synchronize both sides, max over ranks), then e2e, parity
-    and the CPU baseline.  Returns the record (rank 0) or None."""
+def measure(wl, ctx, steps, warmup, with_e2e=True, with_cpu=False, with_parity=True, n_e2e=None, dump_name=None):
+    """Warm up, time `steps` steps with CUDA events (barrier + synchronize both sides, max over ranks), dump the last
+    step's output as `dump_name` (--dump-outputs), then e2e, parity and the CPU baseline.  Returns the record (rank 0)
+    or None."""
     import torch
     import torch.distributed as dist
     rank, world, lib = ctx.rank, ctx.world, ctx.lib
@@ -919,6 +955,8 @@ def measure(wl, ctx, steps, warmup, with_e2e=True, with_cpu=False, with_parity=T
     lib.impdar_b200_kernel_timer(0)   # stop recording; the records stay readable for roofline()
     launches = lib.impdar_b200_launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
+    if ctx.args.dump_outputs and rank == 0:
+        np.save(os.path.join(ctx.args.dump_outputs, dump_name + ".npy"), output_sample(wl.output(), ctx.dump_budget))
     total_ms = sum(a.elapsed_time(b) for a, b in evs)
     t = torch.tensor([total_ms], dtype=torch.float64, device="cuda")
     if world > 1:
@@ -973,6 +1011,21 @@ def measure(wl, ctx, steps, warmup, with_e2e=True, with_cpu=False, with_parity=T
     return rec
 
 
+def sub_records(args, world):
+    """[(records key, Workload class)] measured after the headline, each for args.steps timed steps."""
+    if args.workload != "kirchhoff_c5" or args.no_records:
+        return []
+    subs = [("kirchhoff_4096x2048_per_gpu", KirchhoffC2)]
+    if world == 1:
+        subs.insert(0, ("stolt_65536x8192", StoltC5))
+    return subs
+
+
+def dump_budget(n_records):
+    """Data bytes per --dump-outputs array when the line has `n_records` records (4 KiB of each share for the header)."""
+    return DUMP_BYTES // n_records - 4096
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -987,7 +1040,13 @@ def main():
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--no-records", action="store_true", help="headline only (no Stolt / config-2 sub-records)")
     ap.add_argument("--cpu-samples", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's output of every record as DIR/<name>.npy (see the module doc)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours (the reference arm times bounded samples, not whole outputs)")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -1014,20 +1073,22 @@ def main():
         from impdar_b200 import migrationlib as ml
         ml.set_kirchhoff_mode(int(os.environ["IMPDAR_KIRCH_MODE"]))
 
+    subs = sub_records(args, world)
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+    ctx.dump_budget = dump_budget(1 + len(subs))
+
     wl = WORKLOADS[args.workload](args, rank, world)
     head = measure(wl, ctx, args.steps, args.warmup, with_e2e=not args.no_e2e,
-                   with_cpu=(world == 1 and not args.no_cpu_baseline), with_parity=not args.no_parity)
+                   with_cpu=(world == 1 and not args.no_cpu_baseline), with_parity=not args.no_parity,
+                   dump_name=args.workload)
     records = {}
-    if args.workload == "kirchhoff_c5" and not args.no_records:
-        subs = [("kirchhoff_4096x2048_per_gpu", KirchhoffC2)]
-        if world == 1:
-            subs.insert(0, ("stolt_65536x8192", StoltC5))
-        for key, cls in subs:
-            sub = cls(args, rank, world)
-            r = measure(sub, ctx, min(args.steps, 10), 3, with_e2e=not args.no_e2e, with_cpu=False,
-                        with_parity=not args.no_parity)
-            if rank == 0:
-                records[key] = r
+    for key, cls in subs:
+        sub = cls(args, rank, world)
+        r = measure(sub, ctx, args.steps, 3, with_e2e=not args.no_e2e, with_cpu=False,
+                    with_parity=not args.no_parity, dump_name=key)
+        if rank == 0:
+            records[key] = r
 
     if rank == 0:
         line = {"metric": "migrated samples/s", "value": head["value"], "unit": "samples/s", "n_gpus": world,

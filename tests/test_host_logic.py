@@ -225,16 +225,21 @@ def test_peer_image_and_window_address_arithmetic(monkeypatch):
     assert w.data_ptr() == 1 << 26 and w.shape == (S, 20) and w.stride(0) == 20
 
 
-def test_bench_config_is_the_same_object_for_both_arms():
-    """`bench.py --impl reference` must print the `config` of our arm's line at the same --gpus (the driver compares
-    them): both come from Workload.config(), which depends on the workload and the GPU count only."""
-    import argparse
+def _bench_module():
     import importlib.util
     import os
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     spec = importlib.util.spec_from_file_location("bench_module", os.path.join(root, "bench.py"))
     bench = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(bench)
+    return bench
+
+
+def test_bench_config_is_the_same_object_for_both_arms():
+    """`bench.py --impl reference` must print the `config` of our arm's line at the same --gpus (the driver compares
+    them): both come from Workload.config(), which depends on the workload and the GPU count only."""
+    import argparse
+    bench = _bench_module()
     args = argparse.Namespace(gpus=1, steps=1, warmup=0, profiles=8, workload='kirchhoff_c5', cpu_samples=0)
     for name, cls in bench.WORKLOADS.items():
         for world in (1, 2, 8):
@@ -244,6 +249,90 @@ def test_bench_config_is_the_same_object_for_both_arms():
     c5 = bench.WORKLOADS["kirchhoff_c5"]
     assert c5(args, 0, 1).config()["parallelism"] != c5(args, 0, 8).config()["parallelism"]
     assert "65536" in c5.name and (c5.S, c5.T) == (8192, 65536)
+
+
+def test_bench_output_sample_is_bounded_and_the_same_every_run():
+    """`bench.py --dump-outputs`: an output larger than its byte share keeps every row at a sorted, seeded choice of
+    output traces, the same in every run; an output that fits is written whole; integer outputs become float32."""
+    import torch
+    bench = _bench_module()
+    x = torch.arange(2 * 3 * 1000, dtype=torch.float32).reshape(2, 3, 1000)    # value = row * 1000 + trace
+    s = bench.output_sample(x, 2 * 3 * 100 * 4)
+    assert s.shape == (2, 3, 100) and s.dtype == np.float32
+    cols = s[0, 0].astype(int)
+    assert np.all(np.diff(cols) > 0) and np.array_equal(s, x.numpy()[..., cols])
+    assert np.array_equal(bench.output_sample(x, 2 * 3 * 100 * 4), s)
+    assert np.array_equal(bench.output_sample(x, x.numel() * 4), x.numpy())
+    assert bench.output_sample(x.double(), 10 ** 9).dtype == np.float64
+    assert bench.output_sample(x.int(), 10 ** 9).dtype == np.float32
+    with pytest.raises(ValueError):
+        bench.output_sample(x, 2 * 3 * 4 - 1)
+
+
+def test_bench_dump_of_every_record_line_stays_below_64mb(tmp_path):
+    """The records each line carries and the files --dump-outputs writes for them at the real output shapes (zero-stride
+    stand-ins of the device outputs): together below 64 MB for every record list."""
+    import argparse
+    import os
+    import torch
+    bench = _bench_module()
+    for workload, no_records, world, keys in (("kirchhoff_c5", False, 1, ["stolt_65536x8192", "kirchhoff_4096x2048_per_gpu"]),
+                                              ("kirchhoff_c5", False, 2, ["kirchhoff_4096x2048_per_gpu"]),
+                                              ("kirchhoff_c5", True, 1, []), ("pipeline", False, 1, [])):
+        args = argparse.Namespace(workload=workload, no_records=no_records)
+        subs = bench.sub_records(args, world)
+        assert [k for k, _ in subs] == keys
+        budget = bench.dump_budget(1 + len(subs))
+        total = 0
+        for name, cls in [(workload, bench.WORKLOADS[workload])] + subs:
+            shape = (cls.S, cls.T) if workload != "pipeline" else (8, 2 * (cls.S // 2), cls.T)
+            fn = os.path.join(str(tmp_path), name + ".npy")
+            np.save(fn, bench.output_sample(torch.zeros(()).expand(*shape), budget))
+            total += os.path.getsize(fn)
+        assert total <= 64 * 1000 * 1000, (workload, world, total)
+
+
+@pytest.mark.gpu
+def test_bench_main_dumps_the_last_timed_step_of_every_record(tmp_path, monkeypatch, capsys):
+    """bench.main() with a stand-in workload in every record: the line and every record time --steps steps, and
+    --dump-outputs writes the output of the last timed step (3 warm-up steps + 12 timed ones) under each record's name."""
+    import json
+    import os
+    import torch
+    bench = _bench_module()
+
+    class Stub(bench.Workload):
+        name, S, T = "stub", 64, 48
+
+        def l2_note(self):
+            return "inputs in L2; no flush needed"
+
+        def setup(self):
+            self.x = torch.arange(self.S * self.T, dtype=torch.float32, device="cuda").reshape(self.S, self.T)
+            self.units, self.calls = self.S * self.T, 0
+
+        def step(self):
+            self.calls += 1
+            self.out = self.x * self.calls
+
+        def roofline(self, ms, hbm_gbs, src):
+            return {}
+
+    monkeypatch.setitem(bench.WORKLOADS, "kirchhoff_c5", Stub)
+    monkeypatch.setattr(bench, "StoltC5", Stub)
+    monkeypatch.setattr(bench, "KirchhoffC2", Stub)
+    for k in ("RANK", "LOCAL_RANK", "WORLD_SIZE"):
+        monkeypatch.delenv(k, raising=False)
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--gpus", "1", "--steps", "12", "--warmup", "0", "--no-cpu-baseline",
+                                      "--no-e2e", "--dump-outputs", str(tmp_path)])
+    bench.main()
+    line = json.loads(capsys.readouterr().out.strip().splitlines()[-1])
+    assert line["steps"] == 12 and sorted(line["records"]) == ["kirchhoff_4096x2048_per_gpu", "stolt_65536x8192"]
+    assert all(r["steps"] == 12 for r in line["records"].values())
+    want = np.arange(64 * 48, dtype=np.float32).reshape(64, 48) * 15
+    for name in ("kirchhoff_c5", "stolt_65536x8192", "kirchhoff_4096x2048_per_gpu"):
+        got = np.load(os.path.join(str(tmp_path), name + ".npy"))
+        assert got.dtype == np.float32 and np.array_equal(got, want), name
 
 
 def test_kirchhoff_input_window_covers_the_aperture():
