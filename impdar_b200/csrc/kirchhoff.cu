@@ -34,7 +34,7 @@ struct KirchParams {
     const double *tt;     // S  [s]
     const double *zs;     // S  vel*tt/2
     const double *zs2;    // S  zs^2
-    const int *flags;     // [0] = non-finite input seen
+    const int *flags;     // [0] = 1 + the deepest row of the d/dt (or data) image holding a non-finite value, 0 if none
     unsigned long long *stats;  // [0] pairs, [1] exact pairs
     int S, T, SP, ldo, x_begin, x_end;
     double vel, tmax, tt0, inv_dt, cs;  // cs = 2/(vel*dt_eff)
@@ -311,7 +311,7 @@ __global__ void __launch_bounds__(256) grad_transpose_kernel(const float *__rest
     __shared__ float tg[32][33];
     __shared__ float td[32][33];
     const int s0 = blockIdx.y * 32, x0 = blockIdx.x * 32;
-    bool bad = false;
+    int bad = 0;   // 1 + deepest row with a non-finite value
     for (int r = threadIdx.y; r < 32; r += 8) {
         const int s = s0 + r, x = x0 + threadIdx.x;
         float g = 0.f, dv = 0.f;
@@ -323,7 +323,7 @@ __global__ void __launch_bounds__(256) grad_transpose_kernel(const float *__rest
             if (b != 0.0) acc += b * (double)dv;
             if (s < S - 1 && c != 0.0) acc += c * (double)data[(size_t)(s + 1) * ld + x];
             g = (float)acc;
-            if (!isfinite(g) || !isfinite(dv)) bad = true;
+            if (!isfinite(g) || !isfinite(dv)) bad = s + 1;
         }
         tg[r][threadIdx.x] = g;
         td[r][threadIdx.x] = dv;
@@ -336,7 +336,8 @@ __global__ void __launch_bounds__(256) grad_transpose_kernel(const float *__rest
             if (dataT) dataT[(size_t)x * SP + s] = td[threadIdx.x][r];
         }
     }
-    if (__syncthreads_or(bad) && threadIdx.x == 0 && threadIdx.y == 0) atomicOr(flags, 1);
+    bad = __reduce_max_sync(0xffffffffu, bad);
+    if (bad && threadIdx.x == 0) atomicMax(flags, bad);
 }
 
 __global__ void kirch_prep_vectors_kernel(const double *__restrict__ tt, double *__restrict__ zs,
@@ -371,7 +372,8 @@ struct KirchTabParams {
     unsigned long long *stats;
     int S, T, Tp, Apad, A1, ldo, x_begin, x_end;
     int s_begin, s_end;  // output rows of this launch (the host pipeline runs the image in row chunks)
-    const int *only_if;  // non-null: the launch stands in for the tile kernel and runs only when *only_if or flags[0] is set
+    const int *only_if;  // non-null: the launch stands in for the tile kernel: every row when *only_if is set (wide
+                         // intervals), otherwise only the rows that read non-finite input (ti < flags[0])
 };
 
 __global__ void __launch_bounds__(128) kirch_table_build_kernel(int2 *__restrict__ tab, float *__restrict__ tabn,
@@ -414,7 +416,10 @@ __global__ void __launch_bounds__(128) kirch_table_build_kernel(int2 *__restrict
     if (k == -2) amb_list[atomicAdd(amb_count, 1)] = ti * A1 + m;  // list has room for every entry
 }
 
-// d/dt (np.gradient stencil) into the padded row-major layout; also the non-finite scan.  `data` holds the radargram
+// d/dt (np.gradient stencil) into the padded row-major layout; also the non-finite scan, which records the deepest
+// row of the padded images holding a non-finite value (flags[0] = 1 + row).  An output row ti reads only rows >= ti
+// of those images, so "flags[0] > ti" is known as soon as the rows >= ti are built: a bottom-up sequence of row chunks
+// takes every per-row decision that depends on it exactly as one launch over the whole image does.  `data` holds the radargram
 // columns [c0, c0 + ncols) with row stride ld (the whole image: c0 = 0, ncols = ld = T); trace x lands at column
 // aoff + x of the padded image (aoff = Apad - c0).
 __global__ void __launch_bounds__(256) grad_padded_kernel(const float *__restrict__ data, float *__restrict__ gP,
@@ -449,7 +454,7 @@ __global__ void __launch_bounds__(256) grad_padded_kernel(const float *__restric
             go[j] = make_float4(g[0], g[1], g[2], g[3]);
             if (dout) dout[j] = d0;
         }
-        if (__syncthreads_or(bad) && threadIdx.x == 0) atomicOr(flags, 1);
+        if (__syncthreads_or(bad) && threadIdx.x == 0) atomicMax(flags, s + 1);   // deepest non-finite row
         return;
     }
     for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < ncols; j += gridDim.x * blockDim.x) {
@@ -463,7 +468,7 @@ __global__ void __launch_bounds__(256) grad_padded_kernel(const float *__restric
         gP[(size_t)s * Tp + aoff + c0 + j] = g;
         if (dP) dP[(size_t)s * Tp + aoff + c0 + j] = dv;
     }
-    if (__syncthreads_or(bad) && threadIdx.x == 0) atomicOr(flags, 1);
+    if (__syncthreads_or(bad) && threadIdx.x == 0) atomicMax(flags, s + 1);   // deepest non-finite row
 }
 
 constexpr int KT_R = 4;  // output traces per thread (stride 32)
@@ -531,11 +536,14 @@ __device__ __forceinline__ void kirch_table_loop(const KirchTabParams &p, int ti
 
 template <bool NEAR, bool STATS>
 __global__ void __launch_bounds__(128) kirch_table_kernel(const __grid_constant__ KirchTabParams p) {
-    if (p.only_if && !(p.only_if[0] | p.flags[0])) return;   // the tile kernel has done these rows
+    // Rows ti < nan_end read a non-finite value somewhere (the nansum variant); the tile kernel leaves them to this one.
+    const int nan_end = p.flags[0];
+    const int s_end = (p.only_if && !p.only_if[0]) ? min(p.s_end, nan_end) : p.s_end;
+    if (s_end <= p.s_begin) return;   // the tile kernel has done these rows
     // Work item = (row, block of 4 x 32 KT_R output traces), rows fastest.  The grid holds every item when this kernel
     // is the one that does the work; as the tile kernel's stand-in it is a small grid that strides over the items
     // (half a million CTAs that only test the flag and leave cost 0.5 ms at 65536 x 8192).
-    const int nrows = p.s_end - p.s_begin;
+    const int nrows = s_end - p.s_begin;
     const int ntx = (p.x_end - p.x_begin + 4 * 32 * KT_R - 1) / (4 * 32 * KT_R);
     const long long nitems = (long long)nrows * ntx;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -547,7 +555,7 @@ __global__ void __launch_bounds__(128) kirch_table_kernel(const __grid_constant_
 #pragma unroll
         for (int r = 0; r < KT_R; ++r) acc[r] = 0.f;
         unsigned npairs = 0;
-        if (p.flags[0] != 0)
+        if (ti < nan_end)
             kirch_table_loop<NEAR, true, STATS>(p, ti, xbase, acc, npairs);
         else
             kirch_table_loop<NEAR, false, STATS>(p, ti, xbase, acc, npairs);
@@ -860,7 +868,7 @@ static int kirchhoff_impl(const float *data, float *out, int S, int T, const dou
     unsigned long long *stats = (unsigned long long *)(w + 128);
     w += 256;
     w = (char *)(((uintptr_t)w + 255) & ~(uintptr_t)255);
-    const bool continuing = rows && rows->g_hi < S;   // later call of a bottom-up row sequence: flags, tables, d/dt rows
+    const bool continuing = rows && rows->g_hi < S;   // later call of a bottom-up row sequence: flags, tables, tile schedule, d/dt rows
     if (!continuing) {                                // and the vectors stay (same workspace, same stream)
         // d_tt | d_coef (3 S) | d_dist are contiguous in the workspace: one copy from the page-locked staging slot
         int rcv = kirch_stage_vectors(tt_s, grad_coef, dist_m, S, T, d_tt, st);
@@ -912,13 +920,13 @@ static int kirchhoff_impl(const float *data, float *out, int S, int T, const dou
         w = (char *)(((uintptr_t)w + 255) & ~(uintptr_t)255);
         const bool use_tile = !nearfield && g_kirch_mode != 3;
         const int nchunks = pipe ? pipe->nchunks : 1;
-        const size_t nblk_max = (size_t)(S + KT_Q - 1) / KT_Q + nchunks;
+        const size_t nblk_img = (size_t)(S + KT_Q - 1) / KT_Q;   // tile blocks of the image (schedule kept across row chunks)
         int2 *seg = (int2 *)w;
         int *nstage = nullptr;
         if (use_tile) {
-            w += nblk_max * (size_t)S * sizeof(int2);
+            w += nblk_img * (size_t)S * sizeof(int2);
             nstage = (int *)w;
-            w += nblk_max * sizeof(int);
+            w += nblk_img * sizeof(int);
         }
         IMPDAR_CHECK_ARG((unsigned long long)S * (unsigned long long)A1 < (1ull << 31), "kirchhoff: table too large");
         IMPDAR_CHECK_ARG((size_t)(w - (char *)workspace) <= ws_bytes, "kirchhoff: workspace too small for the table path");
@@ -948,7 +956,6 @@ static int kirchhoff_impl(const float *data, float *out, int S, int T, const dou
         // Row chunks, bottom-up.  Without a host pipeline this is one chunk covering the whole image.
         int g_hi = rows ? rows->g_hi : S;   // d/dt rows [g_hi, S) are built
         int u_hi = S;   // input rows [u_hi, S) are uploaded
-        size_t blk_used = 0;
         for (int j = nchunks - 1; j >= 0; --j) {
             const int r0 = rows ? rows->s_begin : (int)((long long)S * j / nchunks);
             const int r1 = rows ? rows->s_end : (int)((long long)S * (j + 1) / nchunks);
@@ -983,15 +990,21 @@ static int kirchhoff_impl(const float *data, float *out, int S, int T, const dou
                 kirch_table_count_kernel<<<r1 - r0, 256, 0, st>>>(tab, nm, A1, T, x_begin, x_end, r0, stats);
                 IMPDAR_LAUNCH_CHECK();
             }
-            if (use_tile) {
-                const int nblk = (r1 - r0 + KT_Q - 1) / KT_Q;
-                KirchTileParams tq;
-                tq.seg = seg + blk_used * (size_t)S;
-                tq.nstage = nstage + blk_used;
-                tq.sched_flags = sched_flags;
-                blk_used += (size_t)nblk;
-                kirch_tile_sched_kernel<<<nblk, 256, 0, st>>>(tab, nm, S, A1, r0, r1, (int2 *)tq.seg, (int *)tq.nstage, sched_flags);
+            if (use_tile && !continuing && j == nchunks - 1) {
+                // Schedule of every tile block of the image: blocks at absolute multiples of KT_Q rows, so a row chunk
+                // runs its part of the same blocks (clipped; a clipped block's intervals lie inside the full block's).
+                // The stand-down for wide intervals is decided here, once per image (first chunk of the first call),
+                // over all of them: row chunks, the host pipeline and one launch take the same decision.
+                kirch_tile_sched_kernel<<<(S + KT_Q - 1) / KT_Q, 256, 0, st>>>(tab, nm, S, A1, 0, S, seg, nstage, sched_flags);
                 IMPDAR_LAUNCH_CHECK();
+            }
+            if (use_tile) {
+                const int b0 = r0 / KT_Q, nblk = (r1 - 1) / KT_Q - b0 + 1;   // the image's blocks that meet [r0, r1)
+                KirchTileParams tq;
+                tq.seg = seg + (size_t)b0 * S;
+                tq.nstage = nstage + b0;
+                tq.sched_flags = sched_flags;
+                tq.t_base = b0 * KT_Q;
                 dim3 tgrid(nblk, (x_end - x_begin + KT_X - 1) / KT_X);
                 ktimer_begin("kirch_tile_kernel", st);
                 kirch_tile_kernel<<<tgrid, KT_THREADS, KT_SMEM, st>>>(tp, tq);

@@ -14,7 +14,10 @@
 // Summation order per output sample: m ascending, partial sums flushed into a second accumulator after every
 // KT_FLUSH-th stage; stages are windows of KT_W source rows at ABSOLUTE multiples of KT_W (and the flushes at absolute
 // window indices), so the order - and therefore the result, bit for bit - does not depend on how the image is cut
-// into row chunks, trace ranges or CTAs.
+// into row chunks, trace ranges or CTAs.  Nor do the decisions about which rows this kernel does: blocks sit at absolute
+// multiples of KT_Q rows (a row chunk runs the clipped part of the image's blocks), the stand-down for intervals wider
+// than KT_SPAN is taken once per image over all its blocks, and rows that read non-finite input (ti < flags[0], the
+// deepest non-finite row + 1) are left to the gather kernel's nansum variant row by row.
 #pragma once
 
 namespace impdar {
@@ -66,7 +69,8 @@ static_assert(KT_RPP <= 32 && KT_NW + KT_NP <= 32, "tile kernel configuration");
 struct KirchTileParams {
     const int2 *seg;     // [nblocks][S]: {mlo, mhi} per source row (mlo > mhi: not used by the block)
     const int *nstage;   // [nblocks]: stages the block walks (from its first row's absolute window)
-    int *sched_flags;    // [0] != 0: some interval is wider than KT_SPAN -> this kernel stands down (table kernel runs)
+    int *sched_flags;    // [0] != 0: some interval of the image is wider than KT_SPAN -> this kernel stands down (table kernel runs)
+    int t_base;          // first row of block 0: the multiple of KT_Q at or below the launch's first row
 };
 
 __device__ __forceinline__ unsigned kt_smem_u32(const void *p) { return (unsigned)__cvta_generic_to_shared(p); }
@@ -107,7 +111,7 @@ __device__ __forceinline__ void kt_bulk_load(void *smem_dst, const void *gsrc, u
                  : "memory");
 }
 
-// Schedule: for every block of KT_Q output rows of this launch and every source row k, the interval of offsets m with
+// Schedule: for every block of KT_Q output rows of [s_begin, s_end) and every source row k, the interval of offsets m with
 // k(ti, m) == k for some row ti of the block.  One CTA per block; the table rows are walked once (S x A1 entries in all).
 __global__ void __launch_bounds__(256) kirch_tile_sched_kernel(const int2 *__restrict__ tab, const int *__restrict__ nm,
                                                                int S, int A1, int s_begin, int s_end, int2 *__restrict__ seg,
@@ -170,15 +174,18 @@ __global__ void __launch_bounds__(256) kirch_table_count_kernel(const int2 *__re
 __global__ void __launch_bounds__(KT_THREADS, 1) kirch_tile_kernel(const __grid_constant__ KirchTabParams p,
                                                                    const __grid_constant__ KirchTileParams q) {
     extern __shared__ __align__(128) unsigned char kt_smem_raw[];
-    if (q.sched_flags[0] != 0 || p.flags[0] != 0) return;   // wide intervals or non-finite input: the table kernel runs
+    if (q.sched_flags[0] != 0) return;              // wide intervals somewhere in the image: the table kernel runs
+    const int b = blockIdx.x;                       // row block (fast index: concurrent CTAs share the column window in L2)
+    // the image's block at an absolute multiple of KT_Q rows, clipped to this launch's rows [s_begin, s_end)
+    const int t0 = q.t_base + b * KT_Q;
+    const int r_lo = max(t0, p.flags[0]);           // rows ti < flags[0] read non-finite input: the table kernel does them
+    if (min(t0 + KT_Q, p.s_end) <= r_lo) return;
     float *buf = reinterpret_cast<float *>(kt_smem_raw);
     int2 *hdr = reinterpret_cast<int2 *>(buf + (size_t)KT_NST * KT_STAGE_FLOATS);
     int2 *rings = hdr + KT_NST * KT_W;
     unsigned long long *full = reinterpret_cast<unsigned long long *>(rings + KT_NW * KT_RW * KT_RING);
     unsigned long long *empty = full + KT_NST;
 
-    const int b = blockIdx.x;                       // row block (fast index: concurrent CTAs share the column window in L2)
-    const int t0 = p.s_begin + b * KT_Q;
     const int x0 = p.x_begin + blockIdx.y * KT_X;
     const int nst = q.nstage[b];
     const int kbase = (t0 / KT_W) * KT_W;
@@ -244,6 +251,7 @@ __global__ void __launch_bounds__(KT_THREADS, 1) kirch_tile_kernel(const __grid_
     // coalesced load per lane, a chunk ahead of its use, and parked in a warp-private shared-memory ring, so the walk
     // itself never waits on global memory (the L1 left beside 200 KB of staging buffers does not hold 31 table rows).
     int mcur[KT_RW], mend[KT_RW], cready[KT_RW];
+    bool live[KT_RW];                               // the row is this launch's and this kernel's to write
     const int2 *trow[KT_RW];
     int2 pre[KT_RW];
     int2 *ring[KT_RW];
@@ -251,10 +259,10 @@ __global__ void __launch_bounds__(KT_THREADS, 1) kirch_tile_kernel(const __grid_
 #pragma unroll
     for (int w = 0; w < KT_RW; ++w) {
         const int ti = t0 + warp + w * KT_NW;
-        const bool live = ti < p.s_end && (x0 < p.x_end);
+        live[w] = ti >= max(p.s_begin, r_lo) && ti < p.s_end && (x0 < p.x_end);
         mcur[w] = 0;
-        mend[w] = live ? p.nm[ti] : 0;
-        trow[w] = p.tab + (size_t)(live ? ti : t0) * p.A1;
+        mend[w] = live[w] ? p.nm[ti] : 0;
+        trow[w] = p.tab + (size_t)(live[w] ? ti : t0) * p.A1;
         ring[w] = rings + (size_t)(warp * KT_RW + w) * KT_RING;
         ring[w][lane] = lane < mend[w] ? __ldg(trow[w] + lane) : sentinel;              // chunk 0
         pre[w] = 32 + lane < mend[w] ? __ldg(trow[w] + 32 + lane) : sentinel;            // chunk 1, parked when chunk 0 is entered
@@ -317,7 +325,7 @@ __global__ void __launch_bounds__(KT_THREADS, 1) kirch_tile_kernel(const __grid_
 #pragma unroll
     for (int w = 0; w < KT_RW; ++w) {
         const int ti = t0 + warp + w * KT_NW;
-        if (ti >= p.s_end) continue;
+        if (!live[w]) continue;
 #pragma unroll
         for (int r = 0; r < KT_TR / 2; ++r) {
             const float2 v = __fadd2_rn(tot[w][r], acc[w][r]);

@@ -241,8 +241,8 @@ def kirchhoff_last_path():
 
 def kirchhoff_last_kernel():
     """'general', 'table_gather' or 'table_tile' - the kernel that did the far-field sum of the last call ('table_tile'
-    only if the tile kernel really did the work; it stands down for non-finite input and for hyperbola intervals wider
-    than its staged segments).  Synchronises the call's stream."""
+    only if the tile kernel did all of it; it stands down for hyperbola intervals wider than its staged segments, and
+    leaves the rows that read non-finite input to the gather kernel).  Synchronises the call's stream."""
     lib = _lib.load()
     path = lib.impdar_kirchhoff_last_path()
     if path != 3:

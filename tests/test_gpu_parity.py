@@ -74,10 +74,14 @@ def test_kirchhoff_vs_oracle(S, T, tt0, nearfield, mode):
 def test_kirchhoff_host_pipeline_equals_device_path(S, T, nearfield, nchunks, mode):
     """The host-to-host entry (row chunks processed bottom-up with upload / kernels / download overlapped) returns
     bit for bit what the device-resident call returns: the chunking only reorders independent output rows.  The
-    input carries NaNs in its upper rows only, so no chunk is affected by the nansum variant switch."""
+    input carries NaNs in a few rows of its top chunk, which the bottom chunks (processed first) never read: the nansum
+    variant and the tile kernel's stand-down are decided per output row from the deepest non-finite input row, so the
+    chunks that run before the NaN rows are seen decide as the one-launch call does."""
     from impdar_b200 import migrationlib as ml
     import torch
     d = synthetic_dat(S, T, seed=7 * S + T, tt0_us=0.0 if not nearfield else 0.11)
+    top = S // nchunks
+    d.data[sorted({1, max(1, top // 2), top - 1}), T // 3:T // 3 + 5] = np.nan
     if mode == "general":
         d.dist = np.cumsum(0.004 + 0.002 * np.random.default_rng(1).random(T))      # irregular spacing
     ml.set_kirchhoff_mode(ml.KIRCHHOFF_GENERAL if mode == "general" else ml.KIRCHHOFF_AUTO)
@@ -91,6 +95,7 @@ def test_kirchhoff_host_pipeline_equals_device_path(S, T, nearfield, nchunks, mo
     finally:
         ml.set_kirchhoff_mode(ml.KIRCHHOFF_AUTO)
     assert got.dtype == np.float64 and got.shape == (S, T)
+    assert np.isfinite(want).all()           # nansum: the NaN terms are skipped
     assert np.array_equal(got, want) and np.array_equal(got_pinned, want)
 
 
