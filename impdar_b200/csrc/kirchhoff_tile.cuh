@@ -59,9 +59,10 @@ constexpr int KT_FLUSH = KT_CFG_FLUSH;           // stages (absolute index) betw
 constexpr int KT_SPAN = 120;         // widest [mlo, mhi] interval the staged segments hold
 constexpr int KT_SEGW = KT_X + KT_SPAN + 8;                   // floats per staged segment (alignment shift <= 3)
 constexpr int KT_STAGE_FLOATS = KT_W * 2 * KT_SEGW;
-constexpr int KT_RING = 64;           // table entries per (warp, row) ring: two chunks of 32
-constexpr size_t KT_SMEM = (size_t)KT_NST * KT_STAGE_FLOATS * sizeof(float) + KT_NST * KT_W * sizeof(int2) +
-                           (size_t)KT_NW * KT_RW * KT_RING * sizeof(int2) + 2 * KT_NST * sizeof(unsigned long long) + 16;
+constexpr int KT_RING = 33;           // decoded entries per (warp, row) ring: one chunk of 32, plus the slot that the
+                                      // walk's one-ahead read touches after the chunk's last entry
+constexpr size_t KT_SMEM = (size_t)KT_NST * KT_STAGE_FLOATS * sizeof(float) +
+                           (size_t)KT_NW * KT_RW * KT_RING * sizeof(int4) + 2 * KT_NST * sizeof(unsigned long long) + 16;
 constexpr int KT_THREADS = (KT_NW + KT_NP) * 32;
 constexpr int KT_RPP = (KT_W + KT_NP - 1) / KT_NP;   // stage rows per producer warp
 static_assert(KT_RPP <= 32 && KT_NW + KT_NP <= 32, "tile kernel configuration");
@@ -72,6 +73,34 @@ struct KirchTileParams {
     int *sched_flags;    // [0] != 0: some interval of the image is wider than KT_SPAN -> this kernel stands down (table kernel runs)
     int t_base;          // first row of block 0: the multiple of KT_Q at or below the launch's first row
 };
+
+// Where source row k sits in the staging buffer: stage ring slot `slot`, row j of the stage, for the block's offset
+// interval e = {mlo, mhi} = seg[b][k].  The left segment g[k, x0 - mhi ..] and the right segment g[k, x0 + mlo ..] are
+// each copied from the 16-byte boundary at or below their first element (cp.async.bulk alignment), so output trace
+// x0 + i reads offset m at buf[ol + i - m] (left) and buf[orr + i + m] (right).  The producers copy by it and the
+// consumers decode table entries by it: this is the one definition of the layout.
+struct KtPlace {
+    long long gl, gr;   // first element of the left / right copy in gP (multiples of 4)
+    unsigned nl, nr;    // floats per copy (multiples of 4)
+    int dl, dr;         // first float of the left / right copy in buf
+    int ol, orr;        // buf index of output trace x0's element at m = 0, left / right
+};
+__device__ __forceinline__ KtPlace kt_place(const KirchTabParams &p, int x0, int k, int slot, int j, int2 e) {
+    const int span = e.y - e.x;
+    const long long rowoff = (long long)k * p.Tp + p.Apad + x0;
+    const long long il = rowoff - e.y, ir = rowoff + e.x;          // first element of the left / right segment
+    const int shl = (int)(il & 3), shr = (int)(ir & 3);
+    KtPlace r;
+    r.gl = il - shl;
+    r.gr = ir - shr;
+    r.nl = (unsigned)((shl + KT_X + span + 3) & ~3);
+    r.nr = (unsigned)((shr + KT_X + span + 3) & ~3);
+    r.dl = slot * KT_STAGE_FLOATS + j * 2 * KT_SEGW;
+    r.dr = r.dl + KT_SEGW;
+    r.ol = r.dl + shl + e.y;
+    r.orr = r.dr + shr - e.x;
+    return r;
+}
 
 __device__ __forceinline__ unsigned kt_smem_u32(const void *p) { return (unsigned)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void kt_mbar_init(unsigned long long *bar, int count) {
@@ -181,8 +210,7 @@ __global__ void __launch_bounds__(KT_THREADS, 1) kirch_tile_kernel(const __grid_
     const int r_lo = max(t0, p.flags[0]);           // rows ti < flags[0] read non-finite input: the table kernel does them
     if (min(t0 + KT_Q, p.s_end) <= r_lo) return;
     float *buf = reinterpret_cast<float *>(kt_smem_raw);
-    int2 *hdr = reinterpret_cast<int2 *>(buf + (size_t)KT_NST * KT_STAGE_FLOATS);
-    int2 *rings = hdr + KT_NST * KT_W;
+    int4 *rings = reinterpret_cast<int4 *>(buf + (size_t)KT_NST * KT_STAGE_FLOATS);
     unsigned long long *full = reinterpret_cast<unsigned long long *>(rings + KT_NW * KT_RW * KT_RING);
     unsigned long long *empty = full + KT_NST;
 
@@ -190,6 +218,7 @@ __global__ void __launch_bounds__(KT_THREADS, 1) kirch_tile_kernel(const __grid_
     const int nst = q.nstage[b];
     const int kbase = (t0 / KT_W) * KT_W;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int2 *__restrict__ sb = q.seg + (size_t)b * p.S;
 
     if (threadIdx.x == 0) {
         for (int i = 0; i < KT_NST; ++i) {
@@ -203,11 +232,9 @@ __global__ void __launch_bounds__(KT_THREADS, 1) kirch_tile_kernel(const __grid_
     if (warp >= KT_NW) {
         // ------------------------------------------------- producers: warp pw issues rows [pw KT_RPP, (pw + 1) KT_RPP) of a stage
         const int pw = warp - KT_NW;
-        const int2 *__restrict__ sb = q.seg + (size_t)b * p.S;
         for (int s = 0; s < nst; ++s) {
             const int slot = s % KT_NST;
             if (s >= KT_NST) kt_mbar_wait(&empty[slot], (unsigned)((s / KT_NST - 1) & 1));
-            float *sbuf = buf + (size_t)slot * KT_STAGE_FLOATS;
             unsigned bytes = 0, nl = 0, nr = 0;
             const float *gl = nullptr, *gr = nullptr;
             float *dl = nullptr, *dr = nullptr;
@@ -217,18 +244,13 @@ __global__ void __launch_bounds__(KT_THREADS, 1) kirch_tile_kernel(const __grid_
                 int2 e = make_int2(1, 0);
                 if (k >= t0 && k < p.S) e = sb[k];
                 if (e.y >= e.x) {
-                    const int span = e.y - e.x;
-                    const long long rowoff = (long long)k * p.Tp + p.Apad + x0;
-                    const long long il = rowoff - e.y, ir = rowoff + e.x;          // first element of the left / right segment
-                    const int shl = (int)(il & 3), shr = (int)(ir & 3);
-                    nl = (unsigned)((shl + KT_X + span + 3) & ~3);
-                    nr = (unsigned)((shr + KT_X + span + 3) & ~3);
-                    gl = p.gP + (il - shl);
-                    gr = p.gP + (ir - shr);
-                    dl = sbuf + (size_t)j * 2 * KT_SEGW;
-                    dr = dl + KT_SEGW;
-                    // value of output trace x0 + i at offset m: left  buf[offL + i - m], right buf[offR + i + m]
-                    hdr[slot * KT_W + j] = make_int2((int)(dl - buf) + shl + e.y, (int)(dr - buf) + shr - e.x);
+                    const KtPlace pl = kt_place(p, x0, k, slot, j, e);
+                    nl = pl.nl;
+                    nr = pl.nr;
+                    gl = p.gP + pl.gl;
+                    gr = p.gP + pl.gr;
+                    dl = buf + pl.dl;
+                    dr = buf + pl.dr;
                     bytes = (nl + nr) * 4u;
                 }
             }
@@ -247,68 +269,88 @@ __global__ void __launch_bounds__(KT_THREADS, 1) kirch_tile_kernel(const __grid_
     // -------------------------------------------------------------------- consumers: warp = KT_RW output rows x KT_X traces
     // accumulators as fp32x2 pairs: the adds and FMAs issue on the packed pipe (half the instructions, same roundings)
     float2 acc[KT_RW][KT_TR / 2], tot[KT_RW][KT_TR / 2];
-    // The table row of an output sample is walked once, front to back.  It is fetched 32 entries at a time with one
-    // coalesced load per lane, a chunk ahead of its use, and parked in a warp-private shared-memory ring, so the walk
-    // itself never waits on global memory (the L1 left beside 200 KB of staging buffers does not hold 31 table rows).
-    int mcur[KT_RW], mend[KT_RW], cready[KT_RW];
-    bool live[KT_RW];                               // the row is this launch's and this kernel's to write
+    // The table row of an output sample is walked once, front to back, a chunk of 32 entries at a time.  The raw entries
+    // {k, w} come with one coalesced load per lane a chunk ahead of their use (the L1 left beside 200 KB of staging
+    // buffers does not hold 31 table rows).  Each lane then decodes one entry of the chunk into what the walk needs:
+    // the shared-memory offsets of its source row's two segments, already shifted by -m and +m, and the weight.  Skips
+    // (k < 0) are compacted away; the rest go into a warp-private ring, one 16-byte broadcast read per entry, issued an
+    // entry ahead of its use.  Each lane keeps the stage of the entry it decoded (csk), so one ballot per stage gives
+    // the stage's trip count: the walk itself compares nothing but its index.
+    int mnext[KT_RW], mend[KT_RW];     // first table entry of the next chunk; entries in the row
+    int pos[KT_RW], cnt[KT_RW];        // next ring entry to walk; entries in the ring
+    int csk[KT_RW];                    // per lane: stage of the lane's decoded entry (INT_MAX: none)
+    bool live[KT_RW];                  // the row is this launch's and this kernel's to write
     const int2 *trow[KT_RW];
     int2 pre[KT_RW];
-    int2 *ring[KT_RW];
-    const int2 sentinel = make_int2(0x7fffffff, 0);
+    int4 *ring[KT_RW];
+    int4 cur[KT_RW];                   // ring[pos], read ahead
+    const int2 none = make_int2(-1, 0);
+    // Chunk mnext of row w into the ring (which the walk has emptied); the next chunk's load goes out.
+    auto decode = [&](int w) {
+        const int m = mnext[w] + lane;
+        const int2 e = pre[w];
+        pre[w] = m + 32 < mend[w] ? __ldg(trow[w] + m + 32) : none;
+        const unsigned v = __ballot_sync(0xffffffffu, e.x >= 0);
+        __syncwarp();                  // every lane has read the previous chunk's entries
+        csk[w] = 0x7fffffff;
+        if (e.x >= 0) {
+            const unsigned rel = (unsigned)(e.x - kbase), sk = rel / KT_W;
+            const KtPlace pl = kt_place(p, x0, e.x, (int)(sk % KT_NST), (int)(rel % KT_W), __ldg(sb + e.x));
+            // m == 0: left and right segment hold the same element, w/2 (g + g) == w g exactly
+            const float wgt = __int_as_float(e.y) * (m == 0 ? 0.5f : 1.0f);
+            ring[w][__popc(v & ((1u << lane) - 1u))] =
+                make_int4((pl.ol - m) * 4, (pl.orr + m) * 4, __float_as_int(wgt), 0);   // byte offsets
+            csk[w] = (int)sk;
+        }
+        __syncwarp();
+        mnext[w] += 32;
+        pos[w] = 0;
+        cnt[w] = __popc(v);
+        cur[w] = ring[w][0];
+    };
 #pragma unroll
     for (int w = 0; w < KT_RW; ++w) {
         const int ti = t0 + warp + w * KT_NW;
         live[w] = ti >= max(p.s_begin, r_lo) && ti < p.s_end && (x0 < p.x_end);
-        mcur[w] = 0;
+        mnext[w] = 0;
         mend[w] = live[w] ? p.nm[ti] : 0;
         trow[w] = p.tab + (size_t)(live[w] ? ti : t0) * p.A1;
         ring[w] = rings + (size_t)(warp * KT_RW + w) * KT_RING;
-        ring[w][lane] = lane < mend[w] ? __ldg(trow[w] + lane) : sentinel;              // chunk 0
-        pre[w] = 32 + lane < mend[w] ? __ldg(trow[w] + 32 + lane) : sentinel;            // chunk 1, parked when chunk 0 is entered
-        cready[w] = 0;
+        pre[w] = lane < mend[w] ? __ldg(trow[w] + lane) : none;
+        decode(w);
 #pragma unroll
         for (int r = 0; r < KT_TR / 2; ++r) acc[w][r] = tot[w][r] = make_float2(0.f, 0.f);
     }
-    __syncwarp();
-    const float *__restrict__ lbuf = buf + lane;
+    const char *__restrict__ lbuf = reinterpret_cast<const char *>(buf + lane);
     const int sabs0 = kbase / KT_W;                 // absolute index of this block's first stage window
     for (int s = 0; s < nst; ++s) {
         const int slot = s % KT_NST;
         kt_mbar_wait(&full[slot], (unsigned)((s / KT_NST) & 1));
-        const int k0 = kbase + s * KT_W, kend = k0 + KT_W;
-        const int2 *__restrict__ h = hdr + slot * KT_W - k0;
 #pragma unroll
         for (int w = 0; w < KT_RW; ++w) {
-            int m = mcur[w];
             while (true) {
-                const int c = m >> 5;
-                if (c + 1 > cready[w]) {               // entering chunk c: chunk c + 1 goes into the other half of the ring
-                    ring[w][((c + 1) & 1) * 32 + lane] = pre[w];
-                    __syncwarp();
-                    const int nx = (c + 2) * 32 + lane;
-                    pre[w] = nx < mend[w] ? __ldg(trow[w] + nx) : sentinel;
-                    cready[w] = c + 1;
-                }
-                const int2 e = ring[w][m & (KT_RING - 1)];
-                if (e.x >= kend) break;                // next stage, or the sentinel past the end of the row
-                if (e.x >= 0) {
-                    const int2 o = h[e.x];
-                    // m == 0: left and right segment hold the same element, w/2 (g + g) == w g exactly
-                    const float wgt = __int_as_float(e.y) * (m == 0 ? 0.5f : 1.0f);
+                const int end = __popc(__ballot_sync(0xffffffffu, csk[w] <= s));   // the ring's entries of stages <= s
+                int4 d = cur[w];
+#pragma unroll 1   // short trips (at rho 0.169, 62 % of warp-stages walk 2-3 entries): unrolled copies measured slower
+                for (int i = pos[w]; i < end; ++i) {
+                    const int4 nx = ring[w][i + 1];
+                    const float *__restrict__ pl = reinterpret_cast<const float *>(lbuf + d.x);
+                    const float *__restrict__ pr = reinterpret_cast<const float *>(lbuf + d.y);
+                    const float wgt = __int_as_float(d.z);
                     const float2 w2 = make_float2(wgt, wgt);
-                    const float *__restrict__ pl = lbuf + (o.x - m);
-                    const float *__restrict__ pr = lbuf + (o.y + m);
 #pragma unroll
                     for (int r = 0; r < KT_TR / 2; ++r) {
                         const float2 l = make_float2(pl[64 * r], pl[64 * r + 32]);
                         const float2 g = make_float2(pr[64 * r], pr[64 * r + 32]);
                         acc[w][r] = __ffma2_rn(w2, __fadd2_rn(l, g), acc[w][r]);
                     }
+                    d = nx;
                 }
-                ++m;
+                cur[w] = d;
+                pos[w] = end;
+                if (end < cnt[w] || mnext[w] >= mend[w]) break;   // the stage ends inside this chunk, or the row does
+                decode(w);
             }
-            mcur[w] = m;
         }
         if (((sabs0 + s) & (KT_FLUSH - 1)) == KT_FLUSH - 1) {     // second-level accumulation at absolute window indices
 #pragma unroll
