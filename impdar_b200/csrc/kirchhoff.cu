@@ -18,9 +18,14 @@
 //     so the picked sample is the reference's for every pair.
 //   * the aperture cut 2r/v > max(tt) is resolved exactly once per output sample (binary search with the
 //     float64 predicate over the ascending trace positions), so the inner loop only tests a trace range.
+//   * the velocity is one RMS value per output sample, v[ti] (a constant vector is the reference's single vel):
+//     every formula above uses v[ti] for the pairs of output row ti.
 #include <math.h>
 
+#include <cmath>
 #include <mutex>
+#include <type_traits>
+#include <vector>
 
 #include "common.cuh"
 
@@ -32,13 +37,16 @@ struct KirchParams {
     float *out;           // (S, ldo)
     const double *dist;   // T  [m]
     const double *tt;     // S  [s]
-    const double *zs;     // S  vel*tt/2
+    const double *zs;     // S  v*tt/2
     const double *zs2;    // S  zs^2
+    const double *vs;     // S  RMS velocity of each output row
+    const float3 *rowc;   // S  {sigma = (cs_ti / cs)^2, 1/(2 pi v_ti), 4/(v_ti dt)^2/(2 pi)} (kirch_prep_vectors_kernel)
     const int *flags;     // [0] = 1 + the deepest row of the d/dt (or data) image holding a non-finite value, 0 if none
     unsigned long long *stats;  // [0] pairs, [1] exact pairs
     int S, T, SP, ldo, x_begin, x_end;
-    double vel, tmax, tt0, inv_dt, cs;  // cs = 2/(vel*dt_eff)
-    float neg_u0, thr, wfar, wnear;     // thr = 0.5 - delta ; wfar = 1/(2 pi vel) ; wnear = 4/(vel dt)^2/(2 pi)
+    unsigned kmax;                         // SP - 1
+    double tmax, tt0, inv_dt, cs;          // cs = 2/(vmin*dt_eff): the offset scale of the staged C^2
+    float neg_u0, thr;                     // thr = 0.5 - delta; -1 (every pair exact) for non-monotone positions
     int monotone;                       // dist ascending -> per-sample aperture by binary search
     int rowmajor, Tp, Apad;             // table path: gradT/dataT are (S, Tp) row-major, trace x at column Apad + x
 };
@@ -52,7 +60,8 @@ __device__ __forceinline__ float rsqrt_approx(float x) {
     return r;
 }
 
-// The reference's own float64 sequence for one pair: returns t = 2*sqrt(d^2 + zs2)/vel without contraction.
+// The reference's own float64 sequence for one pair: returns t = 2*sqrt(d^2 + zs2)/vel without contraction
+// (vel = v[ti] of the pair's output row).
 __device__ __forceinline__ double exact_time(double d, double zs2, double vel, double &rs) {
     rs = __dsqrt_rn(__dadd_rn(__dmul_rn(d, d), zs2));
     return __ddiv_rn(__dmul_rn(2.0, rs), vel);
@@ -79,13 +88,14 @@ template <bool NEAR>
 __device__ __forceinline__ float exact_term(const KirchParams &p, int ti, int x, double dxi) {
     const double d = __dsub_rn(p.dist[x], dxi);
     double rs;
-    const double t = exact_time(d, p.zs2[ti], p.vel, rs);
+    const double vel = p.vs[ti];
+    const double t = exact_time(d, p.zs2[ti], vel, rs);
     if (t > p.tmax) return 0.f;
     const int k = exact_pick(p.tt, p.S, t, p.tt0, p.inv_dt);
     const double costheta = p.zs[ti] / rs;
     const size_t gi = p.rowmajor ? (size_t)k * p.Tp + p.Apad + x : (size_t)x * p.SP + k;
     const double g = (double)p.gradT[gi];
-    double term = g * costheta / p.vel;
+    double term = g * costheta / vel;
     if (term != term) term = 0.0;
     if (NEAR) {
         const double dv = (double)p.dataT[gi];
@@ -102,7 +112,7 @@ template <bool NEAR, bool STATS, bool HASNAN, typename Flush>
 __device__ __forceinline__ void kirch_chunk(Flush &flush, const float *__restrict__ gT, const float *__restrict__ dT,
                                             const float *__restrict__ sCw, int *__restrict__ sQw, int jend,
                                             unsigned rowoff, unsigned SP, unsigned kmax, int rel, unsigned span,
-                                            int xb, int lane, float u2, float Uw, float Un, float neg_u0, float thr,
+                                            int xb, int lane, float u2, float sigma, float Uw, float Un, float neg_u0, float thr,
                                             float &acc0, float &acc1, int &qn, unsigned &npairs, unsigned &nexact) {
 #pragma unroll 1
     for (int j0 = 0; j0 < jend; j0 += 4) {
@@ -111,7 +121,7 @@ __device__ __forceinline__ void kirch_chunk(Flush &flush, const float *__restric
         unsigned amb4 = 0;
 #pragma unroll
         for (int jj = 0; jj < 4; ++jj) {
-            const float q = u2 + c[jj];
+            const float q = fmaf(c[jj], sigma, u2);   // u2 + c[jj] exactly when sigma == 1 (constant velocity)
             const float s = rsqrt_approx(q);
             const float f = fmaf(q, s, neg_u0);
             const float r = f + KIRCH_MAGIC;
@@ -187,7 +197,6 @@ __global__ void __launch_bounds__(256) kirch_general_kernel(const __grid_constan
     if (warp_active) {
         const double dxi = p.dist[xi];
         const int tic = active ? ti : p.S - 1;
-        const double zs2i = p.zs2[tic];
         const double Ud = p.tt[tic] * p.inv_dt;
         const float U = (float)Ud;
         const float u2 = fmaxf((float)(Ud * Ud), 1e-30f);  // q == 0 only at the apex of a zero-depth sample (weight 0)
@@ -195,19 +204,20 @@ __global__ void __launch_bounds__(256) kirch_general_kernel(const __grid_constan
         // exact per-sample aperture [xlo, xhi]: pairs with 2r/v > max(tt) contribute exactly 0
         int xlo = xi + 1, xhi = xi;
         if (active) {
+            const double zs2i = p.zs2[ti], vi = p.vs[ti];
             double rs;
-            if (!(exact_time(0.0, zs2i, p.vel, rs) > p.tmax)) {
+            if (!(exact_time(0.0, zs2i, vi, rs) > p.tmax)) {
                 if (p.monotone) {
                     int a = 0, b = xi;  // smallest x in [0, xi] inside
                     while (a < b) {
                         int m = (a + b) >> 1;
-                        if (exact_time(__dsub_rn(p.dist[m], dxi), zs2i, p.vel, rs) > p.tmax) a = m + 1; else b = m;
+                        if (exact_time(__dsub_rn(p.dist[m], dxi), zs2i, vi, rs) > p.tmax) a = m + 1; else b = m;
                     }
                     xlo = a;
                     a = xi; b = p.T - 1;  // largest x in [xi, T-1] inside
                     while (a < b) {
                         int m = (a + b + 1) >> 1;
-                        if (exact_time(__dsub_rn(p.dist[m], dxi), zs2i, p.vel, rs) > p.tmax) b = m - 1; else a = m;
+                        if (exact_time(__dsub_rn(p.dist[m], dxi), zs2i, vi, rs) > p.tmax) b = m - 1; else a = m;
                     }
                     xhi = a;
                 } else {
@@ -227,9 +237,12 @@ __global__ void __launch_bounds__(256) kirch_general_kernel(const __grid_constan
             span = 0;
             xlo = 0x40000000;
         }
-        const float thr = p.monotone ? p.thr : -1.f;  // non-monotone positions: every pair takes the exact path
-        const float Uw = U * p.wfar, Un = U * p.wnear;
-        const unsigned SP = (unsigned)p.SP, kmax = SP - 1u;
+        // Per-row velocity (kirch_prep_vectors_kernel): the staged c2v carries the offset scale cs = 2/(vmin dt) and
+        // this row's C^2 is c2v * sigma; the weights are 1/(2 pi v_ti) and 4/(v_ti dt)^2/(2 pi).
+        const float3 rc = p.rowc[tic];
+        const float sigma = rc.x;
+        const float Uw = U * rc.y, Un = U * rc.z;
+        const unsigned SP = (unsigned)p.SP;
         int qn = 0;
 
         auto flush = [&](int count) {
@@ -251,28 +264,29 @@ __global__ void __launch_bounds__(256) kirch_general_kernel(const __grid_constan
             }
         };
 
-        for (int xb = xlo_w; xb <= xhi_w; xb += 32) {
-            {
-                const int xx = xb + lane;
-                float c2v = 0.f;
-                if (xx <= xhi_w) {
-                    const double C = (p.dist[xx] - dxi) * p.cs;
-                    c2v = (float)(C * C);
+        // One trace loop per variant, chosen once: a non-finite flag kept live across the loop spills a register.
+        auto trace_loop = [&](auto nan_variant) {
+            for (int xb = xlo_w; xb <= xhi_w; xb += 32) {
+                {
+                    const int xx = xb + lane;
+                    float c2v = 0.f;
+                    if (xx <= xhi_w) {
+                        const double C = (p.dist[xx] - dxi) * p.cs;
+                        c2v = (float)(C * C);
+                    }
+                    __syncwarp();
+                    sC[warp][lane] = c2v;
+                    __syncwarp();
                 }
-                __syncwarp();
-                sC[warp][lane] = c2v;
-                __syncwarp();
+                const int jend = (min(32, xhi_w - xb + 1) + 3) & ~3;   // padded entries fall outside every lane's range
+                const unsigned rowoff = (unsigned)xb * SP;
+                const int rel = xb - xlo;
+                kirch_chunk<NEAR, STATS, decltype(nan_variant)::value>(
+                    flush, p.gradT, p.dataT, sC[warp], sQ[warp], jend, rowoff, SP, p.kmax, rel, span, xb, lane, u2, sigma, Uw,
+                    Un, p.neg_u0, p.thr, acc0, acc1, qn, npairs, nexact);
             }
-            const int jend = (min(32, xhi_w - xb + 1) + 3) & ~3;   // padded entries fall outside every lane's range
-            const unsigned rowoff = (unsigned)xb * SP;
-            const int rel = xb - xlo;
-            if (hasnan)
-                kirch_chunk<NEAR, STATS, true>(flush, p.gradT, p.dataT, sC[warp], sQ[warp], jend, rowoff, SP, kmax, rel, span,
-                                               xb, lane, u2, Uw, Un, p.neg_u0, thr, acc0, acc1, qn, npairs, nexact);
-            else
-                kirch_chunk<NEAR, STATS, false>(flush, p.gradT, p.dataT, sC[warp], sQ[warp], jend, rowoff, SP, kmax, rel, span,
-                                                xb, lane, u2, Uw, Un, p.neg_u0, thr, acc0, acc1, qn, npairs, nexact);
-        }
+        };
+        if (hasnan) trace_loop(std::true_type{}); else trace_loop(std::false_type{});
         __syncwarp();
         if (qn > 0) flush(qn);
     }
@@ -340,13 +354,23 @@ __global__ void __launch_bounds__(256) grad_transpose_kernel(const float *__rest
     if (bad && threadIdx.x == 0) atomicMax(flags, bad);
 }
 
-__global__ void kirch_prep_vectors_kernel(const double *__restrict__ tt, double *__restrict__ zs,
-                                          double *__restrict__ zs2, int S, double vel) {
+// Per-row vectors: zs, zs2 (float64, the reference's operation order) and the general kernel's float32 row constants.
+// cs_i / cs = 1 exactly when v_ti is the velocity cs was made with, so a constant vector has sigma == 1 and the
+// weights are the single-velocity values bit for bit.
+__global__ void kirch_prep_vectors_kernel(const double *__restrict__ tt, const double *__restrict__ vs,
+                                          double *__restrict__ zs, double *__restrict__ zs2, float3 *__restrict__ rowc,
+                                          int S, double dt_eff, double cs) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < S) {
-        const double z = __ddiv_rn(__dmul_rn(vel, tt[i]), 2.0);  // zs = vel * tt_sec / 2.0   (:101)
+        const double v = vs[i];
+        const double z = __ddiv_rn(__dmul_rn(v, tt[i]), 2.0);   // zs = vel * tt_sec / 2.0   (:101)
         zs[i] = z;
         zs2[i] = __dmul_rn(z, z);                                // zs2 = zs**2.              (:102)
+        const double vdt = __dmul_rn(v, dt_eff);
+        const double sr = __ddiv_rn(__ddiv_rn(2.0, vdt), cs);   // cs_i / cs, cs_i = 2 / (v dt)
+        rowc[i] = make_float3((float)__dmul_rn(sr, sr),
+                              (float)__ddiv_rn(1.0, __dmul_rn(2.0 * 3.14159265358979323846, v)),
+                              (float)__ddiv_rn(__ddiv_rn(4.0, __dmul_rn(vdt, vdt)), 2.0 * 3.14159265358979323846));
     }
 }
 
@@ -380,13 +404,15 @@ __global__ void __launch_bounds__(128) kirch_table_build_kernel(int2 *__restrict
                                                                 int *__restrict__ nm, int S, int A1, double dxm,
                                                                 const double *__restrict__ zs,
                                                                 const double *__restrict__ zs2,
-                                                                const double *__restrict__ tt, double vel, double tmax,
+                                                                const double *__restrict__ tt,
+                                                                const double *__restrict__ vs, double tmax,
                                                                 double tt0, double inv_dt, double eps_t,
                                                                 int *__restrict__ amb_list, int *__restrict__ amb_count) {
     const int m = blockIdx.x * blockDim.x + threadIdx.x;
     const int ti = blockIdx.y;
     if (m >= A1) return;
     const double d = (double)m * dxm;
+    const double vel = vs[ti];
     double rs;
     const double t = exact_time(d, zs2[ti], vel, rs);
     int k = -1;
@@ -639,9 +665,10 @@ struct KirchRows {
     int s_begin, s_end, g_hi;
 };
 // Column window of the input (impdar_kirchhoff_window_f32): `data` holds radargram columns [col0, col0 + ncols), row
-// stride ld; `out` has row stride ldo.
+// stride ld; `out` has row stride ldo.  any_order: the window is the whole image, so trace positions need not ascend.
 struct KirchWindow {
     int col0, ncols, ld, ldo;
+    bool any_order;
 };
 // Side streams and events of the host pipeline: one set per device, created on first use under a lock.  Selection
 // switches and "last call" records are per host thread (SURVEY.md 8b: one host thread - or process - per GPU).
@@ -670,7 +697,7 @@ static int kirch_pipe_streams(KirchPipe **out) {
     return IMPDAR_B200_OK;
 }
 
-// Geometry vectors (travel times, d/dt coefficients, trace positions) go up through a small ring of page-locked staging
+// Geometry vectors (travel times, d/dt coefficients, per-row velocities, trace positions) go up through a small ring of page-locked staging
 // buffers per device: an asynchronous copy from pageable memory makes the HOST wait until the stream has drained, which
 // kept the caller from enqueueing the next call (or the next step of a multi-GPU pipeline) while this one runs.
 constexpr int KV_SLOTS = 4;
@@ -685,12 +712,12 @@ struct KirchVecRing {
     int next;
 };
 static KirchVecRing g_vecs[KP_MAX_DEVICES];
-static int kirch_stage_vectors(const double *tt, const double *coef, const double *dist, int S, int T, double *d_dst,
-                               cudaStream_t st) {
+static int kirch_stage_vectors(const double *tt, const double *coef, const double *vel_s, const double *dist, int S, int T,
+                               double *d_dst, cudaStream_t st) {
     int dev = 0;
     IMPDAR_CUDA(cudaGetDevice(&dev));
     IMPDAR_CHECK_ARG(dev >= 0 && dev < KP_MAX_DEVICES, "kirchhoff: device index %d out of range", dev);
-    const size_t bytes = ((size_t)4 * S + (size_t)T) * sizeof(double);
+    const size_t bytes = ((size_t)5 * S + (size_t)T) * sizeof(double);
     std::lock_guard<std::mutex> lk(g_pipe_mu);
     KirchVecRing &ring = g_vecs[dev];
     KirchVecSlot &sl = ring.slot[ring.next];
@@ -707,7 +734,8 @@ static int kirch_stage_vectors(const double *tt, const double *coef, const doubl
     double *h = (double *)sl.host;
     memcpy(h, tt, (size_t)S * sizeof(double));
     memcpy(h + S, coef, (size_t)3 * S * sizeof(double));
-    memcpy(h + (size_t)4 * S, dist, (size_t)T * sizeof(double));
+    memcpy(h + (size_t)4 * S, vel_s, (size_t)S * sizeof(double));
+    memcpy(h + (size_t)5 * S, dist, (size_t)T * sizeof(double));
     IMPDAR_CUDA(cudaMemcpyAsync(d_dst, h, bytes, cudaMemcpyHostToDevice, st));
     IMPDAR_CUDA(cudaEventRecord(sl.ev, st));
     sl.used = true;
@@ -747,13 +775,27 @@ size_t impdar_kirchhoff_workspace_bytes(int S, int T, int nearfield) {
     const size_t table = ((size_t)S * tp + 4096) * sizeof(float) * nf + (size_t)S * (size_t)T * (sizeof(int2) + sizeof(int) + (nearfield ? 4 : 0)) +
                          (size_t)S * sizeof(int) + nblk * ((size_t)S * sizeof(int2) + sizeof(int)) + 1024;
     size_t b = general > table ? general : table;
-    b += 6 * (size_t)S * sizeof(double);  // zs, zs2, tt, grad coefficients
+    b += 9 * (size_t)S * sizeof(double);  // zs, zs2, general-kernel row constants, tt, grad coefficients, velocity
     b += (size_t)T * sizeof(double);      // dist
     return b + 4096;
 }
 
+// Per-row velocity vectors of the _vz entries: finite and > 0; returns the largest (it bounds the reach of every pair).
+static int kirch_vel_range(const double *vel_s, int S, double *vmax) {
+    IMPDAR_CHECK_ARG(vel_s, "kirchhoff: null velocity vector");
+    double hi = vel_s[0];
+    for (int i = 0; i < S; ++i) {
+        IMPDAR_CHECK_ARG(std::isfinite(vel_s[i]) && vel_s[i] > 0.0,
+                         "kirchhoff: velocity[%d] = %g must be finite and positive", i, vel_s[i]);
+        hi = fmax(hi, vel_s[i]);
+    }
+    *vmax = hi;
+    return IMPDAR_B200_OK;
+}
+
 int impdar_kirchhoff_input_window(int S, int T, const double *dist_m, const double *tt_s, double vel, int x_begin,
                                   int x_end, int *col0, int *col1) {
+    // vel is the largest velocity of the rows (the reach of a pair grows with it)
     IMPDAR_CHECK_ARG(dist_m && tt_s && col0 && col1, "kirchhoff_input_window: null pointer");
     IMPDAR_CHECK_ARG(S >= 2 && T >= 1 && 0 <= x_begin && x_begin < x_end && x_end <= T, "kirchhoff_input_window: bad range");
     double tmax = tt_s[0];
@@ -786,14 +828,20 @@ int impdar_kirchhoff_input_window(int S, int T, const double *dist_m, const doub
 }
 
 static int kirchhoff_impl(const float *data, float *out, int S, int T, const double *dist_m, const double *tt_s,
-                          const double *grad_coef, double vel, int nearfield, int x_begin, int x_end,
+                          const double *grad_coef, const double *vel_s, int nearfield, int x_begin, int x_end,
                           void *workspace, size_t ws_bytes, void *stream, const KirchPipe *pipe,
                           const KirchRows *rows = nullptr, const KirchWindow *win = nullptr) {
-    IMPDAR_CHECK_ARG(data && out && dist_m && tt_s && grad_coef, "kirchhoff: null pointer");
+    IMPDAR_CHECK_ARG(data && out && dist_m && tt_s && grad_coef && vel_s, "kirchhoff: null pointer");
     IMPDAR_CHECK_ARG(S >= 2 && T >= 1, "kirchhoff: need snum >= 2, tnum >= 1");
     IMPDAR_CHECK_ARG(0 <= x_begin && x_begin < x_end && x_end <= T, "kirchhoff: bad output range [%d, %d)",
                      x_begin, x_end);
-    IMPDAR_CHECK_ARG(vel > 0.0, "kirchhoff: vel must be positive");
+    double vmin = vel_s[0], vmax = vel_s[0];
+    for (int i = 0; i < S; ++i) {
+        IMPDAR_CHECK_ARG(vel_s[i] > 0.0, "kirchhoff: vel must be positive");
+        vmin = fmin(vmin, vel_s[i]);
+        vmax = fmax(vmax, vel_s[i]);
+    }
+    const bool vconst = vmin == vmax;
     IMPDAR_CHECK_ARG(T < (1 << 26), "kirchhoff: tnum too large");
     const size_t need = impdar_kirchhoff_workspace_bytes(S, T, nearfield);
     IMPDAR_CHECK_ARG(workspace && ws_bytes >= need, "kirchhoff: workspace too small (%zu < %zu)", ws_bytes, need);
@@ -804,7 +852,7 @@ static int kirchhoff_impl(const float *data, float *out, int S, int T, const dou
         IMPDAR_CHECK_ARG(c0 >= 0 && ncols >= 1 && c0 + ncols <= T && ld >= ncols && ldo >= x_end - x_begin,
                          "kirchhoff_window: bad column window [%d, %d) / strides", c0, c0 + ncols);
         int need0 = 0, need1 = T;
-        int rcw = impdar_kirchhoff_input_window(S, T, dist_m, tt_s, vel, x_begin, x_end, &need0, &need1);
+        int rcw = impdar_kirchhoff_input_window(S, T, dist_m, tt_s, vmax, x_begin, x_end, &need0, &need1);
         if (rcw) return rcw;
         IMPDAR_CHECK_ARG(c0 <= need0 && c0 + ncols >= need1,
                          "kirchhoff_window: output traces [%d, %d) read input columns [%d, %d), the window holds [%d, %d)",
@@ -832,7 +880,11 @@ static int kirchhoff_impl(const float *data, float *out, int S, int T, const dou
     // fp32 error budget of f = sqrt(U^2 + C^2) - U0 (sample units): ~4 ulp relative on a value <= S + |U0|,
     // plus the deviation of tt from a uniform grid.
     const double u0 = tt0 / dt_eff;
+    // A per-row velocity adds one rounding: q = fmaf(c2v, sigma, u2) with sigma = (v_min / v_i)^2 rounded to float,
+    // i.e. <= 2^-24 more relative error on the C^2 part of q (<= q), <= 2^-25 sqrt(q) <= 3e-8 (S + |U0|) on f after the
+    // square root.  A constant vector has sigma == 1 exactly (no extra rounding) and keeps the budget above unchanged.
     double delta = 6e-7 * ((double)S + fabs(u0) + 64.0) + 2.0 * maxdev / dt_eff + 1e-6;
+    if (!vconst) delta += 6e-8 * ((double)S + fabs(u0) + 64.0);
     float thr = (float)(0.5 - delta);
     if (delta > 0.2) thr = -1.f;  // irregular sampling: everything through the exact path
 
@@ -845,11 +897,11 @@ static int kirchhoff_impl(const float *data, float *out, int S, int T, const dou
             if (dev > maxdev_d) maxdev_d = dev;
         }
     }
-    const double eps_t = (2.0 / vel) * (2.0 * maxdev_d) + 1e-15 * (fabs(tmax) + fabs(tt0));
+    const double eps_t = (2.0 / vmin) * (2.0 * maxdev_d) + 1e-15 * (fabs(tmax) + fabs(tt0));
     const bool uniform_ok = monotone && T > 1 && dxm > 0.0 && tmax > 0.0 && eps_t / dt_eff < 1e-5;
     IMPDAR_CHECK_ARG(!(g_kirch_mode >= 2 && !uniform_ok), "kirchhoff: table path forced but trace spacing is not uniform");
     const bool use_table = (g_kirch_mode >= 2) || (g_kirch_mode == 0 && uniform_ok);
-    IMPDAR_CHECK_ARG(!(win && !monotone), "kirchhoff_window: trace positions must be ascending");
+    IMPDAR_CHECK_ARG(!(win && !monotone && !win->any_order), "kirchhoff_window: trace positions must be ascending");
 
     // carve workspace: small vectors first
     char *w = (char *)workspace;
@@ -858,10 +910,14 @@ static int kirchhoff_impl(const float *data, float *out, int S, int T, const dou
     w += (size_t)S * sizeof(double);
     double *zs2 = (double *)w;
     w += (size_t)S * sizeof(double);
+    float3 *rowc = (float3 *)w;
+    w += (size_t)S * 2 * sizeof(double);
     double *d_tt = (double *)w;
     w += (size_t)S * sizeof(double);
     double *d_coef = (double *)w;
     w += 3 * (size_t)S * sizeof(double);
+    double *d_vel = (double *)w;
+    w += (size_t)S * sizeof(double);
     double *d_dist = (double *)w;
     w += (size_t)T * sizeof(double);
     int *flags = (int *)w;                         // [0] non-finite input, [8] ambiguous-entry count, [16] tile stand-down
@@ -870,28 +926,26 @@ static int kirchhoff_impl(const float *data, float *out, int S, int T, const dou
     w = (char *)(((uintptr_t)w + 255) & ~(uintptr_t)255);
     const bool continuing = rows && rows->g_hi < S;   // later call of a bottom-up row sequence: flags, tables, tile schedule, d/dt rows
     if (!continuing) {                                // and the vectors stay (same workspace, same stream)
-        // d_tt | d_coef (3 S) | d_dist are contiguous in the workspace: one copy from the page-locked staging slot
-        int rcv = kirch_stage_vectors(tt_s, grad_coef, dist_m, S, T, d_tt, st);
+        // d_tt | d_coef (3 S) | d_vel | d_dist are contiguous in the workspace: one copy from the page-locked staging slot
+        int rcv = kirch_stage_vectors(tt_s, grad_coef, vel_s, dist_m, S, T, d_tt, st);
         if (rcv) return rcv;
         IMPDAR_CUDA(cudaMemsetAsync(flags, 0, 256, st));
-        kirch_prep_vectors_kernel<<<(S + 255) / 256, 256, 0, st>>>(d_tt, zs, zs2, S, vel);
+        kirch_prep_vectors_kernel<<<(S + 255) / 256, 256, 0, st>>>(d_tt, d_vel, zs, zs2, rowc, S, dt_eff, 2.0 / (vmin * dt_eff));
         IMPDAR_LAUNCH_CHECK();
     }
 
     KirchParams p;
     memset(&p, 0, sizeof(p));
-    p.out = out; p.dist = d_dist; p.tt = d_tt; p.zs = zs; p.zs2 = zs2;
+    p.out = out; p.dist = d_dist; p.tt = d_tt; p.zs = zs; p.zs2 = zs2; p.vs = d_vel; p.rowc = rowc;
     p.flags = flags; p.stats = stats;
     p.S = S; p.T = T; p.ldo = ldo; p.x_begin = x_begin; p.x_end = x_end;
-    p.vel = vel; p.tmax = tmax; p.tt0 = tt0; p.inv_dt = 1.0 / dt_eff; p.cs = 2.0 / (vel * dt_eff);
-    p.neg_u0 = (float)(-u0); p.thr = thr;
-    p.wfar = (float)(1.0 / (2.0 * 3.14159265358979323846 * vel));
-    p.wnear = (float)(4.0 / ((vel * dt_eff) * (vel * dt_eff)) / (2.0 * 3.14159265358979323846));
+    p.tmax = tmax; p.tt0 = tt0; p.inv_dt = 1.0 / dt_eff; p.cs = 2.0 / (vmin * dt_eff);
+    p.neg_u0 = (float)(-u0); p.thr = monotone ? thr : -1.f;   // non-monotone positions: every pair takes the exact path
     p.monotone = monotone;
     int path = 1;
 
     if (use_table) {
-        const int Amax = kirch_amax(T, vel, tmax, dxm);
+        const int Amax = kirch_amax(T, vmax, tmax, dxm);
         const int A1 = Amax + 1;
         const int Apad = (int)kirch_roundup((size_t)Amax, 32);
         const int Tp = (int)kirch_roundup((size_t)ncols + 2 * (size_t)Apad, 32);
@@ -934,7 +988,7 @@ static int kirchhoff_impl(const float *data, float *out, int S, int T, const dou
             IMPDAR_CUDA(cudaMemsetAsync(gP, 0, img * (nearfield ? 2 : 1), st));
             IMPDAR_CUDA(cudaMemsetAsync(nm, 0, (size_t)S * sizeof(int), st));
             dim3 grid((A1 + 127) / 128, S);
-            kirch_table_build_kernel<<<grid, 128, 0, st>>>(tab, tabn, nm, S, A1, dxm, zs, zs2, d_tt, vel, tmax, tt0,
+            kirch_table_build_kernel<<<grid, 128, 0, st>>>(tab, tabn, nm, S, A1, dxm, zs, zs2, d_tt, d_vel, tmax, tt0,
                                                           1.0 / dt_eff, eps_t, amb_list, amb_count);
             IMPDAR_LAUNCH_CHECK();
         }
@@ -1061,6 +1115,7 @@ static int kirchhoff_impl(const float *data, float *out, int S, int T, const dou
         // stay inside the exact aperture, which the window covers (checked above); chunks of 4 traces may run up to 3
         // traces past it into the zero rows / the next traces, with zero weight.
         p.gradT = gradT - (size_t)c0 * SP; p.dataT = dataT ? dataT - (size_t)c0 * SP : nullptr; p.SP = SP;
+        p.kmax = (unsigned)SP - 1u;
         dim3 grid((S + 31) / 32, (x_end - x_begin + 7) / 8), block(32, 8);
         if (g_stats_enabled) {
             if (nearfield) { ktimer_begin("kirch_general_kernel", st); kirch_general_kernel<true, true><<<grid, block, 0, st>>>(p); ktimer_end(st); }
@@ -1084,11 +1139,13 @@ static int kirchhoff_impl(const float *data, float *out, int S, int T, const dou
     return IMPDAR_B200_OK;
 }
 
+// The scalar entries run the per-row code path with a constant vector: the same arithmetic as one velocity.
 int impdar_kirchhoff_f32(const float *data, float *out, int S, int T, const double *dist_m, const double *tt_s,
                          const double *grad_coef, double vel, int nearfield, int x_begin, int x_end,
                          void *workspace, size_t ws_bytes, void *stream) {
-    return kirchhoff_impl(data, out, S, T, dist_m, tt_s, grad_coef, vel, nearfield, x_begin, x_end, workspace, ws_bytes,
-                          stream, nullptr);
+    const std::vector<double> vs(S > 0 ? S : 0, vel);
+    return kirchhoff_impl(data, out, S, T, dist_m, tt_s, grad_coef, vs.data(), nearfield, x_begin, x_end, workspace,
+                          ws_bytes, stream, nullptr);
 }
 
 int impdar_kirchhoff_rows_f32(const float *data, float *out, int S, int T, const double *dist_m, const double *tt_s,
@@ -1096,24 +1153,55 @@ int impdar_kirchhoff_rows_f32(const float *data, float *out, int S, int T, const
                               int s_end, int g_hi, void *workspace, size_t ws_bytes, void *stream) {
     IMPDAR_CHECK_ARG(0 <= s_begin && s_begin < s_end && s_end <= S && s_end <= g_hi && g_hi <= S,
                      "kirchhoff_rows: need 0 <= s_begin < s_end <= g_hi <= snum, got [%d, %d), g_hi %d", s_begin, s_end, g_hi);
+    const std::vector<double> vs(S, vel);
     KirchRows rows = {s_begin, s_end, g_hi};
-    return kirchhoff_impl(data, out, S, T, dist_m, tt_s, grad_coef, vel, nearfield, x_begin, x_end, workspace, ws_bytes,
-                          stream, nullptr, &rows);
+    return kirchhoff_impl(data, out, S, T, dist_m, tt_s, grad_coef, vs.data(), nearfield, x_begin, x_end, workspace,
+                          ws_bytes, stream, nullptr, &rows);
+}
+
+static int kirchhoff_window(const float *data, int col0, int ncols, int ld, float *out, int ldo, int S, int T,
+                            const double *dist_m, const double *tt_s, const double *grad_coef, const double *vel_s,
+                            int nearfield, int x_begin, int x_end, int s_begin, int s_end, int g_hi, void *workspace,
+                            size_t ws_bytes, void *stream, bool any_order) {
+    KirchWindow win = {col0, ncols, ld, ldo, false};
+    if (s_begin == 0 && s_end == S && g_hi == S) {  // whole image: any geometry
+        win.any_order = any_order && col0 == 0 && ncols == T;
+        return kirchhoff_impl(data, out, S, T, dist_m, tt_s, grad_coef, vel_s, nearfield, x_begin, x_end, workspace,
+                              ws_bytes, stream, nullptr, nullptr, &win);
+    }
+    IMPDAR_CHECK_ARG(0 <= s_begin && s_begin < s_end && s_end <= S && s_end <= g_hi && g_hi <= S,
+                     "kirchhoff_window: need 0 <= s_begin < s_end <= g_hi <= snum, got [%d, %d), g_hi %d", s_begin, s_end, g_hi);
+    KirchRows rows = {s_begin, s_end, g_hi};
+    return kirchhoff_impl(data, out, S, T, dist_m, tt_s, grad_coef, vel_s, nearfield, x_begin, x_end, workspace, ws_bytes,
+                          stream, nullptr, &rows, &win);
 }
 
 int impdar_kirchhoff_window_f32(const float *data, int col0, int ncols, int ld, float *out, int ldo, int S, int T,
                                 const double *dist_m, const double *tt_s, const double *grad_coef, double vel,
                                 int nearfield, int x_begin, int x_end, int s_begin, int s_end, int g_hi, void *workspace,
                                 size_t ws_bytes, void *stream) {
-    KirchWindow win = {col0, ncols, ld, ldo};
-    if (s_begin == 0 && s_end == S && g_hi == S)   // whole image: any geometry
-        return kirchhoff_impl(data, out, S, T, dist_m, tt_s, grad_coef, vel, nearfield, x_begin, x_end, workspace,
-                              ws_bytes, stream, nullptr, nullptr, &win);
-    IMPDAR_CHECK_ARG(0 <= s_begin && s_begin < s_end && s_end <= S && s_end <= g_hi && g_hi <= S,
-                     "kirchhoff_window: need 0 <= s_begin < s_end <= g_hi <= snum, got [%d, %d), g_hi %d", s_begin, s_end, g_hi);
-    KirchRows rows = {s_begin, s_end, g_hi};
-    return kirchhoff_impl(data, out, S, T, dist_m, tt_s, grad_coef, vel, nearfield, x_begin, x_end, workspace, ws_bytes,
-                          stream, nullptr, &rows, &win);
+    const std::vector<double> vs(S > 0 ? S : 0, vel);
+    return kirchhoff_window(data, col0, ncols, ld, out, ldo, S, T, dist_m, tt_s, grad_coef, vs.data(), nearfield, x_begin,
+                            x_end, s_begin, s_end, g_hi, workspace, ws_bytes, stream, false);
+}
+
+int impdar_kirchhoff_window_vz_f32(const float *data, int col0, int ncols, int ld, float *out, int ldo, int S, int T,
+                                   const double *dist_m, const double *tt_s, const double *grad_coef, const double *vel_s,
+                                   int nearfield, int x_begin, int x_end, int s_begin, int s_end, int g_hi,
+                                   void *workspace, size_t ws_bytes, void *stream) {
+    IMPDAR_CHECK_ARG(S >= 2, "kirchhoff: need snum >= 2, tnum >= 1");
+    double vmax;
+    if (int rc = kirch_vel_range(vel_s, S, &vmax)) return rc;
+    return kirchhoff_window(data, col0, ncols, ld, out, ldo, S, T, dist_m, tt_s, grad_coef, vel_s, nearfield, x_begin,
+                            x_end, s_begin, s_end, g_hi, workspace, ws_bytes, stream, true);
+}
+
+int impdar_kirchhoff_input_window_vz(int S, int T, const double *dist_m, const double *tt_s, const double *vel_s,
+                                     int x_begin, int x_end, int *col0, int *col1) {
+    IMPDAR_CHECK_ARG(S >= 2, "kirchhoff_input_window: bad range");
+    double vmax;
+    if (int rc = kirch_vel_range(vel_s, S, &vmax)) return rc;
+    return impdar_kirchhoff_input_window(S, T, dist_m, tt_s, vmax, x_begin, x_end, col0, col1);
 }
 
 size_t impdar_kirchhoff_host_workspace_bytes(int S, int T, int nearfield) {
@@ -1121,9 +1209,9 @@ size_t impdar_kirchhoff_host_workspace_bytes(int S, int T, int nearfield) {
     return impdar_kirchhoff_workspace_bytes(S, T, nearfield) + n * (2 * sizeof(float) + sizeof(double)) + 1024;
 }
 
-int impdar_kirchhoff_host_pipelined_f64(const float *h_data, double *h_out, int S, int T, const double *dist_m,
-                                        const double *tt_s, const double *grad_coef, double vel, int nearfield,
-                                        int nchunks, void *workspace, size_t ws_bytes, void *stream) {
+static int kirchhoff_host_pipelined(const float *h_data, double *h_out, int S, int T, const double *dist_m,
+                                    const double *tt_s, const double *grad_coef, const double *vel_s, int nearfield,
+                                    int nchunks, void *workspace, size_t ws_bytes, void *stream) {
     IMPDAR_CHECK_ARG(h_data && h_out, "kirchhoff_host_pipelined: null pointer");
     IMPDAR_CHECK_ARG(S >= 2 && T >= 1, "kirchhoff: need snum >= 2, tnum >= 1");
     IMPDAR_CHECK_ARG(nchunks >= 1 && nchunks <= KP_MAX_CHUNKS, "kirchhoff_host_pipelined: nchunks must be in [1, %d]", KP_MAX_CHUNKS);
@@ -1149,7 +1237,7 @@ int impdar_kirchhoff_host_pipelined_f64(const float *h_data, double *h_out, int 
     IMPDAR_CUDA(cudaEventRecord(pipe.ev_entry, st));
     IMPDAR_CUDA(cudaStreamWaitEvent(pipe.up, pipe.ev_entry, 0));
     IMPDAR_CUDA(cudaStreamWaitEvent(pipe.down, pipe.ev_entry, 0));
-    rc = kirchhoff_impl(pipe.d_in, d_out, S, T, dist_m, tt_s, grad_coef, vel, nearfield, 0, T, w,
+    rc = kirchhoff_impl(pipe.d_in, d_out, S, T, dist_m, tt_s, grad_coef, vel_s, nearfield, 0, T, w,
                         ws_bytes - (size_t)(w - (char *)workspace), stream, &pipe);
     // ... and the caller's stream finishes after them: one synchronisation on `stream` covers the downloads
     cudaEventRecord(pipe.ev_exit, pipe.down);
@@ -1157,6 +1245,24 @@ int impdar_kirchhoff_host_pipelined_f64(const float *h_data, double *h_out, int 
     cudaEventRecord(pipe.ev_exit, pipe.up);
     cudaStreamWaitEvent(st, pipe.ev_exit, 0);
     return rc;
+}
+
+int impdar_kirchhoff_host_pipelined_f64(const float *h_data, double *h_out, int S, int T, const double *dist_m,
+                                        const double *tt_s, const double *grad_coef, double vel, int nearfield,
+                                        int nchunks, void *workspace, size_t ws_bytes, void *stream) {
+    const std::vector<double> vs(S > 0 ? S : 0, vel);
+    return kirchhoff_host_pipelined(h_data, h_out, S, T, dist_m, tt_s, grad_coef, vs.data(), nearfield, nchunks, workspace,
+                                    ws_bytes, stream);
+}
+
+int impdar_kirchhoff_host_pipelined_vz_f64(const float *h_data, double *h_out, int S, int T, const double *dist_m,
+                                           const double *tt_s, const double *grad_coef, const double *vel_s,
+                                           int nearfield, int nchunks, void *workspace, size_t ws_bytes, void *stream) {
+    IMPDAR_CHECK_ARG(S >= 2 && T >= 1, "kirchhoff: need snum >= 2, tnum >= 1");
+    double vmax;
+    if (int rc = kirch_vel_range(vel_s, S, &vmax)) return rc;
+    return kirchhoff_host_pipelined(h_data, h_out, S, T, dist_m, tt_s, grad_coef, vel_s, nearfield, nchunks, workspace,
+                                    ws_bytes, stream);
 }
 
 int impdar_kirchhoff_set_mode(int mode) {

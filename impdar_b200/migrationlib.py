@@ -81,6 +81,35 @@ def _torch_dtype(data):
 
 
 # ---------------------------------------------------------------------------------------- Kirchhoff
+# Every Kirchhoff entry below takes `vel` as a scalar (the reference's single velocity) or as a length-snum vector of
+# RMS velocities, one per output sample (rms_velocity; straight rays: row ti migrates with vel[ti] wherever the
+# reference's formula uses vel).  A scalar runs the single-velocity C entries exactly as before.
+def _kirch_vel_vector(vel, snum):
+    """None for a scalar velocity; otherwise the validated contiguous float64 per-sample vector."""
+    if np.ndim(vel) == 0:
+        return None
+    v = np.ascontiguousarray(device.host_f64(vel))
+    if v.shape != (int(snum),):
+        raise ValueError('Kirchhoff velocity vector must have one value per sample (%d), got shape %s'
+                         % (int(snum), str(v.shape)))
+    if not (np.all(np.isfinite(v)) and np.all(v > 0)):
+        raise ValueError('Kirchhoff velocity vector must be finite and positive')
+    return v
+
+
+def _kirch_window_vz(lib, win_ptr, col0, ncols, ld, out, S, T, dist_m, tt_sec, coef, v, nearfield, x_begin, x_end,
+                     rows):
+    s_begin, s_end, g_hi = (0, S, S) if rows is None else rows
+    ws = device.workspace(lib.impdar_kirchhoff_workspace_bytes(S, int(T), int(bool(nearfield))))
+    rc = lib.impdar_kirchhoff_window_vz_f32(win_ptr, int(col0), int(ncols), int(ld), device.ptr(out), int(out.stride(0)),
+                                            S, int(T), device.ptr(dist_m), device.ptr(tt_sec), device.ptr(coef),
+                                            device.ptr(v), int(bool(nearfield)), int(x_begin), int(x_end),
+                                            int(s_begin), int(s_end), int(g_hi), device.ptr(ws), ws.numel(),
+                                            device.current_stream_ptr())
+    _lib.check(rc)
+    return out
+
+
 def kirchhoff_device(data_dev, travel_time_us, dist_km, vel, nearfield, x_begin=0, x_end=None, out=None):
     """Run the Kirchhoff kernel on a (snum, tnum) float32 CUDA tensor; returns the (snum, x_end-x_begin)
     float32 block of migrated output traces (the unit of multi-GPU sharding)."""
@@ -88,6 +117,7 @@ def kirchhoff_device(data_dev, travel_time_us, dist_km, vel, nearfield, x_begin=
     lib = _lib.load()
     S, T = data_dev.shape
     x_end = T if x_end is None else x_end
+    v = _kirch_vel_vector(vel, S)
     tt_sec = device.host_f64(travel_time_us) / 1.0e6                     # mig_python.py:98
     dist_m = np.ascontiguousarray(device.host_f64(dist_km) * 1.0e3)      # :108
     if not np.all(np.diff(tt_sec) > 0):
@@ -95,6 +125,9 @@ def kirchhoff_device(data_dev, travel_time_us, dist_km, vel, nearfield, x_begin=
     coef = gradient_coefficients(tt_sec)                                 # np.gradient of :93
     if out is None:
         out = torch.empty((S, x_end - x_begin), dtype=torch.float32, device=data_dev.device)
+    if v is not None:   # the whole-image window: any trace order, like impdar_kirchhoff_f32
+        return _kirch_window_vz(lib, device.ptr(data_dev), 0, T, T, out, S, T, dist_m, tt_sec, coef, v, nearfield,
+                                x_begin, x_end, None)
     nbytes = lib.impdar_kirchhoff_workspace_bytes(S, T, int(bool(nearfield)))
     ws = device.workspace(nbytes)
     rc = lib.impdar_kirchhoff_f32(device.ptr(data_dev), device.ptr(out), S, T, device.ptr(dist_m),
@@ -112,9 +145,13 @@ def kirchhoff_rows_device(data_dev, travel_time_us, dist_km, vel, nearfield, x_b
     ValueError for irregular trace spacing (use kirchhoff_device)."""
     lib = _lib.load()
     S, T = data_dev.shape
+    v = _kirch_vel_vector(vel, S)
     tt_sec = device.host_f64(travel_time_us) / 1.0e6
     dist_m = np.ascontiguousarray(device.host_f64(dist_km) * 1.0e3)
     coef = gradient_coefficients(tt_sec)
+    if v is not None:
+        return _kirch_window_vz(lib, device.ptr(data_dev), 0, T, T, out, S, T, dist_m, tt_sec, coef, v, nearfield,
+                                x_begin, x_end, (s_begin, s_end, g_hi))
     ws = device.workspace(lib.impdar_kirchhoff_workspace_bytes(S, T, int(bool(nearfield))))
     rc = lib.impdar_kirchhoff_rows_f32(device.ptr(data_dev), device.ptr(out), S, T, device.ptr(dist_m),
                                        device.ptr(tt_sec), device.ptr(coef), float(vel), int(bool(nearfield)),
@@ -131,6 +168,12 @@ def kirchhoff_input_window(snum, travel_time_us, dist_km, vel, x_begin, x_end):
     tt_sec = device.host_f64(travel_time_us) / 1.0e6
     dist_m = np.ascontiguousarray(device.host_f64(dist_km) * 1.0e3)
     c0, c1 = ctypes.c_int(0), ctypes.c_int(0)
+    v = _kirch_vel_vector(vel, snum)
+    if v is not None:
+        _lib.check(lib.impdar_kirchhoff_input_window_vz(int(snum), len(dist_m), device.ptr(dist_m), device.ptr(tt_sec),
+                                                        device.ptr(v), int(x_begin), int(x_end), ctypes.byref(c0),
+                                                        ctypes.byref(c1)))
+        return c0.value, c1.value
     _lib.check(lib.impdar_kirchhoff_input_window(int(snum), len(dist_m), device.ptr(dist_m), device.ptr(tt_sec), float(vel),
                                                  int(x_begin), int(x_end), ctypes.byref(c0), ctypes.byref(c1)))
     return c0.value, c1.value
@@ -156,6 +199,10 @@ def kirchhoff_window_device(win_dev, col0, tnum, travel_time_us, dist_km, vel, n
     if out is None:
         out = torch.empty((S, x_end - x_begin), dtype=torch.float32, device=win_dev.device)
     assert out.stride(1) == 1 and out.shape == (S, x_end - x_begin)
+    v = _kirch_vel_vector(vel, S)
+    if v is not None:
+        return _kirch_window_vz(lib, device.ptr(win_dev), col0, ncols, win_dev.stride(0), out, S, tnum, dist_m, tt_sec,
+                                coef, v, nearfield, x_begin, x_end, rows)
     s_begin, s_end, g_hi = (0, S, S) if rows is None else rows
     ws = device.workspace(lib.impdar_kirchhoff_workspace_bytes(S, int(tnum), int(bool(nearfield))))
     rc = lib.impdar_kirchhoff_window_f32(device.ptr(win_dev), int(col0), int(ncols), int(win_dev.stride(0)),
@@ -177,6 +224,7 @@ def kirchhoff_host(data, travel_time_us, dist_km, vel, nearfield, nchunks=None):
     if a.dtype != np.float32 or not a.flags.c_contiguous:
         a = np.ascontiguousarray(a, dtype=np.float32)         # the device path computes in float32
     S, T = a.shape
+    v = _kirch_vel_vector(vel, S)
     tt_sec = device.host_f64(travel_time_us) / 1.0e6
     dist_m = np.ascontiguousarray(device.host_f64(dist_km) * 1.0e3)
     if not np.all(np.diff(tt_sec) > 0):
@@ -186,9 +234,16 @@ def kirchhoff_host(data, travel_time_us, dist_km, vel, nearfield, nchunks=None):
         nchunks = 8 if S * T >= (1 << 20) and S >= 64 else 1
     host_out = torch.empty((S, T), dtype=torch.float64, pin_memory=True)
     ws = device.workspace(lib.impdar_kirchhoff_host_workspace_bytes(S, T, int(bool(nearfield))))
-    rc = lib.impdar_kirchhoff_host_pipelined_f64(device.ptr(a), device.ptr(host_out), S, T, device.ptr(dist_m),
-                                                 device.ptr(tt_sec), device.ptr(coef), float(vel), int(bool(nearfield)),
-                                                 int(nchunks), device.ptr(ws), ws.numel(), device.current_stream_ptr())
+    if v is None:
+        rc = lib.impdar_kirchhoff_host_pipelined_f64(device.ptr(a), device.ptr(host_out), S, T, device.ptr(dist_m),
+                                                     device.ptr(tt_sec), device.ptr(coef), float(vel),
+                                                     int(bool(nearfield)), int(nchunks), device.ptr(ws), ws.numel(),
+                                                     device.current_stream_ptr())
+    else:
+        rc = lib.impdar_kirchhoff_host_pipelined_vz_f64(device.ptr(a), device.ptr(host_out), S, T, device.ptr(dist_m),
+                                                        device.ptr(tt_sec), device.ptr(coef), device.ptr(v),
+                                                        int(bool(nearfield)), int(nchunks), device.ptr(ws), ws.numel(),
+                                                        device.current_stream_ptr())
     torch.cuda.current_stream().synchronize()                 # `a` and the vectors stay alive until here
     _lib.check(rc)
     return host_out.numpy()
@@ -205,6 +260,57 @@ def migrationKirchhoff(dat, vel=1.69e8, nearfield=False):
         dat.data = out if out.dtype == in_dt or not in_dt.is_floating_point else out.to(in_dt)
     else:
         dat.data = kirchhoff_host(dat.data, dat.travel_time, dat.dist, vel, nearfield)
+    print('Kirchhoff Migration of %.0fx%.0f matrix complete in %.2f seconds'
+          % (dat.snum, dat.tnum, time.time() - start))
+    return dat
+
+
+def rms_velocity(travel_time_us, vmig):
+    """RMS velocity per sample from the interval velocity `vmig` (getVelocityProfile's (v, z) result) against two-way
+    time: v[i] = sqrt(I[i] / t[i]) with I the trapezoid integral of vmig^2 dt from the first sample at t >= 0 (whose
+    own term is vmig^2 t), summed sequentially in float64; samples with t <= 0 (pre-trigger, time zero) keep vmig."""
+    t = np.asarray(travel_time_us, dtype=np.float64) / 1.0e6
+    vm = np.asarray(vmig, dtype=np.float64)
+    if vm.shape != t.shape:
+        raise ValueError('vmig must have one value per sample (%d), got shape %s' % (len(t), str(vm.shape)))
+    v = vm.copy()
+    nonneg = np.nonzero(t >= 0)[0]
+    if len(nonneg):
+        j0 = nonneg[0]
+        v2 = vm[j0:] ** 2
+        steps = (v2[1:] + v2[:-1]) / 2. * np.diff(t[j0:])
+        integral = np.cumsum(np.concatenate([[v2[0] * t[j0]], steps]))   # sequential, left to right
+        pos = t[j0:] > 0
+        v[j0:][pos] = np.sqrt(integral[pos] / t[j0:][pos])
+    return v
+
+
+def migrationKirchhoffLayered(dat, vel=1.69e8, vel_fn=None, nearfield=False, **genfromtxt_kwargs):
+    """Kirchhoff migration with a depth-varying velocity: `vel` (or the file `vel_fn`, loaded like
+    migrationPhaseShift does) is a scalar or a (v, z) table; the table becomes the interval velocity per sample
+    (getVelocityProfile) and then the RMS velocity per sample (rms_velocity), and output sample ti migrates with its
+    own v[ti] along straight rays.  A scalar is exactly migrationKirchhoff.  dat.data becomes float64 on the host
+    lane, a tensor on the device lane.  A lateral (v, z, x) table raises ValueError."""
+    if vel_fn is not None:
+        try:
+            vel = np.genfromtxt(vel_fn, **genfromtxt_kwargs)
+            print('Velocities loaded from %s.' % vel_fn)
+        except Exception:
+            raise TypeError('File %s was given for input velocity array, but cannot be loaded. Please reformat to txt file.' % vel_fn)
+    if np.ndim(vel) == 0:
+        return migrationKirchhoff(dat, vel=vel, nearfield=nearfield)
+    if len(np.shape(vel)) == 2 and np.shape(vel)[1] == 3:
+        raise ValueError('Kirchhoff migration takes a (v, z) velocity table; lateral (v, z, x) tables are not supported')
+    print('Kirchhoff Migration (diffraction summation, layered velocity) of %.0fx%.0f matrix' % (dat.snum, dat.tnum))
+    _check_data_shape(dat)
+    start = time.time()
+    v = rms_velocity(dat.travel_time, getVelocityProfile(dat, np.asarray(vel, dtype=np.float64)))
+    if device.is_device_array(dat.data):
+        in_dt = dat.data.dtype
+        out = kirchhoff_device(device.to_device(dat.data), dat.travel_time, dat.dist, v, nearfield)
+        dat.data = out if out.dtype == in_dt or not in_dt.is_floating_point else out.to(in_dt)
+    else:
+        dat.data = kirchhoff_host(dat.data, dat.travel_time, dat.dist, v, nearfield)
     print('Kirchhoff Migration of %.0fx%.0f matrix complete in %.2f seconds'
           % (dat.snum, dat.tnum, time.time() - start))
     return dat

@@ -40,14 +40,16 @@ def kirchhoff_trace_cost(travel_time_us, dist_km, vel, n_depths=32, n_traces=204
 
     The count is a smooth (piecewise linear) function of the trace position, so for monotone trace positions it is
     evaluated at `n_traces` evenly spaced traces and interpolated: O(n_depths * n_traces * log tnum) host work,
-    well under a millisecond, instead of a searchsorted over every trace per depth."""
+    well under a millisecond, instead of a searchsorted over every trace per depth.  `vel`: a scalar or one RMS
+    velocity per sample."""
     tt = np.asarray(travel_time_us, dtype=np.float64) / 1e6
     dist = np.asarray(dist_km, dtype=np.float64) * 1e3
     T = len(dist)
     tmax = tt.max()
-    zs = vel * tt / 2.0
+    v = np.broadcast_to(np.asarray(vel, dtype=np.float64), tt.shape)
+    zs = v * tt / 2.0
     idx = np.unique(np.linspace(0, len(tt) - 1, min(n_depths, len(tt))).astype(int))
-    a2 = (vel * tmax / 2.0) ** 2 - zs[idx] ** 2
+    a2 = (v[idx] * tmax / 2.0) ** 2 - zs[idx] ** 2
     a = np.sqrt(a2[a2 >= 0])
     if T < 2 or not np.all(np.diff(dist) >= 0):
         return np.full(T, float(len(a) * T) + 1.0)
@@ -70,7 +72,8 @@ def kirchhoff_output_ranges(tnum, world, travel_time_us, dist_km, vel, align=8):
     boundaries aligned to the kernel's 8-trace CTA tile."""
     tt = np.ascontiguousarray(travel_time_us, dtype=np.float64)
     dk = np.ascontiguousarray(dist_km, dtype=np.float64)
-    key = (int(tnum), int(world), float(vel), int(align), hash(tt.tobytes()), hash(dk.tobytes()))
+    vkey = float(vel) if np.ndim(vel) == 0 else hash(np.ascontiguousarray(vel, dtype=np.float64).tobytes())
+    key = (int(tnum), int(world), vkey, int(align), hash(tt.tobytes()), hash(dk.tobytes()))
     hit = _range_cache.get(key)
     if hit is not None:
         return list(hit)
@@ -616,7 +619,8 @@ def _side_stream(dev):
 
 def _spacing_is_uniform(travel_time_us, dist_km, vel):
     """The table path's own criterion (csrc/kirchhoff.cu: uniform_ok), evaluated on the host from vectors every rank
-    has, so that all ranks take the same branch before any collective is issued."""
+    has, so that all ranks take the same branch before any collective is issued.  A per-sample velocity enters through
+    its smallest value, as in the kernel."""
     tt = np.asarray(travel_time_us, dtype=np.float64) / 1e6
     d = np.asarray(dist_km, dtype=np.float64) * 1e3
     T, S = len(d), len(tt)
@@ -628,7 +632,7 @@ def _spacing_is_uniform(travel_time_us, dist_km, vel):
         return False
     dev = np.max(np.abs(d - (d[0] + np.arange(T) * dxm)))
     dt_eff = (tt[-1] - tt[0]) / (S - 1)
-    eps_t = (2.0 / vel) * (2.0 * dev) + 1e-15 * (abs(tmax) + abs(tt[0]))
+    eps_t = (2.0 / float(np.min(vel))) * (2.0 * dev) + 1e-15 * (abs(tmax) + abs(tt[0]))
     return bool(eps_t / dt_eff < 1e-5)
 
 
@@ -638,6 +642,7 @@ def kirchhoff_sharded_device(x, travel_time_us, dist_km, vel, nearfield, rank=No
     """Kirchhoff migration of one radargram over all ranks of the process group.
 
     x : (snum, tnum) float32 tensor on this rank's device; only rank `src`'s content matters.
+    vel : a scalar, or one RMS velocity per sample (length snum, see migrationlib.rms_velocity).
     exchange = 'halo' (default with gather in ('src', False)): every rank receives only the input columns its output
         range can read, and the output blocks go to rank `src` only (gather='src': returns the image there, None
         elsewhere) or stay put (gather=False: returns (block, range)).  `x` is not written on the other ranks.

@@ -179,6 +179,21 @@ size_t impdar_kirchhoff_host_workspace_bytes(int snum, int tnum, int nearfield);
 int impdar_kirchhoff_host_pipelined_f64(const float *h_data, double *h_out, int snum, int tnum, const double *dist_m,
                                         const double *tt_s, const double *grad_coef, double vel, int nearfield,
                                         int nchunks, void *workspace, size_t workspace_bytes, void *stream);
+/* Depth-varying velocity: the _vz forms take vel_s, HOST, snum doubles - the RMS velocity of each output row (straight
+ * rays; row ti migrates with v[ti] wherever the scalar forms use vel).  Each must be finite and > 0 (status 1
+ * otherwise).  A constant vector gives bit for bit the scalar form's result.  impdar_kirchhoff_window_vz_f32 with
+ * (col0, ncols) = (0, tnum) and rows (0, snum, snum) is the whole-image call, for any trace order, like
+ * impdar_kirchhoff_f32; otherwise it is the column-window / row-chunk form above.                                  */
+int impdar_kirchhoff_window_vz_f32(const float *data, int col0, int ncols, int ld, float *out, int ldo, int snum,
+                                   int tnum, const double *dist_m, const double *tt_s, const double *grad_coef,
+                                   const double *vel_s, int nearfield, int x_begin, int x_end, int s_begin, int s_end,
+                                   int g_hi, void *workspace, size_t workspace_bytes, void *stream);
+int impdar_kirchhoff_input_window_vz(int snum, int tnum, const double *dist_m, const double *tt_s, const double *vel_s,
+                                     int x_begin, int x_end, int *col0, int *col1);
+int impdar_kirchhoff_host_pipelined_vz_f64(const float *h_data, double *h_out, int snum, int tnum,
+                                           const double *dist_m, const double *tt_s, const double *grad_coef,
+                                           const double *vel_s, int nearfield, int nchunks, void *workspace,
+                                           size_t workspace_bytes, void *stream);
 /* Counters of the last impdar_kirchhoff_f32 call (for the roofline): (output sample, input trace) pairs
  * inside the aperture and pairs that took the float64 exact path.  Counting pairs costs an instruction
  * per pair, so it is off unless enabled.  last_stats synchronises the stream of that call.            */

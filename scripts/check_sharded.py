@@ -1,7 +1,8 @@
 """torchrun check of the multi-GPU Kirchhoff on real GPUs: the sharded result (halo exchange: every rank receives only
 its window of input columns; output blocks gathered to rank 0; exchanges overlapped with the kernels in bottom-up row
 chunks) must equal, BIT FOR BIT, the unsharded image that rank 0 computes alone, for every pipeline depth, and so must
-the round-1 scheme (full broadcast + all-gather).  Prints the timings of both schemes.
+the round-1 scheme (full broadcast + all-gather).  Prints the timings of both schemes.  Finally repeats the bit-for-bit
+checks with a layered velocity (synthetic.layered_velocity as per-sample RMS velocities).
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 scripts/check_sharded.py [S T]"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -89,5 +90,21 @@ for chunks in (1, parallel.DEFAULT_CHUNKS):
     dist.all_reduce(ok, op=dist.ReduceOp.MIN)
     if rank == 0:
         print("exchange=halo pipeline_chunks=%s, next radargram through the same image: bit for bit: %s" % (chunks, ok.item() == 1.0), flush=True)
+# layered velocity: one RMS velocity per sample, passed through every layer (ranges, windows, kernels)
+from impdar_b200 import RadarData
+geo = RadarData(np.zeros((S, 1), np.float32), dt=synthetic.DT, travel_time=tt, dist=dk[:1])
+VEL = ml.rms_velocity(tt, ml.getVelocityProfile(geo, synthetic.layered_velocity(tt)))
+if rank == 0:
+    whole = ml.kirchhoff_device(full, tt, dk, VEL, False)
+    print("layered velocity %.3e .. %.3e; single-GPU kernel: %s" % (VEL.max(), VEL.min(), ml.kirchhoff_last_kernel()),
+          flush=True)
+for exchange, chunks in VARIANTS:
+    got = run(exchange, chunks)
+    ok = torch.tensor([1.0 if (rank != 0 or torch.equal(got, whole)) else 0.0], device="cuda")
+    if exchange == "broadcast" and rank != 0:
+        ok[0] = 1.0 if got.shape == (S, T) else 0.0
+    dist.all_reduce(ok, op=dist.ReduceOp.MIN)
+    if rank == 0:
+        print("layered: exchange=%s pipeline_chunks=%s: sharded == unsharded bit for bit: %s" % (exchange, chunks, ok.item() == 1.0), flush=True)
 parallel.free_exchange_buffers()
 dist.destroy_process_group()
