@@ -10,7 +10,8 @@ from . import migrationlib, filtering, processing, process  # noqa: F401  (proce
 from .radardata import RadarData, RadarFlags  # noqa: F401
 from .matio import load_mat  # noqa: F401  (StoDeep / ImpDAR .mat files, SURVEY.md 8f rank 4)
 from .migrationlib import (migrationKirchhoff, migrationStolt, migrationPhaseShift,  # noqa: F401
-                           migrationTimeWavenumber, getVelocityProfile, migrationKirchhoffLayered, rms_velocity)
+                           migrationTimeWavenumber, getVelocityProfile, migrationKirchhoffLayered, rms_velocity,
+                           migrationKirchhoffLateral)
 
 __version__ = "0.1.0"
 

@@ -63,6 +63,9 @@ PROTOTYPES = {
     "impdar_kirchhoff_input_window_vz": (_c_int, [_c_int, _c_int, _vp, _vp, _vp, _c_int, _c_int, _vp, _vp]),
     "impdar_kirchhoff_host_pipelined_vz_f64": (_c_int, [_vp, _vp, _c_int, _c_int, _vp, _vp, _vp, _vp, _c_int, _c_int,
                                                         _vp, _c_sz, _vp]),
+    "impdar_kirchhoff_lateral_workspace_bytes": (_c_sz, [_c_int, _c_int, _c_int, _c_int]),
+    "impdar_kirchhoff_window_vxz_f32": (_c_int, [_vp, _c_int, _c_int, _c_int, _vp, _c_int, _c_int, _c_int, _vp, _vp,
+                                                 _vp, _vp, _c_int, _vp, _c_int, _c_int, _c_int, _vp, _c_sz, _vp]),
     "impdar_kirchhoff_enable_stats": (_c_int, [_c_int]),
     "impdar_kirchhoff_last_stats": (_c_int, [_vp, _vp]),
     "impdar_kirchhoff_set_mode": (_c_int, [_c_int]),

@@ -20,6 +20,8 @@
 //     float64 predicate over the ascending trace positions), so the inner loop only tests a trace range.
 //   * the velocity is one RMS value per output sample, v[ti] (a constant vector is the reference's single vel):
 //     every formula above uses v[ti] for the pairs of output row ti.
+//   * lateral variant (LAT): V[ti, xi], one of P RMS profiles per output trace (colp[xi]); the warp of trace xi reads
+//     its profile's row vectors and its profile's cs / thr, so column xi is the single-profile call bit for bit.
 #include <math.h>
 
 #include <cmath>
@@ -49,6 +51,8 @@ struct KirchParams {
     float neg_u0, thr;                     // thr = 0.5 - delta; -1 (every pair exact) for non-monotone positions
     int monotone;                       // dist ascending -> per-sample aperture by binary search
     int rowmajor, Tp, Apad;             // table path: gradT/dataT are (S, Tp) row-major, trace x at column Apad + x
+    const int *colp;                    // lateral: profile of each output trace (T); zs, zs2, vs, rowc are then (P, S)
+    const double2 *pc;                  // lateral: {cs, thr} of each profile
 };
 
 #define KIRCH_MAGIC 12582912.0f  // 1.5 * 2^23
@@ -84,15 +88,16 @@ __device__ __forceinline__ int exact_pick(const double *__restrict__ tt, int S, 
     return k;
 }
 
+// roff: offset of the output row's profile in the (P, S) row vectors of the lateral variant (0 otherwise)
 template <bool NEAR>
-__device__ __forceinline__ float exact_term(const KirchParams &p, int ti, int x, double dxi) {
+__device__ __forceinline__ float exact_term(const KirchParams &p, int ti, int x, double dxi, size_t roff = 0) {
     const double d = __dsub_rn(p.dist[x], dxi);
     double rs;
-    const double vel = p.vs[ti];
-    const double t = exact_time(d, p.zs2[ti], vel, rs);
+    const double vel = (p.vs + roff)[ti];
+    const double t = exact_time(d, (p.zs2 + roff)[ti], vel, rs);
     if (t > p.tmax) return 0.f;
     const int k = exact_pick(p.tt, p.S, t, p.tt0, p.inv_dt);
-    const double costheta = p.zs[ti] / rs;
+    const double costheta = (p.zs + roff)[ti] / rs;
     const size_t gi = p.rowmajor ? (size_t)k * p.Tp + p.Apad + x : (size_t)x * p.SP + k;
     const double g = (double)p.gradT[gi];
     double term = g * costheta / vel;
@@ -107,8 +112,18 @@ __device__ __forceinline__ float exact_term(const KirchParams &p, int ti, int x,
 
 #define KQ_CAP 192
 
+// The lateral variant keeps its per-warp profile values in the warp's c2v staging row, after the 32 staged values:
+// [32] the fast/exact threshold, [33] the profile index, [34..35] cs (float64).  They are re-read where they are used
+// (thr once per group of 4 traces): kept in registers across the trace loop they push the kernel past 64 registers.
+constexpr int KL_THR = 32, KL_PROF = 33, KL_CS = 34, KL_ROW = 36;
+template <bool LAT>
+__device__ __forceinline__ double kirch_cs(const KirchParams &p, const float *sCw) {
+    if constexpr (LAT) return *reinterpret_cast<const volatile double *>(sCw + KL_CS);
+    else return p.cs;
+}
+
 // Fast path over one staged chunk of <= 32 input traces (4 per iteration, straight-line, predicated).
-template <bool NEAR, bool STATS, bool HASNAN, typename Flush>
+template <bool NEAR, bool STATS, bool HASNAN, bool LAT, typename Flush>
 __device__ __forceinline__ void kirch_chunk(Flush &flush, const float *__restrict__ gT, const float *__restrict__ dT,
                                             const float *__restrict__ sCw, int *__restrict__ sQw, int jend,
                                             unsigned rowoff, unsigned SP, unsigned kmax, int rel, unsigned span,
@@ -116,6 +131,7 @@ __device__ __forceinline__ void kirch_chunk(Flush &flush, const float *__restric
                                             float &acc0, float &acc1, int &qn, unsigned &npairs, unsigned &nexact) {
 #pragma unroll 1
     for (int j0 = 0; j0 < jend; j0 += 4) {
+        if constexpr (LAT) thr = *reinterpret_cast<const volatile float *>(sCw + KL_THR);
         const float4 c4 = *reinterpret_cast<const float4 *>(sCw + j0);
         const float c[4] = {c4.x, c4.y, c4.z, c4.w};
         unsigned amb4 = 0;
@@ -175,9 +191,9 @@ __device__ __forceinline__ void kirch_chunk(Flush &flush, const float *__restric
     }
 }
 
-template <bool NEAR, bool STATS>
+template <bool NEAR, bool STATS, bool LAT = false>
 __global__ void __launch_bounds__(256) kirch_general_kernel(const __grid_constant__ KirchParams p) {
-    __shared__ __align__(16) float sC[8][32];
+    __shared__ __align__(16) float sC[8][LAT ? KL_ROW : 32];
     __shared__ int sQ[8][KQ_CAP];
     __shared__ float sT[8][32];
     __shared__ int sO[8][32];
@@ -196,6 +212,19 @@ __global__ void __launch_bounds__(256) kirch_general_kernel(const __grid_constan
 
     if (warp_active) {
         const double dxi = p.dist[xi];
+        // lateral: this trace's profile (its row vectors start at roff); its cs / thr go to shared memory, out of the
+        // registers of the trace loop
+        const int prof = LAT ? p.colp[xi] : 0;
+        const size_t roff = LAT ? (size_t)prof * p.S : 0;
+        if constexpr (LAT) {
+            if (lane == 0) {
+                const double2 pc = p.pc[prof];
+                sC[warp][KL_THR] = (float)pc.y;
+                reinterpret_cast<int *>(sC[warp])[KL_PROF] = prof;
+                *reinterpret_cast<double *>(sC[warp] + KL_CS) = pc.x;
+            }
+            __syncwarp();
+        }
         const int tic = active ? ti : p.S - 1;
         const double Ud = p.tt[tic] * p.inv_dt;
         const float U = (float)Ud;
@@ -204,7 +233,7 @@ __global__ void __launch_bounds__(256) kirch_general_kernel(const __grid_constan
         // exact per-sample aperture [xlo, xhi]: pairs with 2r/v > max(tt) contribute exactly 0
         int xlo = xi + 1, xhi = xi;
         if (active) {
-            const double zs2i = p.zs2[ti], vi = p.vs[ti];
+            const double zs2i = (p.zs2 + roff)[ti], vi = (p.vs + roff)[ti];
             double rs;
             if (!(exact_time(0.0, zs2i, vi, rs) > p.tmax)) {
                 if (p.monotone) {
@@ -239,7 +268,7 @@ __global__ void __launch_bounds__(256) kirch_general_kernel(const __grid_constan
         }
         // Per-row velocity (kirch_prep_vectors_kernel): the staged c2v carries the offset scale cs = 2/(vmin dt) and
         // this row's C^2 is c2v * sigma; the weights are 1/(2 pi v_ti) and 4/(v_ti dt)^2/(2 pi).
-        const float3 rc = p.rowc[tic];
+        const float3 rc = (p.rowc + roff)[tic];
         const float sigma = rc.x;
         const float Uw = U * rc.y, Un = U * rc.z;
         const unsigned SP = (unsigned)p.SP;
@@ -252,7 +281,8 @@ __global__ void __launch_bounds__(256) kirch_general_kernel(const __grid_constan
                 if (base + lane < count) {
                     const int e = sQ[warp][base + lane];
                     owner = e & 31;
-                    term = exact_term<NEAR>(p, ti0 + owner, e >> 5, dxi);
+                    const size_t ro = LAT ? (size_t)reinterpret_cast<const volatile int *>(sC[warp])[KL_PROF] * p.S : 0;
+                    term = exact_term<NEAR>(p, ti0 + owner, e >> 5, dxi, ro);
                 }
                 sT[warp][lane] = term;
                 sO[warp][lane] = owner;
@@ -271,7 +301,7 @@ __global__ void __launch_bounds__(256) kirch_general_kernel(const __grid_constan
                     const int xx = xb + lane;
                     float c2v = 0.f;
                     if (xx <= xhi_w) {
-                        const double C = (p.dist[xx] - dxi) * p.cs;
+                        const double C = (p.dist[xx] - dxi) * kirch_cs<LAT>(p, sC[warp]);
                         c2v = (float)(C * C);
                     }
                     __syncwarp();
@@ -281,9 +311,9 @@ __global__ void __launch_bounds__(256) kirch_general_kernel(const __grid_constan
                 const int jend = (min(32, xhi_w - xb + 1) + 3) & ~3;   // padded entries fall outside every lane's range
                 const unsigned rowoff = (unsigned)xb * SP;
                 const int rel = xb - xlo;
-                kirch_chunk<NEAR, STATS, decltype(nan_variant)::value>(
+                kirch_chunk<NEAR, STATS, decltype(nan_variant)::value, LAT>(
                     flush, p.gradT, p.dataT, sC[warp], sQ[warp], jend, rowoff, SP, p.kmax, rel, span, xb, lane, u2, sigma, Uw,
-                    Un, p.neg_u0, p.thr, acc0, acc1, qn, npairs, nexact);
+                    Un, p.neg_u0, LAT ? 0.f : p.thr, acc0, acc1, qn, npairs, nexact);
             }
         };
         if (hasnan) trace_loop(std::true_type{}); else trace_loop(std::false_type{});
@@ -357,21 +387,35 @@ __global__ void __launch_bounds__(256) grad_transpose_kernel(const float *__rest
 // Per-row vectors: zs, zs2 (float64, the reference's operation order) and the general kernel's float32 row constants.
 // cs_i / cs = 1 exactly when v_ti is the velocity cs was made with, so a constant vector has sigma == 1 and the
 // weights are the single-velocity values bit for bit.
+__device__ __forceinline__ void kirch_prep_row(int i, const double *__restrict__ tt, const double *__restrict__ vs,
+                                               double *__restrict__ zs, double *__restrict__ zs2,
+                                               float3 *__restrict__ rowc, double dt_eff, double cs) {
+    const double v = vs[i];
+    const double z = __ddiv_rn(__dmul_rn(v, tt[i]), 2.0);   // zs = vel * tt_sec / 2.0   (:101)
+    zs[i] = z;
+    zs2[i] = __dmul_rn(z, z);                                // zs2 = zs**2.              (:102)
+    const double vdt = __dmul_rn(v, dt_eff);
+    const double sr = __ddiv_rn(__ddiv_rn(2.0, vdt), cs);   // cs_i / cs, cs_i = 2 / (v dt)
+    rowc[i] = make_float3((float)__dmul_rn(sr, sr),
+                          (float)__ddiv_rn(1.0, __dmul_rn(2.0 * 3.14159265358979323846, v)),
+                          (float)__ddiv_rn(__ddiv_rn(4.0, __dmul_rn(vdt, vdt)), 2.0 * 3.14159265358979323846));
+}
+
 __global__ void kirch_prep_vectors_kernel(const double *__restrict__ tt, const double *__restrict__ vs,
                                           double *__restrict__ zs, double *__restrict__ zs2, float3 *__restrict__ rowc,
                                           int S, double dt_eff, double cs) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < S) {
-        const double v = vs[i];
-        const double z = __ddiv_rn(__dmul_rn(v, tt[i]), 2.0);   // zs = vel * tt_sec / 2.0   (:101)
-        zs[i] = z;
-        zs2[i] = __dmul_rn(z, z);                                // zs2 = zs**2.              (:102)
-        const double vdt = __dmul_rn(v, dt_eff);
-        const double sr = __ddiv_rn(__ddiv_rn(2.0, vdt), cs);   // cs_i / cs, cs_i = 2 / (v dt)
-        rowc[i] = make_float3((float)__dmul_rn(sr, sr),
-                              (float)__ddiv_rn(1.0, __dmul_rn(2.0 * 3.14159265358979323846, v)),
-                              (float)__ddiv_rn(__ddiv_rn(4.0, __dmul_rn(vdt, vdt)), 2.0 * 3.14159265358979323846));
-    }
+    if (i < S) kirch_prep_row(i, tt, vs, zs, zs2, rowc, dt_eff, cs);
+}
+
+// The same row constants for each of P profiles (lateral variant): profile blockIdx.x, rows of block blockIdx.y, each
+// with its own cs = pc[p].x, so a profile's vectors are bit for bit those of a single-profile call.
+__global__ void kirch_prep_profiles_kernel(const double *__restrict__ tt, const double *__restrict__ vs,
+                                           double *__restrict__ zs, double *__restrict__ zs2, float3 *__restrict__ rowc,
+                                           const double2 *__restrict__ pc, int S, double dt_eff) {
+    const int i = blockIdx.y * blockDim.x + threadIdx.x;
+    const size_t o = (size_t)blockIdx.x * S;
+    if (i < S) kirch_prep_row(i, tt, vs + o, zs + o, zs2 + o, rowc + o, dt_eff, pc[blockIdx.x].x);
 }
 
 // =====================================================================================================
@@ -640,6 +684,18 @@ namespace impdar {
 
 static inline int kirch_sp(int S) { return ((S + 64 + 31) / 32) * 32; }
 
+// Per-run path of the lateral entry: folds one run's non-finite / stand-down flags and pair counters into the summary
+// block (same layout as the flags block: [0] any run left work to the gather kernel, +128 pairs, exact pairs).
+__global__ void kirch_run_summary_kernel(const int *__restrict__ flags, int *__restrict__ sum) {
+    if (threadIdx.x == 0) {
+        if (flags[0] | flags[16]) sum[0] = 1;
+        const unsigned long long *st = reinterpret_cast<const unsigned long long *>(flags + 32);
+        unsigned long long *acc = reinterpret_cast<unsigned long long *>(sum + 32);
+        acc[0] += st[0];
+        acc[1] += st[1];
+    }
+}
+
 // float32 rows -> float64 rows (the reference returns float64, mig_python.py:95/:118); runs on the download stream
 __global__ void __launch_bounds__(256) widen_f32_f64_kernel(const float *__restrict__ x, double *__restrict__ y, size_t n) {
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x)
@@ -670,6 +726,24 @@ struct KirchWindow {
     int col0, ncols, ld, ldo;
     bool any_order;
 };
+// Lateral velocity (impdar_kirchhoff_window_vxz_f32, general-kernel side): P RMS profiles (host, (P, S)), the profile of
+// each trace (host, T), each profile's smallest velocity and whether it is constant; `block` is the device area after
+// the single-profile workspace (kirch_lateral_block_bytes).
+struct KirchLateral {
+    const double *profiles;
+    int P;
+    const int *colp;
+    const double *vmin;
+    const unsigned char *vconst;
+    char *block;
+};
+static inline size_t kirch_a256(size_t v) { return (v + 255) / 256 * 256; }
+static size_t kirch_lateral_block_bytes(int S, int T, int P) {
+    const size_t ps = (size_t)P * (size_t)S;
+    // run summary (flags | stats) | {cs, thr} per profile | trace -> profile | v, zs, zs2 | float3 row constants
+    return 256 + 256 + kirch_a256((size_t)P * sizeof(double2)) + kirch_a256((size_t)T * sizeof(int)) +
+           3 * kirch_a256(ps * sizeof(double)) + kirch_a256(ps * sizeof(float3));
+}
 // Side streams and events of the host pipeline: one set per device, created on first use under a lock.  Selection
 // switches and "last call" records are per host thread (SURVEY.md 8b: one host thread - or process - per GPU).
 constexpr int KP_MAX_DEVICES = 64;
@@ -827,10 +901,40 @@ int impdar_kirchhoff_input_window(int S, int T, const double *dist_m, const doub
     return IMPDAR_B200_OK;
 }
 
+// Uniform trace spacing?  Deviation of the real positions from the fitted grid, in seconds of travel time (vmin: the
+// smallest velocity, whose travel time changes most per metre of position error).  uniform_ok admits the table path.
+struct KirchSpacing {
+    double dxm, eps_t;
+    bool uniform_ok;
+};
+static KirchSpacing kirch_spacing(int S, int T, const double *h_dist, const double *h_tt, double vmin, bool monotone) {
+    double tmax = h_tt[0];
+    for (int i = 0; i < S; ++i) tmax = fmax(tmax, h_tt[i]);
+    const double tt0 = h_tt[0];
+    const double dt_eff = (h_tt[S - 1] - h_tt[0]) / (double)(S - 1);
+    double dxm = 0.0, maxdev_d = 0.0;
+    if (T > 1) {
+        dxm = (h_dist[T - 1] - h_dist[0]) / (double)(T - 1);
+        for (int i = 0; i < T; ++i) {
+            const double dev = fabs(h_dist[i] - (h_dist[0] + i * dxm));
+            if (dev > maxdev_d) maxdev_d = dev;
+        }
+    }
+    const double eps_t = (2.0 / vmin) * (2.0 * maxdev_d) + 1e-15 * (fabs(tmax) + fabs(tt0));
+    return {dxm, eps_t, monotone && T > 1 && dxm > 0.0 && tmax > 0.0 && eps_t / dt_eff < 1e-5};
+}
+
+static bool kirch_monotone(int T, const double *h_dist) {
+    for (int i = 1; i < T; ++i)
+        if (!(h_dist[i] >= h_dist[i - 1])) return false;
+    return true;
+}
+
 static int kirchhoff_impl(const float *data, float *out, int S, int T, const double *dist_m, const double *tt_s,
                           const double *grad_coef, const double *vel_s, int nearfield, int x_begin, int x_end,
                           void *workspace, size_t ws_bytes, void *stream, const KirchPipe *pipe,
-                          const KirchRows *rows = nullptr, const KirchWindow *win = nullptr) {
+                          const KirchRows *rows = nullptr, const KirchWindow *win = nullptr,
+                          const KirchLateral *lat = nullptr) {
     IMPDAR_CHECK_ARG(data && out && dist_m && tt_s && grad_coef && vel_s, "kirchhoff: null pointer");
     IMPDAR_CHECK_ARG(S >= 2 && T >= 1, "kirchhoff: need snum >= 2, tnum >= 1");
     IMPDAR_CHECK_ARG(0 <= x_begin && x_begin < x_end && x_end <= T, "kirchhoff: bad output range [%d, %d)",
@@ -874,33 +978,27 @@ static int kirchhoff_impl(const float *data, float *out, int S, int T, const dou
         const double dev = fabs(h_tt[i] - (tt0 + i * dt_eff));
         if (dev > maxdev) maxdev = dev;
     }
-    int monotone = 1;
-    for (int i = 1; i < T; ++i)
-        if (!(h_dist[i] >= h_dist[i - 1])) { monotone = 0; break; }
+    const int monotone = kirch_monotone(T, h_dist) ? 1 : 0;
     // fp32 error budget of f = sqrt(U^2 + C^2) - U0 (sample units): ~4 ulp relative on a value <= S + |U0|,
     // plus the deviation of tt from a uniform grid.
     const double u0 = tt0 / dt_eff;
     // A per-row velocity adds one rounding: q = fmaf(c2v, sigma, u2) with sigma = (v_min / v_i)^2 rounded to float,
     // i.e. <= 2^-24 more relative error on the C^2 part of q (<= q), <= 2^-25 sqrt(q) <= 3e-8 (S + |U0|) on f after the
     // square root.  A constant vector has sigma == 1 exactly (no extra rounding) and keeps the budget above unchanged.
-    double delta = 6e-7 * ((double)S + fabs(u0) + 64.0) + 2.0 * maxdev / dt_eff + 1e-6;
-    if (!vconst) delta += 6e-8 * ((double)S + fabs(u0) + 64.0);
-    float thr = (float)(0.5 - delta);
-    if (delta > 0.2) thr = -1.f;  // irregular sampling: everything through the exact path
+    const double delta0 = 6e-7 * ((double)S + fabs(u0) + 64.0) + 2.0 * maxdev / dt_eff + 1e-6;
+    const double delta_vz = 6e-8 * ((double)S + fabs(u0) + 64.0);   // non-constant velocity only
+    auto fast_thr = [&](bool constant_velocity) {
+        const double delta = constant_velocity ? delta0 : delta0 + delta_vz;
+        return delta > 0.2 ? -1.f : (float)(0.5 - delta);   // irregular sampling: everything through the exact path
+    };
+    const float thr = fast_thr(vconst);
 
-    // uniform trace spacing?  (deviation of the real positions from the fitted grid, in seconds of travel time)
-    double dxm = 0.0, maxdev_d = 0.0;
-    if (T > 1) {
-        dxm = (h_dist[T - 1] - h_dist[0]) / (double)(T - 1);
-        for (int i = 0; i < T; ++i) {
-            const double dev = fabs(h_dist[i] - (h_dist[0] + i * dxm));
-            if (dev > maxdev_d) maxdev_d = dev;
-        }
-    }
-    const double eps_t = (2.0 / vmin) * (2.0 * maxdev_d) + 1e-15 * (fabs(tmax) + fabs(tt0));
-    const bool uniform_ok = monotone && T > 1 && dxm > 0.0 && tmax > 0.0 && eps_t / dt_eff < 1e-5;
-    IMPDAR_CHECK_ARG(!(g_kirch_mode >= 2 && !uniform_ok), "kirchhoff: table path forced but trace spacing is not uniform");
-    const bool use_table = (g_kirch_mode >= 2) || (g_kirch_mode == 0 && uniform_ok);
+    const KirchSpacing spacing = kirch_spacing(S, T, h_dist, h_tt, vmin, monotone);
+    const double dxm = spacing.dxm, eps_t = spacing.eps_t;
+    const bool uniform_ok = spacing.uniform_ok;
+    IMPDAR_CHECK_ARG(lat || !(g_kirch_mode >= 2 && !uniform_ok),
+                     "kirchhoff: table path forced but trace spacing is not uniform");
+    const bool use_table = !lat && ((g_kirch_mode >= 2) || (g_kirch_mode == 0 && uniform_ok));
     IMPDAR_CHECK_ARG(!(win && !monotone && !win->any_order), "kirchhoff_window: trace positions must be ascending");
 
     // carve workspace: small vectors first
@@ -930,8 +1028,10 @@ static int kirchhoff_impl(const float *data, float *out, int S, int T, const dou
         int rcv = kirch_stage_vectors(tt_s, grad_coef, vel_s, dist_m, S, T, d_tt, st);
         if (rcv) return rcv;
         IMPDAR_CUDA(cudaMemsetAsync(flags, 0, 256, st));
-        kirch_prep_vectors_kernel<<<(S + 255) / 256, 256, 0, st>>>(d_tt, d_vel, zs, zs2, rowc, S, dt_eff, 2.0 / (vmin * dt_eff));
-        IMPDAR_LAUNCH_CHECK();
+        if (!lat) {
+            kirch_prep_vectors_kernel<<<(S + 255) / 256, 256, 0, st>>>(d_tt, d_vel, zs, zs2, rowc, S, dt_eff, 2.0 / (vmin * dt_eff));
+            IMPDAR_LAUNCH_CHECK();
+        }
     }
 
     KirchParams p;
@@ -943,6 +1043,36 @@ static int kirchhoff_impl(const float *data, float *out, int S, int T, const dou
     p.neg_u0 = (float)(-u0); p.thr = monotone ? thr : -1.f;   // non-monotone positions: every pair takes the exact path
     p.monotone = monotone;
     int path = 1;
+
+    if (lat) {
+        // Per profile: cs and thr exactly as a single-profile call with that profile computes them, then its row
+        // vectors (kirch_prep_row): column xi of the lateral kernel is that call's column xi.
+        const int P = lat->P;
+        std::vector<double2> pc(P);
+        for (int q = 0; q < P; ++q)
+            pc[q] = make_double2(2.0 / (lat->vmin[q] * dt_eff), monotone ? (double)fast_thr(lat->vconst[q] != 0) : -1.0);
+        char *b = lat->block + 256;   // [0, 256): run summary of the per-run path
+        double2 *d_pc = (double2 *)b;
+        b += kirch_a256((size_t)P * sizeof(double2));
+        int *d_colp = (int *)b;
+        b += kirch_a256((size_t)T * sizeof(int));
+        const size_t ps = (size_t)P * S;
+        double *l_vs = (double *)b;
+        b += kirch_a256(ps * sizeof(double));
+        double *l_zs = (double *)b;
+        b += kirch_a256(ps * sizeof(double));
+        double *l_zs2 = (double *)b;
+        b += kirch_a256(ps * sizeof(double));
+        float3 *l_rowc = (float3 *)b;
+        // pageable sources: each copy returns once its source has been staged, so the host vectors may go
+        IMPDAR_CUDA(cudaMemcpyAsync(d_pc, pc.data(), (size_t)P * sizeof(double2), cudaMemcpyHostToDevice, st));
+        IMPDAR_CUDA(cudaMemcpyAsync(d_colp, lat->colp, (size_t)T * sizeof(int), cudaMemcpyHostToDevice, st));
+        IMPDAR_CUDA(cudaMemcpyAsync(l_vs, lat->profiles, ps * sizeof(double), cudaMemcpyHostToDevice, st));
+        kirch_prep_profiles_kernel<<<dim3(P, (S + 255) / 256), 256, 0, st>>>(d_tt, l_vs, l_zs, l_zs2, l_rowc, d_pc, S, dt_eff);
+        IMPDAR_LAUNCH_CHECK();
+        p.vs = l_vs; p.zs = l_zs; p.zs2 = l_zs2; p.rowc = l_rowc; p.colp = d_colp; p.pc = d_pc;
+        path = 4;
+    }
 
     if (use_table) {
         const int Amax = kirch_amax(T, vmax, tmax, dxm);
@@ -1117,7 +1247,17 @@ static int kirchhoff_impl(const float *data, float *out, int S, int T, const dou
         p.gradT = gradT - (size_t)c0 * SP; p.dataT = dataT ? dataT - (size_t)c0 * SP : nullptr; p.SP = SP;
         p.kmax = (unsigned)SP - 1u;
         dim3 grid((S + 31) / 32, (x_end - x_begin + 7) / 8), block(32, 8);
-        if (g_stats_enabled) {
+        if (lat) {
+            ktimer_begin("kirch_general_lateral_kernel", st);
+            if (nearfield) {
+                if (g_stats_enabled) kirch_general_kernel<true, true, true><<<grid, block, 0, st>>>(p);
+                else kirch_general_kernel<true, false, true><<<grid, block, 0, st>>>(p);
+            } else {
+                if (g_stats_enabled) kirch_general_kernel<false, true, true><<<grid, block, 0, st>>>(p);
+                else kirch_general_kernel<false, false, true><<<grid, block, 0, st>>>(p);
+            }
+            ktimer_end(st);
+        } else if (g_stats_enabled) {
             if (nearfield) { ktimer_begin("kirch_general_kernel", st); kirch_general_kernel<true, true><<<grid, block, 0, st>>>(p); ktimer_end(st); }
             else { ktimer_begin("kirch_general_kernel", st); kirch_general_kernel<false, true><<<grid, block, 0, st>>>(p); ktimer_end(st); }
         } else {
@@ -1263,6 +1403,101 @@ int impdar_kirchhoff_host_pipelined_vz_f64(const float *h_data, double *h_out, i
     if (int rc = kirch_vel_range(vel_s, S, &vmax)) return rc;
     return kirchhoff_host_pipelined(h_data, h_out, S, T, dist_m, tt_s, grad_coef, vel_s, nearfield, nchunks, workspace,
                                     ws_bytes, stream);
+}
+
+size_t impdar_kirchhoff_lateral_workspace_bytes(int S, int T, int P, int nearfield) {
+    if (S < 2 || T < 1 || P < 1) return 0;
+    return impdar_kirchhoff_workspace_bytes(S, T, nearfield) + kirch_lateral_block_bytes(S, T, P);
+}
+
+// Lateral velocity: output trace xi migrates with profile col_profile[xi] of `profiles` (P x S RMS velocities).  Path:
+// with uniform spacing and runs (maximal ranges of traces with one profile) at least KIRCH_RUN_MIN traces wide on
+// average over the whole profile, one single-profile table / tile call per run of [x_begin, x_end) on its own input
+// sub-window; otherwise the lateral general kernel in one launch.  KIRCHHOFF_GENERAL forces the kernel, the table modes
+// force the runs.
+constexpr int KIRCH_RUN_MIN = 192;
+
+int impdar_kirchhoff_window_vxz_f32(const float *data, int col0, int ncols, int ld, float *out, int ldo, int S, int T,
+                                    const double *dist_m, const double *tt_s, const double *grad_coef,
+                                    const double *profiles, int P, const int *col_profile, int nearfield, int x_begin,
+                                    int x_end, void *workspace, size_t ws_bytes, void *stream) {
+    IMPDAR_CHECK_ARG(data && out && dist_m && tt_s && grad_coef && profiles && col_profile, "kirchhoff_vxz: null pointer");
+    IMPDAR_CHECK_ARG(S >= 2 && T >= 1 && P >= 1, "kirchhoff_vxz: need snum >= 2, tnum >= 1, nprof >= 1");
+    IMPDAR_CHECK_ARG(T < (1 << 26), "kirchhoff: tnum too large");
+    IMPDAR_CHECK_ARG(0 <= x_begin && x_begin < x_end && x_end <= T, "kirchhoff: bad output range [%d, %d)", x_begin, x_end);
+    const size_t base = impdar_kirchhoff_workspace_bytes(S, T, nearfield);
+    const size_t need = impdar_kirchhoff_lateral_workspace_bytes(S, T, P, nearfield);
+    IMPDAR_CHECK_ARG(workspace && ws_bytes >= need, "kirchhoff_vxz: workspace too small (%zu < %zu)", ws_bytes, need);
+    std::vector<double> vmin(P), vmax(P), vrow(S, 0.0);   // vrow: largest velocity of each row (the reach of a pair)
+    std::vector<unsigned char> vconst(P);
+    for (int q = 0; q < P; ++q) {
+        const double *v = profiles + (size_t)q * S;
+        double lo = v[0], hi = v[0];
+        for (int i = 0; i < S; ++i) {
+            IMPDAR_CHECK_ARG(std::isfinite(v[i]) && v[i] > 0.0,
+                             "kirchhoff_vxz: profile %d velocity[%d] = %g must be finite and positive", q, i, v[i]);
+            lo = fmin(lo, v[i]);
+            hi = fmax(hi, v[i]);
+            vrow[i] = fmax(vrow[i], v[i]);
+        }
+        vmin[q] = lo;
+        vmax[q] = hi;
+        vconst[q] = lo == hi;
+    }
+    for (int x = 0; x < T; ++x)
+        IMPDAR_CHECK_ARG(col_profile[x] >= 0 && col_profile[x] < P, "kirchhoff_vxz: col_profile[%d] = %d outside [0, %d)",
+                         x, col_profile[x], P);
+    // The path depends on the whole trace -> profile map (not on [x_begin, x_end) or the window), so sub-ranges and
+    // windows take the whole image's path.
+    long long runs_all = 1;
+    for (int x = 1; x < T; ++x) runs_all += col_profile[x] != col_profile[x - 1];
+    std::vector<int> run0;   // first output trace of each run of [x_begin, x_end)
+    for (int x = x_begin; x < x_end; ++x)
+        if (x == x_begin || col_profile[x] != col_profile[x - 1]) run0.push_back(x);
+    const int nruns = (int)run0.size();
+    run0.push_back(x_end);
+    double vmin_all = vmin[0];
+    for (int q = 1; q < P; ++q) vmin_all = fmin(vmin_all, vmin[q]);
+    // a run's own spacing test (its vmin >= vmin_all) passes whenever this one does
+    const bool uniform_ok = kirch_spacing(S, T, dist_m, tt_s, vmin_all, kirch_monotone(T, dist_m)).uniform_ok;
+    IMPDAR_CHECK_ARG(!(g_kirch_mode >= 2 && !uniform_ok), "kirchhoff: table path forced but trace spacing is not uniform");
+    const bool per_run = g_kirch_mode >= 2 ||
+                         (g_kirch_mode == 0 && uniform_ok && (long long)T >= (long long)KIRCH_RUN_MIN * runs_all);
+    char *block = (char *)(((uintptr_t)workspace + base + 255) & ~(uintptr_t)255);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (!per_run) {
+        KirchLateral lat = {profiles, P, col_profile, vmin.data(), vconst.data(), block};
+        KirchWindow win = {col0, ncols, ld, ldo, col0 == 0 && ncols == T};
+        return kirchhoff_impl(data, out, S, T, dist_m, tt_s, grad_coef, vrow.data(), nearfield, x_begin, x_end, workspace,
+                              base, stream, nullptr, nullptr, &win, &lat);
+    }
+    IMPDAR_CHECK_ARG(col0 >= 0 && ncols >= 1 && col0 + ncols <= T && ld >= ncols,
+                     "kirchhoff_window: bad column window [%d, %d) / strides", col0, col0 + ncols);
+    int *sum = (int *)block;
+    IMPDAR_CUDA(cudaMemsetAsync(sum, 0, 256, st));
+    int path = 0;
+    for (int r = 0; r < nruns; ++r) {
+        const int a = run0[r], b = run0[r + 1], q = col_profile[a];
+        // the run's input window, inside the caller's, cut at multiples of 4 columns from col0 (128-bit d/dt pass)
+        int w0 = 0, w1 = T;
+        if (int rc = impdar_kirchhoff_input_window(S, T, dist_m, tt_s, vmax[q], a, b, &w0, &w1)) return rc;
+        w0 = w0 > col0 ? w0 : col0;
+        w1 = w1 < col0 + ncols ? w1 : col0 + ncols;
+        w0 = col0 + ((w0 - col0) & ~3);
+        w1 = col0 + ((w1 - col0 + 3) & ~3);
+        if (w1 > col0 + ncols) w1 = col0 + ncols;
+        KirchWindow win = {w0, w1 - w0, ld, ldo, false};
+        int rc = kirchhoff_impl(data + (w0 - col0), out + (a - x_begin), S, T, dist_m, tt_s, grad_coef,
+                                profiles + (size_t)q * S, nearfield, a, b, workspace, base, stream, nullptr, nullptr, &win);
+        if (rc) return rc;
+        kirch_run_summary_kernel<<<1, 32, 0, st>>>(g_last_flags, sum);
+        IMPDAR_LAUNCH_CHECK();
+        path = g_last_path;
+    }
+    g_last_flags = sum;
+    g_last_stats = (unsigned long long *)(sum + 32);
+    g_last_path = path;
+    return IMPDAR_B200_OK;
 }
 
 int impdar_kirchhoff_set_mode(int mode) {

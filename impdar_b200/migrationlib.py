@@ -316,6 +316,125 @@ def migrationKirchhoffLayered(dat, vel=1.69e8, vel_fn=None, nearfield=False, **g
     return dat
 
 
+def rms_velocity_profiles(travel_time_us, profiles):
+    """rms_velocity of each row of a (P, snum) array of interval-velocity profiles.  The same operations along axis 1
+    (the cumulative sum runs left to right within each row), so row i equals rms_velocity(travel_time_us, profiles[i])
+    bit for bit."""
+    t = np.asarray(travel_time_us, dtype=np.float64) / 1.0e6
+    vm = np.asarray(profiles, dtype=np.float64)
+    if vm.ndim != 2 or vm.shape[1] != t.shape[0]:
+        raise ValueError('profiles must have shape (P, %d), got %s' % (len(t), str(vm.shape)))
+    v = vm.copy()
+    nonneg = np.nonzero(t >= 0)[0]
+    if len(nonneg):
+        j0 = nonneg[0]
+        v2 = vm[:, j0:] ** 2
+        steps = (v2[:, 1:] + v2[:, :-1]) / 2. * np.diff(t[j0:])
+        integral = np.cumsum(np.concatenate([v2[:, :1] * t[j0], steps], axis=1), axis=1)
+        pos = t[j0:] > 0
+        v[:, j0:][:, pos] = np.sqrt(integral[:, pos] / t[j0:][pos])
+    return v
+
+
+def _kirch_lateral_args(profiles, col_profile, snum, tnum):
+    """Validated contiguous (P, snum) float64 profiles and (tnum,) int32 trace -> profile map."""
+    v = np.ascontiguousarray(device.host_f64(profiles))
+    if v.ndim != 2 or v.shape[1] != int(snum) or v.shape[0] < 1:
+        raise ValueError('Kirchhoff lateral profiles must have shape (P, %d), got %s' % (int(snum), str(v.shape)))
+    if not (np.all(np.isfinite(v)) and np.all(v > 0)):
+        raise ValueError('Kirchhoff lateral profiles must be finite and positive')
+    c = np.asarray(col_profile)
+    if c.shape != (int(tnum),) or not (np.issubdtype(c.dtype, np.integer) or c.dtype == bool):
+        raise ValueError('col_profile must be an integer array of shape (%d,), got %s %s' % (int(tnum), c.dtype, c.shape))
+    if c.size and (c.min() < 0 or c.max() >= v.shape[0]):
+        raise ValueError('col_profile values must lie in [0, %d)' % v.shape[0])
+    return v, np.ascontiguousarray(c, dtype=np.int32)
+
+
+def _kirch_window_vxz(lib, win_ptr, col0, ncols, ld, out, S, T, dist_m, tt_sec, coef, profiles, colp, nearfield,
+                      x_begin, x_end):
+    ws = device.workspace(lib.impdar_kirchhoff_lateral_workspace_bytes(S, int(T), profiles.shape[0],
+                                                                       int(bool(nearfield))))
+    rc = lib.impdar_kirchhoff_window_vxz_f32(win_ptr, int(col0), int(ncols), int(ld), device.ptr(out),
+                                             int(out.stride(0)), S, int(T), device.ptr(dist_m), device.ptr(tt_sec),
+                                             device.ptr(coef), device.ptr(profiles), int(profiles.shape[0]),
+                                             device.ptr(colp), int(bool(nearfield)), int(x_begin), int(x_end),
+                                             device.ptr(ws), ws.numel(), device.current_stream_ptr())
+    _lib.check(rc)
+    return out
+
+
+def kirchhoff_lateral_device(data_dev, travel_time_us, dist_km, profiles, col_profile, nearfield, x_begin=0,
+                             x_end=None, out=None):
+    """Kirchhoff with a laterally varying velocity on a (snum, tnum) float32 CUDA tensor: output trace xi migrates with
+    the RMS profile profiles[col_profile[xi]] ((P, snum) velocities, finite and positive); returns the
+    (snum, x_end - x_begin) float32 block.  Column xi equals kirchhoff_device's column xi with that profile
+    (impdar_kirchhoff_window_vxz_f32)."""
+    import torch
+    lib = _lib.load()
+    S, T = data_dev.shape
+    x_end = T if x_end is None else x_end
+    v, colp = _kirch_lateral_args(profiles, col_profile, S, T)
+    tt_sec = device.host_f64(travel_time_us) / 1.0e6
+    dist_m = np.ascontiguousarray(device.host_f64(dist_km) * 1.0e3)
+    if not np.all(np.diff(tt_sec) > 0):
+        raise ValueError('travel_time must be strictly ascending for Kirchhoff migration')
+    coef = gradient_coefficients(tt_sec)
+    if out is None:
+        out = torch.empty((S, x_end - x_begin), dtype=torch.float32, device=data_dev.device)
+    return _kirch_window_vxz(lib, device.ptr(data_dev), 0, T, T, out, S, T, dist_m, tt_sec, coef, v, colp, nearfield,
+                             x_begin, x_end)
+
+
+def lateral_rms_field(dat, vel):
+    """(P, snum) RMS profiles and the (tnum,) trace -> profile map of a (v, z, x) table: lateral_velocity_profiles
+    then rms_velocity_profiles."""
+    profiles, col_profile = lateral_velocity_profiles(dat, np.asarray(vel, dtype=np.float64))
+    return rms_velocity_profiles(dat.travel_time, profiles), col_profile
+
+
+def migrationKirchhoffLateral(dat, vel=1.69e8, vel_fn=None, nearfield=False, **genfromtxt_kwargs):
+    """Kirchhoff migration with a laterally varying velocity: a (v, z, x) table (or the file `vel_fn`, loaded like
+    migrationKirchhoffLayered does) gives each trace the RMS velocity of its column of getVelocityProfile, and output
+    sample (ti, xi) migrates with V[ti, xi] along straight rays.  A scalar or a (v, z) table is exactly
+    migrationKirchhoffLayered; a field with a single profile runs the layered path with that vector.  dat.data becomes
+    float64 on the host lane, a tensor on the device lane."""
+    if vel_fn is not None:
+        try:
+            vel = np.genfromtxt(vel_fn, **genfromtxt_kwargs)
+            print('Velocities loaded from %s.' % vel_fn)
+        except Exception:
+            raise TypeError('File %s was given for input velocity array, but cannot be loaded. Please reformat to txt file.' % vel_fn)
+    if not (len(np.shape(vel)) == 2 and np.shape(vel)[1] == 3):
+        return migrationKirchhoffLayered(dat, vel=vel, nearfield=nearfield)
+    print('Kirchhoff Migration (diffraction summation, lateral velocity) of %.0fx%.0f matrix' % (dat.snum, dat.tnum))
+    _check_data_shape(dat)
+    start = time.time()
+    profiles, col_profile = lateral_rms_field(dat, vel)
+    on_device = device.is_device_array(dat.data)
+    if profiles.shape[0] == 1:
+        v = profiles[0]
+        if on_device:
+            in_dt = dat.data.dtype
+            out = kirchhoff_device(device.to_device(dat.data), dat.travel_time, dat.dist, v, nearfield)
+            dat.data = out if out.dtype == in_dt or not in_dt.is_floating_point else out.to(in_dt)
+        else:
+            dat.data = kirchhoff_host(dat.data, dat.travel_time, dat.dist, v, nearfield)
+    elif on_device:
+        in_dt = dat.data.dtype
+        out = kirchhoff_lateral_device(device.to_device(dat.data), dat.travel_time, dat.dist, profiles, col_profile,
+                                       nearfield)
+        dat.data = out if out.dtype == in_dt or not in_dt.is_floating_point else out.to(in_dt)
+    else:   # upload, migrate, download back to back; float32 results widened like kirchhoff_host's
+        device.require_cuda()
+        x = device.to_device(np.asarray(dat.data))
+        out = kirchhoff_lateral_device(x, dat.travel_time, dat.dist, profiles, col_profile, nearfield)
+        dat.data = out.cpu().numpy().astype(np.float64)
+    print('Kirchhoff Migration of %.0fx%.0f matrix complete in %.2f seconds'
+          % (dat.snum, dat.tnum, time.time() - start))
+    return dat
+
+
 def kirchhoff_stats():
     """(pairs, exact_pairs) of the last Kirchhoff call (needs enable_kirchhoff_stats(True) beforehand)."""
     lib = _lib.load()
@@ -342,17 +461,18 @@ def set_kirchhoff_mode(mode=KIRCHHOFF_AUTO):
 
 def kirchhoff_last_path():
     """'general' or 'table': which path the last Kirchhoff call ran."""
-    return {1: 'general', 2: 'table', 3: 'table'}.get(_lib.load().impdar_kirchhoff_last_path(), 'none')
+    return {1: 'general', 2: 'table', 3: 'table', 4: 'general'}.get(_lib.load().impdar_kirchhoff_last_path(), 'none')
 
 
 def kirchhoff_last_kernel():
-    """'general', 'table_gather' or 'table_tile' - the kernel that did the far-field sum of the last call ('table_tile'
-    only if the tile kernel did all of it; it stands down for hyperbola intervals wider than its staged segments, and
-    leaves the rows that read non-finite input to the gather kernel).  Synchronises the call's stream."""
+    """'general', 'general_lateral', 'table_gather' or 'table_tile' - the kernel that did the far-field sum of the last
+    call ('table_tile' only if the tile kernel did all of it - for a lateral field, in every run; it stands down for
+    hyperbola intervals wider than its staged segments, and leaves the rows that read non-finite input to the gather
+    kernel).  Synchronises the call's stream."""
     lib = _lib.load()
     path = lib.impdar_kirchhoff_last_path()
     if path != 3:
-        return {1: 'general', 2: 'table_gather'}.get(path, 'none')
+        return {1: 'general', 2: 'table_gather', 4: 'general_lateral'}.get(path, 'none')
     v = ctypes.c_int(0)
     _lib.check(lib.impdar_kirchhoff_last_tile_standdown(ctypes.byref(v)), RuntimeError)
     return 'table_gather' if v.value else 'table_tile'
@@ -444,28 +564,49 @@ def getVelocityProfile(dat, vels_in):
         zoft = interp1d(tofz, zs)(twtt)
         vmig = 2. * np.gradient(zoft, twtt)
     elif dimension == 3:
-        vel_x = vels_in[:, 2]
-        zs = np.linspace(np.min(vel_v) * twtt[0], np.max(vel_v) * twtt[-1], dat.snum) / 2.
-        if dat.dist is None or all(dat.dist == 0):
-            raise ValueError('The distance vector was never set.')
-        XS, ZS = np.meshgrid(dat.dist, zs)
-        VS = griddata(np.transpose([vel_x, vel_z]), vel_v,
-                      np.transpose([XS.flatten(), ZS.flatten()]), method='nearest')
-        VS = np.reshape(VS, np.shape(XS))
-        vmig = np.zeros_like(VS)
-        trapz = getattr(np, 'trapezoid', None) or np.trapz
-        for i in range(dat.tnum):
-            vz = ZS[:, i]
-            vv = VS[:, i]
-            vel_t = 2 * np.array([trapz(1. / vv[:j], vz[:j]) for j in range(dat.snum)])
-            tofz = interp1d(ZS[:, i], vel_t)(zs)
-            zinterp = interp1d(tofz, zs)
-            if twtt[-1] > tofz[-1]:
-                raise ValueError('Two-way travel time array extends outside of interpolation range')
-            vmig[:, i] = 2. * np.gradient(zinterp(twtt), twtt)
+        profiles, col_profile = lateral_velocity_profiles(dat, vels_in)
+        vmig = np.zeros((dat.snum, dat.tnum), dtype=profiles.dtype)
+        vmig[:] = profiles.T[:, col_profile]
     else:
         raise ValueError('Input must be 2d with 2 or 3 columns')
     return vmig
+
+
+def lateral_velocity_profiles(dat, vels_in):
+    """getVelocityProfile's (v, z, x) branch in compact form: (profiles, col_profile) with profiles[p] the interval
+    velocity (P, snum) of the p-th distinct column and col_profile (tnum,) the profile of each trace, so that
+    getVelocityProfile(dat, vels_in)[:, i] == profiles[col_profile[i]].  The reference's per-trace loop (O(snum^2)
+    trapezoids per trace) depends on a trace only through its nearest-neighbour griddata column, so it runs once per
+    distinct column - columns are compared bit for bit - in order of first appearance (the same first ValueError)."""
+    from scipy.interpolate import griddata, interp1d
+    vel_v, vel_z, vel_x = vels_in[:, 0], vels_in[:, 1], vels_in[:, 2]
+    twtt = np.asarray(dat.travel_time, dtype=np.float64).copy() / 1.0e6
+    zs = np.linspace(np.min(vel_v) * twtt[0], np.max(vel_v) * twtt[-1], dat.snum) / 2.
+    if dat.dist is None or all(dat.dist == 0):
+        raise ValueError('The distance vector was never set.')
+    XS, ZS = np.meshgrid(dat.dist, zs)
+    VS = griddata(np.transpose([vel_x, vel_z]), vel_v,
+                  np.transpose([XS.flatten(), ZS.flatten()]), method='nearest')
+    VS = np.reshape(VS, np.shape(XS))
+    cols = np.ascontiguousarray(VS.T)
+    keys = cols.view(np.dtype((np.void, cols.dtype.itemsize * cols.shape[1]))).ravel()
+    _, first, inverse = np.unique(keys, return_index=True, return_inverse=True)
+    order = np.argsort(first)                       # profiles in order of first appearance
+    rank = np.empty_like(order)
+    rank[order] = np.arange(len(order))
+    col_profile = rank[inverse.ravel()]
+    profiles = np.zeros((len(order), dat.snum), dtype=VS.dtype)
+    trapz = getattr(np, 'trapezoid', None) or np.trapz
+    for p, i in enumerate(first[order]):
+        vz = ZS[:, i]
+        vv = VS[:, i]
+        vel_t = 2 * np.array([trapz(1. / vv[:j], vz[:j]) for j in range(dat.snum)])
+        tofz = interp1d(ZS[:, i], vel_t)(zs)
+        zinterp = interp1d(tofz, zs)
+        if twtt[-1] > tofz[-1]:
+            raise ValueError('Two-way travel time array extends outside of interpolation range')
+        profiles[p] = 2. * np.gradient(zinterp(twtt), twtt)
+    return profiles, col_profile
 
 
 def phase_shift_device(data_dev, dt, dx, travel_time_us, vmig, htaper, vtaper, out=None):

@@ -194,6 +194,20 @@ int impdar_kirchhoff_host_pipelined_vz_f64(const float *h_data, double *h_out, i
                                            const double *dist_m, const double *tt_s, const double *grad_coef,
                                            const double *vel_s, int nearfield, int nchunks, void *workspace,
                                            size_t workspace_bytes, void *stream);
+/* Laterally varying velocity: output trace xi migrates with profile col_profile[xi] of `profiles` (HOST, nprof x snum
+ * doubles, RMS velocities, each finite and > 0; col_profile: HOST, tnum ints in [0, nprof); status 1 otherwise).
+ * Column xi equals column xi of impdar_kirchhoff_window_vz_f32 run with that profile.  Window arguments as there (the
+ * window must cover impdar_kirchhoff_input_window_vz's interval for the row-wise largest velocity); whole image only
+ * (no row chunks); (col0, ncols) = (0, tnum) accepts any trace order.  Path: with uniform trace spacing and runs of one
+ * profile at least 192 traces wide on average over all tnum traces, one single-profile table-path call per run of
+ * [x_begin, x_end) on its own input sub-window
+ * (bit for bit the whole-image single-profile call for finite input); otherwise the lateral general kernel
+ * (impdar_kirchhoff_last_path() == 4).  The workspace has impdar_kirchhoff_lateral_workspace_bytes() bytes.      */
+size_t impdar_kirchhoff_lateral_workspace_bytes(int snum, int tnum, int nprof, int nearfield);
+int impdar_kirchhoff_window_vxz_f32(const float *data, int col0, int ncols, int ld, float *out, int ldo, int snum,
+                                    int tnum, const double *dist_m, const double *tt_s, const double *grad_coef,
+                                    const double *profiles, int nprof, const int *col_profile, int nearfield,
+                                    int x_begin, int x_end, void *workspace, size_t workspace_bytes, void *stream);
 /* Counters of the last impdar_kirchhoff_f32 call (for the roofline): (output sample, input trace) pairs
  * inside the aperture and pairs that took the float64 exact path.  Counting pairs costs an instruction
  * per pair, so it is off unless enabled.  last_stats synchronises the stream of that call.            */
@@ -201,7 +215,8 @@ int impdar_kirchhoff_enable_stats(int on);
 /* Kernel selection (per host thread): 0 = automatic (uniform-geometry table path when the trace spacing is uniform,
  * the general-geometry kernel otherwise), 1 = always the general kernel, 2 = require the table path (shared-memory
  * tile kernel for the far-field sum, global-gather table kernel for near field / non-finite input), 3 = table path
- * with the global-gather kernel only.  impdar_kirchhoff_last_path(): 1 general, 2 table (gather), 3 table (tile). */
+ * with the global-gather kernel only.  impdar_kirchhoff_last_path(): 1 general, 2 table (gather), 3 table (tile),
+ * 4 lateral general kernel.                                                                                        */
 int impdar_kirchhoff_set_mode(int mode);
 int impdar_kirchhoff_last_path(void);
 /* After a table-path call whose last_path is 3 (shared-memory tile kernel launched): *stood_down = 1 when the tile
