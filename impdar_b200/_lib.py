@@ -84,6 +84,9 @@ PROTOTYPES = {
     "impdar_stolt_set_pipeline": (_c_int, [_c_int]),
     "impdar_stolt_last_pipeline": (_c_int, []),
     "impdar_stolt_debug_stop_after": (_c_int, [_c_int]),
+    "impdar_stolt_scan_workspace_bytes": (_c_sz, [_c_int, _c_int, _c_int]),
+    "impdar_stolt_scan_f32": (_c_int, [_vp, _c_int, _c_int, _c_dbl, _c_dbl, _vp, _c_int, _c_dbl, _c_dbl, _c_int, _c_int,
+                                       _c_int, _vp, _vp, _vp, _c_sz, _vp]),
     "impdar_phsh_set_legacy": (_c_int, [_c_int]),
     "impdar_phsh_workspace_bytes": (_c_sz, [_c_int, _c_int]),
     "impdar_phsh_ffd_workspace_bytes": (_c_sz, [_c_int, _c_int]),

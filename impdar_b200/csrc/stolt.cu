@@ -18,6 +18,7 @@
 // interpolation weight is its fractional part); the interpolation itself is fp32 complex FMA.
 #include <cufft.h>
 
+#include <cmath>
 #include <map>
 #include <mutex>
 #include <tuple>
@@ -198,6 +199,13 @@ size_t stolt_fft_workspace_bytes(int S, int T);
 int stolt_fft_run(const float *data, float *out, int S, int T, int batch, double dt, double dx, double vel, double htaper,
                   double vtaper, int trunc_int, void *workspace, int stop_after, cudaStream_t st);
 
+int stolt_fft_scan_forward(const float *data, float *W1, float *W2, int S, int T, double htaper, double vtaper,
+                           int trunc_int, cudaStream_t st);
+int stolt_fft_scan_velocity(const float *W2, float *W3, float *img, int S, int T, double dt, double dx, double vel,
+                            cudaStream_t st);
+size_t stolt_focus_workspace_bytes(int rows, int cols);
+int stolt_focus_run(const float *img, int rows, int cols, int ws, int wt, double *focus, void *part, cudaStream_t st);
+
 static int get_plans(int S, int T, cudaStream_t st, StoltPlans &out) {
     int dev = 0;
     IMPDAR_CUDA(cudaGetDevice(&dev));
@@ -354,6 +362,123 @@ int impdar_stolt_f32(const float *data, float *out, int S, int T, int batch, dou
         IMPDAR_CUFFT(cufftExecC2C(pl.c2c, (cufftComplex *)bufKK, (cufftComplex *)bufKK, CUFFT_INVERSE));
         IMPDAR_CUFFT(cufftExecC2R(pl.c2r, (cufftComplex *)bufKK, dout));
         count_launch(2);
+    }
+    return IMPDAR_B200_OK;
+}
+
+static inline size_t align256(size_t b) { return (b + 255) & ~(size_t)255; }
+
+// Velocities run one after another through the same buffers, so the scratch does not grow with nvel.
+size_t impdar_stolt_scan_workspace_bytes(int S, int T, int nvel) {
+    (void)nvel;
+    if (S < 2 || T < 1) return 0;
+    const size_t M = (size_t)(S / 2 + 1);
+    const size_t img = (size_t)S * (size_t)T * sizeof(float);
+    const size_t cplx = M * (size_t)T * sizeof(float2);
+    // five-pass: W1 (P1 output and the image when the caller keeps none), W2 (forward spectrum), W3 (one velocity's
+    // spectrum); cuFFT: the taper / remapped-spectrum buffer, the forward spectrum and the image
+    const size_t five = 3 * align256(img);
+    const size_t fft = align256(cplx > img ? cplx : img) + align256(cplx) + align256(img);
+    return (five > fft ? five : fft) + align256(stolt_focus_workspace_bytes(2 * (S / 2), T)) + 256;
+}
+
+int impdar_stolt_scan_f32(const float *data, int S, int T, double dt, double dx, const double *vels, int nvel,
+                          double htaper, double vtaper, int trunc_int, int win_s, int win_t, double *focus,
+                          float *images, void *workspace, size_t ws_bytes, void *stream) {
+    IMPDAR_CHECK_ARG(data && focus, "stolt_scan: null pointer");
+    IMPDAR_CHECK_ARG(S >= 2 && T >= 1, "stolt_scan: need snum >= 2, tnum >= 1");
+    IMPDAR_CHECK_ARG(dt > 0.0 && dx != 0.0, "stolt_scan: dt must be positive and dx non-zero");
+    IMPDAR_CHECK_ARG(vels && nvel >= 1, "stolt_scan: need at least one velocity");
+    for (int v = 0; v < nvel; ++v)
+        IMPDAR_CHECK_ARG(std::isfinite(vels[v]) && vels[v] > 0.0, "stolt_scan: velocity %d (%g) must be finite and positive",
+                         v, vels[v]);
+    IMPDAR_CHECK_ARG(win_s >= 1 && win_t >= 1, "stolt_scan: window (%d, %d) must be at least 1 x 1", win_s, win_t);
+    const size_t need = impdar_stolt_scan_workspace_bytes(S, T, nvel);
+    IMPDAR_CHECK_ARG(workspace && ws_bytes >= need, "stolt_scan: workspace too small (%zu < %zu)", ws_bytes, need);
+    IMPDAR_CHECK_ARG(!(g_stolt_mode == 3 && !stolt_fft_supported(S, T)),
+                     "stolt: the five-pass pipeline does not cover snum = %d, tnum = %d", S, T);
+    cudaStream_t st = (cudaStream_t)stream;
+    const int M = S / 2 + 1;
+    const int S2 = 2 * (M - 1);
+    const size_t per_img = (size_t)S2 * T;
+    const size_t per_focus = (size_t)((S2 + win_s - 1) / win_s) * (size_t)((T + win_t - 1) / win_t);
+    const size_t img = (size_t)S * T * sizeof(float);
+    const size_t cplx = (size_t)M * T * sizeof(float2);
+    char *w = (char *)(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
+    const size_t five = 3 * align256(img);
+    const size_t fft = align256(cplx > img ? cplx : img) + align256(cplx) + align256(img);
+    void *part = w + (five > fft ? five : fft);
+    int rc;
+
+    if ((g_stolt_mode == 0 || g_stolt_mode == 3) && stolt_fft_supported(S, T)) {
+        float *W1 = (float *)w, *W2 = (float *)(w + align256(img)), *W3 = (float *)(w + 2 * align256(img));
+        if ((rc = stolt_fft_scan_forward(data, W1, W2, S, T, htaper, vtaper, trunc_int, st))) return rc;
+        for (int v = 0; v < nvel; ++v) {
+            float *dout = images ? images + v * per_img : W1;
+            if ((rc = stolt_fft_scan_velocity(W2, W3, dout, S, T, dt, dx, vels[v], st))) return rc;
+            if ((rc = stolt_focus_run(dout, S2, T, win_s, win_t, focus + v * per_focus, part, st))) return rc;
+        }
+        g_stolt_last = 3;
+        return IMPDAR_B200_OK;
+    }
+    StoltPlans pl;
+    rc = get_plans(S, T, st, pl);
+    if (rc) return rc;
+    g_stolt_last = pl.paired ? 2 : 1;
+    float *bufA = (float *)w;  // tapered input, later each velocity's remapped spectrum KK
+    float2 *bufKK = (float2 *)w;
+    float2 *bufFK = (float2 *)(w + align256(cplx > img ? cplx : img));
+    float *scratch = (float *)(w + align256(cplx > img ? cplx : img) + align256(cplx));
+    rc = impdar_taper_f32(data, bufA, S, T, 1, htaper, vtaper, trunc_int, stream);
+    if (rc) return rc;
+    if (pl.paired) {
+        IMPDAR_CUFFT(cufftSetStream(pl.c2c2d, st));
+        IMPDAR_CUFFT(cufftExecC2C(pl.c2c2d, (cufftComplex *)bufA, (cufftComplex *)bufA, CUFFT_FORWARD));
+        count_launch(1);
+        StoltPairedParams pp;
+        pp.S = S; pp.Th = T / 2; pp.T = T; pp.nz = S / 2;
+        pp.norm = (float)(1.0 / ((double)S * (double)T));
+        pp.Zh = (const float2 *)bufA;
+        for (int v = 0; v < nvel; ++v) {
+            float *dout = images ? images + v * per_img : scratch;
+            pp.beta_unit = vels[v] * (double)S * dt / (2.0 * (double)T * dx);
+            pp.Zq = (float2 *)dout;
+            const int rows_per_cta = 32;
+            dim3 grid((pp.Th + 127) / 128, (pp.nz + rows_per_cta - 1) / rows_per_cta);
+            ktimer_begin("stolt_remap_paired_kernel", st);
+            stolt_remap_paired_kernel<<<grid, 128, 0, st>>>(pp, rows_per_cta);
+            ktimer_end(st);
+            IMPDAR_LAUNCH_CHECK();
+            IMPDAR_CUFFT(cufftExecC2C(pl.c2c2d, (cufftComplex *)dout, (cufftComplex *)dout, CUFFT_INVERSE));
+            count_launch(1);
+            if ((rc = stolt_focus_run(dout, S2, T, win_s, win_t, focus + v * per_focus, part, st))) return rc;
+        }
+        return IMPDAR_B200_OK;
+    }
+    IMPDAR_CUFFT(cufftSetStream(pl.r2c, st));
+    IMPDAR_CUFFT(cufftSetStream(pl.c2c, st));
+    IMPDAR_CUFFT(cufftSetStream(pl.c2r, st));
+    IMPDAR_CUFFT(cufftExecR2C(pl.r2c, bufA, (cufftComplex *)bufFK));
+    IMPDAR_CUFFT(cufftExecC2C(pl.c2c, (cufftComplex *)bufFK, (cufftComplex *)bufFK, CUFFT_FORWARD));
+    count_launch(2);
+    StoltRemapParams rp;
+    rp.M = M; rp.T = T; rp.nz = S / 2;
+    rp.norm = (float)(1.0 / ((double)S2 * (double)T));
+    rp.FK = bufFK;
+    rp.KK = bufKK;
+    for (int v = 0; v < nvel; ++v) {
+        float *dout = images ? images + v * per_img : scratch;
+        rp.beta_unit = vels[v] * (double)S * dt / (2.0 * (double)T * dx);
+        const int rows_per_cta = 32;
+        dim3 grid((T + 127) / 128, (M + rows_per_cta - 1) / rows_per_cta);
+        ktimer_begin("stolt_remap_kernel", st);
+        stolt_remap_kernel<<<grid, 128, 0, st>>>(rp, rows_per_cta);
+        ktimer_end(st);
+        IMPDAR_LAUNCH_CHECK();
+        IMPDAR_CUFFT(cufftExecC2C(pl.c2c, (cufftComplex *)bufKK, (cufftComplex *)bufKK, CUFFT_INVERSE));
+        IMPDAR_CUFFT(cufftExecC2R(pl.c2r, (cufftComplex *)bufKK, dout));
+        count_launch(2);
+        if ((rc = stolt_focus_run(dout, S2, T, win_s, win_t, focus + v * per_focus, part, st))) return rc;
     }
     return IMPDAR_B200_OK;
 }

@@ -608,16 +608,23 @@ FFTR_DI void stockham_step(cf *__restrict__ buf, const cf *__restrict__ twS, con
 // PF (prefetch): the column is brought into the (then idle) transform buffer by one 1-D TMA bulk copy issued as soon as the
 // previous column's last step has its operands in registers, so the load overlaps that step's butterflies and global
 // stores instead of being waited for at the top of the loop; without PF the first step loads straight from global memory.
+//
+// SPLIT (velocity scan): the prefetch reads the column from `src` and the last step stores to p.Dt, so the forward
+// spectrum in `src` survives for the next velocity.  Without SPLIT the column is transformed in place in p.Dt and `src`
+// is unused; those instantiations compile to the same SASS as before SPLIT existed.
 #ifndef COL_MINB_8192
 #define COL_MINB_8192 2
 #define COL_MINB_4096 4
 #define COL_MINB_SMALL 8
 #endif
 #define COL_MINB(S) ((S) >= 8192 ? COL_MINB_8192 : ((S) >= 4096 ? COL_MINB_4096 : COL_MINB_SMALL))
-template <int S, int R3, bool PF>
-__global__ void __launch_bounds__(S / 32, COL_MINB(S)) stolt_col_kernel(const __grid_constant__ ColParams p) {
+template <int S, int R3, bool PF, bool SPLIT>
+__global__ void __launch_bounds__(S / 32, COL_MINB(S)) stolt_col_kernel(const __grid_constant__ ColParams p,
+                                                                         const cf *__restrict__ src) {
     constexpr int NT = S / 32, NI = S / 16, NZ = S / 2;
     static_assert(16 * 16 * R3 == S && NT >= 32, "factorisation");
+    static_assert(PF || !SPLIT, "the split variant loads through the prefetch");
+    const cf *const srcb = SPLIT ? src : p.Dt;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     cf *buf = reinterpret_cast<cf *>(smem_raw);
     cf *twS = buf + (S + S / 16);
@@ -632,7 +639,7 @@ __global__ void __launch_bounds__(S / 32, COL_MINB(S)) stolt_col_kernel(const __
     unsigned phase = 0;
     if (PF && tid == 0) {
         mbar_init(bar, 1);
-        if ((int)blockIdx.x < p.ncols) bulk_load_column(buf, p.Dt + (size_t)blockIdx.x * S, S * (unsigned)sizeof(cf), bar);
+        if ((int)blockIdx.x < p.ncols) bulk_load_column(buf, srcb + (size_t)blockIdx.x * S, S * (unsigned)sizeof(cf), bar);
     }
     if (PF) __syncthreads();  // the barrier is initialised before anyone waits on it
 
@@ -732,7 +739,7 @@ __global__ void __launch_bounds__(S / 32, COL_MINB(S)) stolt_col_kernel(const __
             const int nxt = cb + gridDim.x;
             stockham_step<S, R3, 256, 1, NT, true>(buf, twS, tw2, tid, col, [&]() {
                 __syncthreads();  // nobody reads the buffer any more: the next column may land in it
-                if (tid == 0 && nxt < p.ncols) bulk_load_column(buf, p.Dt + (size_t)nxt * S, S * (unsigned)sizeof(cf), bar);
+                if (tid == 0 && nxt < p.ncols) bulk_load_column(buf, srcb + (size_t)nxt * S, S * (unsigned)sizeof(cf), bar);
             });
         } else {
             stockham_step<S, R3, 256, 1, NT, true>(buf, twS, tw2, tid, col);
@@ -848,15 +855,15 @@ static int launch_col(const ColParams &p, cudaStream_t st) {
     static int ctas_per_sm_dev[IMPDAR_MAX_DEVICES];
     int &ctas_per_sm = ctas_per_sm_dev[current_device_slot()];
     if (!ctas_per_sm) {
-        IMPDAR_CUDA(cudaFuncSetAttribute(stolt_col_kernel<S, R3, PF>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        IMPDAR_CUDA(cudaFuncSetAttribute(stolt_col_kernel<S, R3, PF, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         int n = 0;
-        IMPDAR_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, stolt_col_kernel<S, R3, PF>, NT, smem));
+        IMPDAR_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, stolt_col_kernel<S, R3, PF, false>, NT, smem));
         ctas_per_sm = n > 0 ? n : 1;
     }
     int grid = num_sms() * ctas_per_sm;
     if (grid > p.ncols) grid = p.ncols;
     ktimer_begin("stolt_col_kernel", st);
-    stolt_col_kernel<S, R3, PF><<<grid, NT, smem, st>>>(p);
+    stolt_col_kernel<S, R3, PF, false><<<grid, NT, smem, st>>>(p, nullptr);
     ktimer_end(st);
     IMPDAR_LAUNCH_CHECK();
     return IMPDAR_B200_OK;
@@ -885,6 +892,50 @@ static int dispatch_col(int S, const ColParams &p, cudaStream_t st) {
     }
     set_error("stolt: unsupported column length %d", S);
     return IMPDAR_B200_EINVAL;
+}
+
+template <int S, int R3>
+static int launch_col_scan(const ColParams &p, const cf *src, cudaStream_t st) {
+    constexpr int NT = S / 32;
+    const size_t smem = (size_t)(S + S / 16 + 512) * sizeof(cf) + 16;  // + the mbarrier
+    static int ctas_per_sm_dev[IMPDAR_MAX_DEVICES];
+    int &ctas_per_sm = ctas_per_sm_dev[current_device_slot()];
+    if (!ctas_per_sm) {
+        IMPDAR_CUDA(cudaFuncSetAttribute(stolt_col_kernel<S, R3, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        int n = 0;
+        IMPDAR_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, stolt_col_kernel<S, R3, true, true>, NT, smem));
+        ctas_per_sm = n > 0 ? n : 1;
+    }
+    int grid = num_sms() * ctas_per_sm;
+    if (grid > p.ncols) grid = p.ncols;
+    ktimer_begin("stolt_col_scan_kernel", st);
+    stolt_col_kernel<S, R3, true, true><<<grid, NT, smem, st>>>(p, src);
+    ktimer_end(st);
+    IMPDAR_LAUNCH_CHECK();
+    return IMPDAR_B200_OK;
+}
+
+static int dispatch_col_scan(int S, const ColParams &p, const cf *src, cudaStream_t st) {
+    switch (S) {
+        case 1024: return launch_col_scan<1024, 4>(p, src, st);
+        case 2048: return launch_col_scan<2048, 8>(p, src, st);
+        case 4096: return launch_col_scan<4096, 16>(p, src, st);
+        case 8192: return launch_col_scan<8192, 32>(p, src, st);
+    }
+    set_error("stolt: unsupported column length %d", S);
+    return IMPDAR_B200_EINVAL;
+}
+
+// Parameters of the five passes for one profile (batch 1), as stolt_fft_run sets them.
+static void scan_params(int S, int T, const Tables &tb, RowAParams &pa, RowBParams &pb, ColParams &pc) {
+    const int Th = T / 2, N1 = Th / N2;
+    pa = RowAParams();
+    pa.S = S; pa.T = T; pa.Th = Th; pa.N1 = N1; pa.rows_per_cta = 64; pa.batch = 1; pa.twTh = tb.twTh;
+    pb = RowBParams();
+    pb.S = S; pb.T = T; pb.Th = Th; pb.N1 = N1; pb.batch = 1; pb.tw512 = tb.tw512;
+    pc = ColParams();
+    pc.Th = Th; pc.N1 = N1; pc.T = T; pc.ncols = Th; pc.twS = tb.twS; pc.tw2 = tb.tw2;
+    pc.norm = (float)(1.0 / ((double)S * (double)T));
 }
 
 }  // namespace sfft
@@ -931,6 +982,48 @@ int stolt_fft_run(const float *data, float *out, int S, int T, int batch, double
     if (stop_after == 3) return IMPDAR_B200_OK;
     if ((rc = launch_rowB<1>(pb, st))) return rc;
     if (stop_after == 4) return IMPDAR_B200_OK;
+    return dispatch_rowA<1>(pa, st);
+}
+
+// Velocity scan, forward half: P1 (taper, data -> W1) and P2 (W1 -> W2) once.  W1 and W2 hold snum x tnum floats
+// each; W2 keeps the transposed half spectrum that every velocity starts from.
+int stolt_fft_scan_forward(const float *data, float *W1, float *W2, int S, int T, double htaper, double vtaper,
+                           int trunc_int, cudaStream_t st) {
+    using namespace sfft;
+    Tables tb;
+    int rc = get_tables(S, T, st, tb);
+    if (rc) return rc;
+    RowAParams pa;
+    RowBParams pb;
+    ColParams pc;
+    scan_params(S, T, tb, pa, pb, pc);
+    pa.data = data; pa.W1 = reinterpret_cast<cf *>(W1);
+    pa.htaper = htaper; pa.vtaper = vtaper; pa.trunc_int = trunc_int;
+    pa.hceil = (htaper == htaper && htaper < 2.0e9) ? (int)ceil(htaper) : 0x7fffffff;
+    pa.vceil = (vtaper == vtaper && vtaper < 2.0e9) ? (int)ceil(vtaper) : 0x7fffffff;
+    pb.W1 = reinterpret_cast<cf *>(W1); pb.Dt = reinterpret_cast<cf *>(W2);
+    if ((rc = dispatch_rowA<-1>(pa, st))) return rc;
+    return launch_rowB<-1>(pb, st);
+}
+
+// Velocity scan, one velocity: P3 from W2 (left intact) into W3, P4 (W3 -> img) and P5 (in place in img), the same
+// kernels and arithmetic as stolt_fft_run's P3..P5, so img is stolt_fft_run's output at this velocity bit for bit.
+int stolt_fft_scan_velocity(const float *W2, float *W3, float *img, int S, int T, double dt, double dx, double vel,
+                            cudaStream_t st) {
+    using namespace sfft;
+    Tables tb;
+    int rc = get_tables(S, T, st, tb);
+    if (rc) return rc;
+    RowAParams pa;
+    RowBParams pb;
+    ColParams pc;
+    scan_params(S, T, tb, pa, pb, pc);
+    pc.Dt = reinterpret_cast<cf *>(W3);
+    pc.beta_unit = vel * (double)S * dt / (2.0 * (double)T * dx);
+    pb.W1 = reinterpret_cast<cf *>(img); pb.Dt = reinterpret_cast<cf *>(W3);
+    pa.W1 = reinterpret_cast<cf *>(img);
+    if ((rc = dispatch_col_scan(S, pc, reinterpret_cast<const cf *>(W2), st))) return rc;
+    if ((rc = launch_rowB<1>(pb, st))) return rc;
     return dispatch_rowA<1>(pa, st);
 }
 

@@ -7,6 +7,7 @@ libimpdar_b200.so on the current CUDA device; this module only validates, prepar
 vectors in float64 numpy and moves buffers.  There is no CPU fallback.
 """
 import ctypes
+import dataclasses
 import time
 
 import numpy as np
@@ -531,6 +532,141 @@ def migrationStolt(dat, vel=1.68e8, htaper=100, vtaper=1000):
     print('Stolt Migration of %.0fx%.0f matrix complete in %.2f seconds'
           % (dat.snum, dat.tnum, time.time() - start))
     return dat
+
+
+# -------------------------------------------------------------------------------- migration velocity scan
+# Constant-velocity Stolt images over a velocity grid, one focus measure per image window (n E4 / E2^2, the varimax),
+# and the best velocity per window.  Constant-velocity time migration focuses a diffraction with apex time t0 when the
+# velocity equals the hyperbola's straight-ray RMS velocity at t0, the model the layered and lateral Kirchhoff kernels
+# take, so the picks feed kirchhoff_device / kirchhoff_lateral_device directly (scan_rms_field).
+def _scan_vels(vels):
+    try:
+        v = np.array(vels, dtype=np.float64)
+    except (TypeError, ValueError):
+        raise ValueError('scan velocities must be a 1-D array of numbers')
+    if v.ndim != 1 or v.size == 0:
+        raise ValueError('scan velocities must be a non-empty 1-D array, got shape %s' % (v.shape,))
+    if not (np.all(np.isfinite(v)) and np.all(v > 0)):
+        raise ValueError('scan velocities must be finite and positive')
+    return np.ascontiguousarray(v)
+
+
+def _scan_window(window):
+    try:
+        ws, wt = window
+    except (TypeError, ValueError):
+        raise ValueError('window must be a pair (rows, traces), got %r' % (window,))
+    out = []
+    for w in (ws, wt):
+        if isinstance(w, (bool, np.bool_)) or not isinstance(w, (int, np.integer)) or w < 1:
+            raise ValueError('window sizes must be integers >= 1, got %r' % (window,))
+        out.append(int(w))
+    return tuple(out)
+
+
+def stolt_scan_device(data_dev, dt, dx, vels, htaper, vtaper, window, trunc_int=False, images=None):
+    """Focus panel of a Stolt velocity scan of a (snum, tnum) float32 CUDA tensor: returns the (nv, nws, nwt) float64
+    focus tensor (impdar_stolt_scan_f32).  `images`, a (nv, 2*(snum//2), tnum) float32 CUDA tensor, receives each
+    velocity's image, equal to stolt_device at that velocity; without it no image-sized buffer is allocated per velocity."""
+    import torch
+    v = _scan_vels(vels)
+    ws, wt = _scan_window(window)
+    if not (device.is_device_array(data_dev) and data_dev.dim() == 2 and data_dev.dtype == torch.float32):
+        raise ValueError('stolt_scan_device needs a 2-D float32 CUDA tensor')
+    lib = _lib.load()
+    x = data_dev.contiguous()
+    S, T = x.shape
+    S2 = 2 * (S // 2)
+    if images is not None and not (device.is_device_array(images) and images.dtype == torch.float32
+                                   and tuple(images.shape) == (len(v), S2, T) and images.is_contiguous()):
+        raise ValueError('images must be a contiguous float32 CUDA tensor of shape %s' % ((len(v), S2, T),))
+    focus = torch.empty((len(v), -(-S2 // ws), -(-T // wt)), dtype=torch.float64, device=x.device)
+    wsb = device.workspace(lib.impdar_stolt_scan_workspace_bytes(S, T, len(v)))
+    rc = lib.impdar_stolt_scan_f32(device.ptr(x), S, T, float(dt), float(dx), v.ctypes.data_as(ctypes.c_void_p), len(v),
+                                   float(htaper) if htaper != 0 else 0.0, float(vtaper) if vtaper != 0 else 0.0,
+                                   int(bool(trunc_int)), ws, wt, device.ptr(focus), device.ptr(images),
+                                   device.ptr(wsb), wsb.numel(), device.current_stream_ptr())
+    _lib.check(rc)
+    return focus
+
+
+@dataclasses.dataclass
+class VelocityScan:
+    """Result of migrationVelocityScan.  focus[k, i, j] is the focus of window (i, j) of the image at vels[k];
+    vrms[i, j] the velocity of its largest focus (the first on ties), NaN where every focus is 0; center_rows[i] the
+    centre row of window row i."""
+    vels: np.ndarray
+    window: tuple
+    snum: int
+    tnum: int
+    center_rows: np.ndarray
+    focus: np.ndarray
+    vrms: np.ndarray
+
+
+def velocity_scan_result(focus, vels, window, snum, tnum):
+    """VelocityScan from a (nv, nws, nwt) focus panel: the per-window picks and the window-row centres."""
+    focus = np.asarray(focus, dtype=np.float64)
+    v = np.asarray(vels, dtype=np.float64)
+    ws, wt = window
+    S2 = 2 * (int(snum) // 2)
+    starts = np.arange(focus.shape[1]) * ws
+    n_i = np.minimum(starts + ws, S2) - starts
+    vrms = v[np.argmax(focus, axis=0)]
+    vrms[np.all(focus == 0, axis=0)] = np.nan
+    return VelocityScan(vels=v, window=(int(ws), int(wt)), snum=int(snum), tnum=int(tnum),
+                        center_rows=starts + (n_i - 1) / 2.0, focus=focus, vrms=vrms)
+
+
+def migrationVelocityScan(dat, vels, window=(64, 64), htaper=100, vtaper=1000):
+    """Migration velocity scan: Stolt-migrate dat at every constant velocity of `vels` (one shared forward transform),
+    measure the focus of every window (rows x traces) of every image, and pick the best velocity per window.
+    dat is not modified.  Returns a VelocityScan; scan_rms_field turns it into Kirchhoff's lateral RMS field."""
+    print('Stolt velocity scan of %.0fx%.0f matrix over %d velocities' % (dat.snum, dat.tnum, np.size(vels)))
+    _check_data_shape(dat)
+    v = _scan_vels(vels)
+    window = _scan_window(window)
+    start = time.time()
+    in_dtype = _np_dtype(dat.data)
+    trunc_int = in_dtype is not None and np.issubdtype(in_dtype, np.integer)  # as migrationStolt
+    x = device.to_device(dat.data)
+    focus = stolt_scan_device(x, dat.dt, _mean_trace_spacing(dat), v, htaper, vtaper, window, trunc_int)
+    scan = velocity_scan_result(focus.cpu().numpy(), v, window, dat.snum, dat.tnum)
+    print('Stolt velocity scan of %.0fx%.0f matrix complete in %.2f seconds'
+          % (dat.snum, dat.tnum, time.time() - start))
+    return scan
+
+
+def scan_rms_field(scan, min_focus=0.0):
+    """(profiles (P, snum), col_profile (tnum,)) from a VelocityScan, the compact field kirchhoff_lateral_device takes:
+    picks whose best focus is below min_focus are dropped; each window column's picks are interpolated linearly over
+    the rows (np.interp: constant beyond the first and last window centre); a column without picks takes the nearest
+    column that has some (the left one on ties); trace x takes window column x // wt; identical profiles (bit for bit)
+    are merged in order of first appearance.  With one window column P == 1 and profiles[0] suits kirchhoff_device."""
+    vrms = np.array(scan.vrms, dtype=np.float64)
+    best = np.max(scan.focus, axis=0)
+    vrms[best < min_focus] = np.nan
+    rows = np.arange(scan.snum, dtype=np.float64)
+    nwt = vrms.shape[1]
+    cols = []
+    for j in range(nwt):
+        ok = np.isfinite(vrms[:, j])
+        cols.append(np.interp(rows, scan.center_rows[ok], vrms[ok, j]) if ok.any() else None)
+    have = [j for j in range(nwt) if cols[j] is not None]
+    if not have:
+        raise ValueError('velocity scan: no window has a pick (min_focus = %g)' % min_focus)
+    for j in range(nwt):
+        if cols[j] is None:
+            cols[j] = cols[min(have, key=lambda k: (abs(k - j), k))]
+    index, profiles, win_profile = {}, [], []
+    for c in cols:
+        key = c.tobytes()
+        if key not in index:
+            index[key] = len(profiles)
+            profiles.append(c)
+        win_profile.append(index[key])
+    col_profile = np.asarray(win_profile, dtype=np.intp)[np.arange(scan.tnum) // scan.window[1]]
+    return np.array(profiles), col_profile
 
 
 # -------------------------------------------------------------------------------------- phase shift

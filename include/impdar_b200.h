@@ -269,6 +269,21 @@ int impdar_stolt_last_pipeline(void);
  * spectrum (tnum/2 x snum complex).  tests/stolt_stage_model.py restates each stage.                    */
 int impdar_stolt_debug_stop_after(int stage);
 
+/* Migration velocity scan: Stolt images of data (snum, tnum) at each of the nvel constant velocities vels[] (HOST
+ * memory), sharing one forward transform, and the focus of every window of every image:
+ *   focus (DEVICE, nvel x nws x nwt float64, row-major), nws = ceil(S2 / win_s), nwt = ceil(tnum / win_t),
+ *   S2 = 2*(snum/2); window (i, j) covers rows [i win_s, min((i+1) win_s, S2)) and columns
+ *   [j win_t, min((j+1) win_t, tnum)); focus = n E4 / E2^2 with E2 = sum m^2, E4 = sum m^4 over its n samples in
+ *   float64 (0 where E2 == 0).  Deterministic: the same bits on every call.
+ *   images (DEVICE, nullable): nvel x S2 x tnum float32, each equal to impdar_stolt_f32 at that velocity.
+ * The lane is chosen as for impdar_stolt_f32 (impdar_stolt_last_pipeline reports it).  Status 1, before any CUDA call,
+ * for a null data or focus, snum < 2, dt <= 0, dx == 0, nvel < 1, a velocity that is not finite and positive, a window
+ * under 1 x 1, or a workspace smaller than impdar_stolt_scan_workspace_bytes (which does not depend on nvel).      */
+size_t impdar_stolt_scan_workspace_bytes(int snum, int tnum, int nvel);
+int impdar_stolt_scan_f32(const float *data, int snum, int tnum, double dt, double dx, const double *vels, int nvel,
+                          double htaper, double vtaper, int trunc_int, int win_s, int win_t, double *focus,
+                          float *images, void *workspace, size_t workspace_bytes, void *stream);
+
 /* -------------------------------------- phase shift (mig_python.py:211-287, 361-493) --- */
 /* data (snum, tnum) -> out (snum, tnum).  vmig == NULL: constant velocity `vel` (:396-420);
  * otherwise vmig: device, snum doubles, the layered profile from getVelocityProfile (:439-487) and
