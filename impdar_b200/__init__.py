@@ -11,7 +11,8 @@ from .radardata import RadarData, RadarFlags  # noqa: F401
 from .matio import load_mat  # noqa: F401  (StoDeep / ImpDAR .mat files, SURVEY.md 8f rank 4)
 from .migrationlib import (migrationKirchhoff, migrationStolt, migrationPhaseShift,  # noqa: F401
                            migrationTimeWavenumber, getVelocityProfile, migrationKirchhoffLayered, rms_velocity,
-                           migrationKirchhoffLateral, migrationVelocityScan, scan_rms_field)
+                           migrationKirchhoffLateral, migrationVelocityScan, scan_rms_field,
+                           scan_interval_field, depth_curves, interval_table, depthConvert)
 
 __version__ = "0.1.0"
 

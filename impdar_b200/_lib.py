@@ -114,6 +114,13 @@ PROTOTYPES = {
     "impdar_interp_cols_f32": (_c_int, [_vp, _vp, _c_int, _c_int, _c_int, _vp, _c_int, _vp]),
     "impdar_interp_cols_f32_f64": (_c_int, [_vp, _vp, _c_int, _c_int, _c_int, _vp, _c_int, _vp]),
     "impdar_interp_cols_f64": (_c_int, [_vp, _vp, _c_int, _c_int, _c_int, _vp, _c_int, _vp]),
+    "impdar_depth_workspace_bytes": (_c_sz, [_c_int, _c_int, _c_int, _c_int]),
+    "impdar_depth_convert_f32": (_c_int, [_vp, _vp, _c_int, _c_int, _c_int, _vp, _vp, _c_int, _vp, _vp, _vp, _c_sz,
+                                          _vp]),
+    "impdar_depth_convert_f32_f64": (_c_int, [_vp, _vp, _c_int, _c_int, _c_int, _vp, _vp, _c_int, _vp, _vp, _vp,
+                                              _c_sz, _vp]),
+    "impdar_depth_convert_f64": (_c_int, [_vp, _vp, _c_int, _c_int, _c_int, _vp, _vp, _c_int, _vp, _vp, _vp, _c_sz,
+                                          _vp]),
 }
 
 _lib = None

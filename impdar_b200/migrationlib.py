@@ -602,9 +602,10 @@ class VelocityScan:
     center_rows: np.ndarray
     focus: np.ndarray
     vrms: np.ndarray
+    travel_time: np.ndarray = None    # us, snum: what scan_interval_field places the picks by
 
 
-def velocity_scan_result(focus, vels, window, snum, tnum):
+def velocity_scan_result(focus, vels, window, snum, tnum, travel_time=None):
     """VelocityScan from a (nv, nws, nwt) focus panel: the per-window picks and the window-row centres."""
     focus = np.asarray(focus, dtype=np.float64)
     v = np.asarray(vels, dtype=np.float64)
@@ -615,7 +616,8 @@ def velocity_scan_result(focus, vels, window, snum, tnum):
     vrms = v[np.argmax(focus, axis=0)]
     vrms[np.all(focus == 0, axis=0)] = np.nan
     return VelocityScan(vels=v, window=(int(ws), int(wt)), snum=int(snum), tnum=int(tnum),
-                        center_rows=starts + (n_i - 1) / 2.0, focus=focus, vrms=vrms)
+                        center_rows=starts + (n_i - 1) / 2.0, focus=focus, vrms=vrms,
+                        travel_time=None if travel_time is None else np.array(travel_time, dtype=np.float64))
 
 
 def migrationVelocityScan(dat, vels, window=(64, 64), htaper=100, vtaper=1000):
@@ -631,7 +633,7 @@ def migrationVelocityScan(dat, vels, window=(64, 64), htaper=100, vtaper=1000):
     trunc_int = in_dtype is not None and np.issubdtype(in_dtype, np.integer)  # as migrationStolt
     x = device.to_device(dat.data)
     focus = stolt_scan_device(x, dat.dt, _mean_trace_spacing(dat), v, htaper, vtaper, window, trunc_int)
-    scan = velocity_scan_result(focus.cpu().numpy(), v, window, dat.snum, dat.tnum)
+    scan = velocity_scan_result(focus.cpu().numpy(), v, window, dat.snum, dat.tnum, dat.travel_time)
     print('Stolt velocity scan of %.0fx%.0f matrix complete in %.2f seconds'
           % (dat.snum, dat.tnum, time.time() - start))
     return scan
@@ -643,15 +645,28 @@ def scan_rms_field(scan, min_focus=0.0):
     the rows (np.interp: constant beyond the first and last window centre); a column without picks takes the nearest
     column that has some (the left one on ties); trace x takes window column x // wt; identical profiles (bit for bit)
     are merged in order of first appearance.  With one window column P == 1 and profiles[0] suits kirchhoff_device."""
+    vrms = _scan_picks(scan, min_focus)
+    rows = np.arange(scan.snum, dtype=np.float64)
+    cols = []
+    for j in range(vrms.shape[1]):
+        ok = np.isfinite(vrms[:, j])
+        cols.append(np.interp(rows, scan.center_rows[ok], vrms[ok, j]) if ok.any() else None)
+    return _scan_field(scan, cols, min_focus)
+
+
+def _scan_picks(scan, min_focus):
+    """The (nws, nwt) picks of a VelocityScan, NaN where the best focus is below min_focus."""
     vrms = np.array(scan.vrms, dtype=np.float64)
     best = np.max(scan.focus, axis=0)
     vrms[best < min_focus] = np.nan
-    rows = np.arange(scan.snum, dtype=np.float64)
-    nwt = vrms.shape[1]
-    cols = []
-    for j in range(nwt):
-        ok = np.isfinite(vrms[:, j])
-        cols.append(np.interp(rows, scan.center_rows[ok], vrms[ok, j]) if ok.any() else None)
+    return vrms
+
+
+def _scan_field(scan, cols, min_focus):
+    """(profiles, col_profile) from one profile per window column (None: no pick there): an empty column takes the
+    nearest column that has one (the left one on ties), identical profiles (bit for bit) merge in order of first
+    appearance, and trace x takes window column x // wt."""
+    nwt = len(cols)
     have = [j for j in range(nwt) if cols[j] is not None]
     if not have:
         raise ValueError('velocity scan: no window has a pick (min_focus = %g)' % min_focus)
@@ -667,6 +682,325 @@ def scan_rms_field(scan, min_focus=0.0):
         win_profile.append(index[key])
     col_profile = np.asarray(win_profile, dtype=np.intp)[np.arange(scan.tnum) // scan.window[1]]
     return np.array(profiles), col_profile
+
+
+# ---------------------------------------------------------------------- interval velocities (Dix) and depth
+# RMS picks -> interval velocities by a bounded, smoothed least-squares Dix inversion (closed-form Dix takes differences
+# of noisy picks and turns negative), and a time section -> depth section with interval profiles (csrc/depth.cu).
+def depth_curves(travel_time_us, profiles):
+    """(P, snum) float64 one-way depth of every sample for (P, snum) interval velocities: with t = tt / 1e6 and j0 the
+    first sample with t >= 0 (the last sample if there is none), z[j0] = v[j0] t[j0] / 2, then the trapezoid
+    (v[i-1] + v[i]) / 2 (t[i] - t[i-1]) / 2 summed sequentially left to right for the samples after j0 and subtracted
+    right to left for those before it - rms_velocity's trapezoid and anchor, so a constant profile gives v t / 2 (to rounding; exactly when v
+    is a power of two and neighbouring sample times differ exactly).  Strictly increasing for
+    positive velocities and strictly ascending times.  impdar_depth_convert_* computes the same bits on the GPU."""
+    t = np.asarray(travel_time_us, dtype=np.float64) / 1.0e6
+    v = np.asarray(profiles, dtype=np.float64)
+    if v.ndim != 2 or v.shape[1] != t.shape[0] or t.shape[0] < 1:
+        raise ValueError('profiles must have shape (P, %d), got %s' % (len(t), str(v.shape)))
+    nonneg = np.nonzero(t >= 0)[0]
+    j0 = nonneg[0] if len(nonneg) else len(t) - 1
+    z = np.empty_like(v)
+    z0 = v[:, j0:j0 + 1] * t[j0] / 2.
+    steps = (v[:, j0:-1] + v[:, j0 + 1:]) / 2. * np.diff(t[j0:]) / 2.
+    z[:, j0:] = np.cumsum(np.concatenate([z0, steps], axis=1), axis=1)          # sequential, left to right
+    if j0 > 0:
+        back = (v[:, :j0] + v[:, 1:j0 + 1]) / 2. * np.diff(t[:j0 + 1]) / 2.
+        z[:, :j0 + 1] = np.cumsum(np.concatenate([z0, -back[:, ::-1]], axis=1), axis=1)[:, ::-1]   # right to left
+    return z
+
+
+def _dix_normal(tk, Vk):
+    """Normal equations H w = g (n, K, K), (n, K) of the Dix least squares of n columns of K picks (t_k > 0 ascending,
+    RMS V_k) in normalised unknowns w = u / mean(V^2), u = v_int^2 at the pick times, without the smoothing term.
+    D = A u with A = C B: C the lower-triangular ones (a running sum), B bidiagonal (b_m = B[m, m]: t_1, then
+    (t_m - t_{m-1}) / 2; s_m = B[m + 1, m] = (t_{m+1} - t_m) / 2, s_{K-1} = 0).  With W = (ub / D)^2 and
+    R_i = sum_{k >= i} W_k (R_K = 0), A^T W A = B^T G B with G[i, j] = R_max(i, j), which is
+      H[a, b] = (b_a + s_a) (b_b R_b + s_b R_{b+1})                        for a < b (and symmetric),
+      H[a, a] = b_a^2 R_a + (2 b_a s_a + s_a^2) R_{a+1},
+    so H costs O(K^2) per column, not O(K^3)."""
+    n, K = tk.shape
+    ub = np.mean(Vk ** 2, axis=1)
+    r = ub[:, None] / (tk * Vk ** 2)
+    R = np.zeros((n, K + 1))
+    R[:, :K] = np.cumsum((r ** 2)[:, ::-1], axis=1)[:, ::-1]
+    half = np.diff(tk, axis=1) / 2.
+    bd = np.concatenate([tk[:, :1], half], axis=1)
+    bs = np.concatenate([half, np.zeros((n, 1))], axis=1)
+    c = bd + bs
+    e = bd * R[:, :K] + bs * R[:, 1:]
+    O = c[:, :, None] * e[:, None, :]
+    H = np.where(np.triu(np.ones((K, K), dtype=bool), 1), O, O.transpose(0, 2, 1))
+    di = np.arange(K)
+    H[:, di, di] = bd ** 2 * R[:, :K] + (2. * bd * bs + bs ** 2) * R[:, 1:]
+    y = np.zeros((n, K + 1))
+    y[:, :K] = np.cumsum(r[:, ::-1], axis=1)[:, ::-1]               # C^T (ub / D)
+    g = bd * y[:, :K] + bs * y[:, 1:]
+    return H, g, ub
+
+
+def _solve_free(H, g, pinned, wfix):
+    """Minimise 1/2 w H w - g w over the free variables with the pinned ones held at wfix (batched)."""
+    if not pinned.any():
+        return np.linalg.solve(H, g[..., None])[..., 0]
+    free = ~pinned
+    Hf = np.where(free[:, :, None] & free[:, None, :], H, np.eye(H.shape[1]))
+    fix = np.where(pinned, wfix, 0.0)
+    rhs = np.where(free, g - np.einsum('nij,nj->ni', H, fix), fix)
+    return np.linalg.solve(Hf, rhs[..., None])[..., 0]
+
+
+def box_qp(H, g, lo, hi):
+    """argmin 1/2 w H w - g w subject to lo <= w <= hi for a batch of positive definite H (n, K, K), by a primal active
+    set: from a feasible point, solve for the free variables with the pinned ones at their bounds; if that leaves the box,
+    step towards it up to the first bound and pin the variable there; otherwise take it, and release every pinned
+    variable whose gradient points into the box.  Stops when no free variable violates and every pinned gradient points
+    out of the box (the KKT conditions).  Each full step lowers the objective, so no active set repeats."""
+    n, K = g.shape
+    lo = np.broadcast_to(lo, (n, K))
+    hi = np.broadcast_to(hi, (n, K))
+    w = np.clip(np.linalg.solve(H, g[..., None])[..., 0], lo, hi)
+    at_lo, at_hi = w <= lo, w >= hi
+    tol = 1e-12 * (1.0 + np.abs(g).max(axis=1))
+    todo = np.nonzero((at_lo | at_hi).any(axis=1))[0]     # the others hold the unconstrained minimum
+    for _ in range(10 * K + 50):
+        if todo.size == 0:
+            break
+        Ht, gt, lt, ht, wt = H[todo], g[todo], lo[todo], hi[todo], w[todo]
+        al, ah = at_lo[todo], at_hi[todo]
+        pinned = al | ah
+        ws = _solve_free(Ht, gt, pinned, np.where(al, lt, ht))
+        viol = ~pinned & ((ws < lt) | (ws > ht))
+        stepped = viol.any(axis=1)
+        # columns that leave the box: move to the first bound on the way
+        d = ws - wt
+        with np.errstate(divide='ignore', invalid='ignore'):
+            ratio = np.where(viol & (d < 0), (lt - wt) / d, np.where(viol & (d > 0), (ht - wt) / d, np.inf))
+        alpha = np.clip(ratio.min(axis=1), 0.0, 1.0)
+        first = viol & (ratio <= alpha[:, None])
+        wn = np.where(stepped[:, None], np.clip(wt + alpha[:, None] * d, lt, ht), ws)
+        wn = np.where(first & (d < 0), lt, np.where(first & (d > 0), ht, wn))
+        al = al | (first & (d < 0))
+        ah = ah | (first & (d > 0))
+        # columns that stay inside: release the pinned variables whose gradient points into the box
+        grad = np.einsum('nij,nj->ni', Ht, wn) - gt
+        rel = ~stepped[:, None] & ((al & (grad < -tol[todo, None])) | (ah & (grad > tol[todo, None])))
+        al, ah = al & ~rel, ah & ~rel
+        w[todo], at_lo[todo], at_hi[todo] = wn, al, ah
+        todo = todo[stepped | rel.any(axis=1)]
+    return w
+
+
+def _dix_columns(tk_list, V_list, vmin, vmax, smooth):
+    """u = v_int^2 at the picks of every column (lists of 1-D arrays), columns with the same pick count solved together."""
+    out = [None] * len(tk_list)
+    by_k = {}
+    for i, tk in enumerate(tk_list):
+        by_k.setdefault(len(tk), []).append(i)
+    for K, cols in by_k.items():
+        tk = np.array([tk_list[i] for i in cols])
+        Vk = np.array([V_list[i] for i in cols])
+        H, g, ub = _dix_normal(tk, Vk)
+        if K > 1 and smooth > 0:    # + smooth^2 L^T L, L the first difference
+            di = np.arange(K)
+            H[:, di, di] += smooth ** 2 * np.r_[1., 2. * np.ones(K - 2), 1.]
+            H[:, di[:-1], di[1:]] -= smooth ** 2
+            H[:, di[1:], di[:-1]] -= smooth ** 2
+        w = box_qp(H, g, (vmin ** 2 / ub)[:, None], (vmax ** 2 / ub)[:, None])
+        for c, i in enumerate(cols):
+            out[i] = w[c] * ub[c]
+    return out
+
+
+def scan_interval_field(scan, min_focus=0.0, vmin=None, vmax=2.99792458e8, smooth=0.3, travel_time=None):
+    """(profiles (P, snum), col_profile (tnum,)) of INTERVAL velocities from a VelocityScan, the field depthConvert and
+    interval_table take.  Masking, empty-column fill, merging and the trace map are scan_rms_field's.  Per window column
+    the picks (t_k > 0, V_k) sit at the window-centre times; the unknowns u_k = v_int^2 at those times are linear in t
+    between picks and constant (u_1) on [0, t_1], so D_k = t_k V_k^2 = (A u)_k.  The fit minimises
+    sum_k ((A u)_k / D_k - 1)^2 + smooth^2 sum_k ((u_{k+1} - u_k) / mean(V^2))^2 with vmin^2 <= u <= vmax^2 (vmin
+    defaults to half the slowest scan velocity, vmax to the speed of light), all columns at once (box_qp).  Sample i
+    gets sqrt(np.interp(t_i, t_k, u)): constant beyond the first and last pick.  `travel_time` (us, snum) defaults to
+    the scan's own."""
+    tt = scan.travel_time if travel_time is None else travel_time
+    if tt is None:
+        raise ValueError('scan_interval_field needs the travel times of the scanned radargram')
+    t = np.asarray(tt, dtype=np.float64) / 1.0e6
+    if t.shape != (scan.snum,) or not np.all(np.isfinite(t)) or not np.all(np.diff(t) > 0):
+        raise ValueError('travel_time must be %d finite, strictly ascending values' % scan.snum)
+    vmin = 0.5 * float(np.min(scan.vels)) if vmin is None else float(vmin)
+    vmax = float(vmax)
+    if not (np.isfinite(vmin) and np.isfinite(vmax) and 0 < vmin < vmax):
+        raise ValueError('need finite bounds 0 < vmin < vmax, got vmin = %g, vmax = %g' % (vmin, vmax))
+    smooth = float(smooth)
+    if not (np.isfinite(smooth) and smooth >= 0):
+        raise ValueError('smooth must be finite and >= 0, got %g' % smooth)
+    vrms = _scan_picks(scan, min_focus)
+    tc = np.interp(scan.center_rows, np.arange(scan.snum, dtype=np.float64), t)
+    have = [j for j in range(vrms.shape[1]) if np.any(np.isfinite(vrms[:, j]) & (tc > 0))]
+    oks = [np.isfinite(vrms[:, j]) & (tc > 0) for j in have]
+    tks = [tc[ok] for ok in oks]
+    us = _dix_columns(tks, [vrms[ok, j] for ok, j in zip(oks, have)], vmin, vmax, smooth)
+    cols = [None] * vrms.shape[1]
+    for j, tk, u in zip(have, tks, us):
+        cols[j] = np.sqrt(np.interp(t, tk, u))
+    return _scan_field(scan, cols, min_focus)
+
+
+def interval_table(travel_time_us, vint):
+    """A (v, z) table of the interval profile `vint` (snum) that getVelocityProfile maps back onto these travel times,
+    for migrationPhaseShift / migrationKirchhoffLayered or as a vel_fn file (np.savetxt).  getVelocityProfile reads
+    the v column as the AVERAGE velocity down to z (t = 2 z / v), so the rows are (2 z_i / t_i, z_i) with z =
+    depth_curves for every sample with t_i > 0, after a row (v, 0) at the surface, and a last row that continues the
+    deepest interval velocity to max(v) t_end / 2 or deeper, which getVelocityProfile's coverage check asks for when the
+    velocity decreases with depth (firn)."""
+    t = np.asarray(travel_time_us, dtype=np.float64) / 1.0e6
+    v = np.asarray(vint, dtype=np.float64)
+    if v.shape != t.shape or v.ndim != 1:
+        raise ValueError('vint must have one value per sample (%d), got shape %s' % (len(t), str(v.shape)))
+    if not (np.all(np.isfinite(v)) and np.all(v > 0)):
+        raise ValueError('interval velocities must be finite and positive')
+    if not (np.all(np.isfinite(t)) and np.all(np.diff(t) > 0)):
+        raise ValueError('travel_time must be finite and strictly ascending')
+    pos = t > 0
+    if not pos.any():
+        raise ValueError('no sample after time zero')
+    z = depth_curves(travel_time_us, v[None, :])[0][pos]
+    tp = t[pos]
+    va = 2. * z / tp
+    rows = [(va[0], 0.0)] + list(zip(va, z))
+    z_end = max(va.max(), v[-1]) * tp[-1] / 2.
+    if z_end > z[-1]:
+        te = tp[-1] + 2. * (z_end - z[-1]) / v[-1]
+        rows.append((2. * z_end / te, z_end))
+    return np.array(rows, dtype=np.float64)
+
+
+def _depth_args(profiles, col_profile, snum, tnum, zgrid):
+    v, colp = _kirch_lateral_args(profiles, col_profile, snum, tnum)
+    zg = np.ascontiguousarray(np.asarray(zgrid, dtype=np.float64))
+    if zg.ndim != 1 or zg.size < 1 or not np.all(np.isfinite(zg)) or not np.all(np.diff(zg) > 0):
+        raise ValueError('zgrid must be a non-empty 1-D array of finite, strictly ascending depths')
+    return v, colp, zg
+
+
+_DEPTH_ENTRIES = {('float32', 'float32'): 'impdar_depth_convert_f32', ('float32', 'float64'): 'impdar_depth_convert_f32_f64',
+                  ('float64', 'float64'): 'impdar_depth_convert_f64'}
+
+
+def depth_convert_device(data_dev, travel_time_us, profiles, col_profile, zgrid, out=None):
+    """Depth section (nz, tnum) of a (snum, tnum) float32 or float64 CUDA tensor: out[k, x] = np.interp(zgrid[k], z_p,
+    data[:, x], left=nan, right=nan) with z_p = depth_curves(travel_time_us, profiles)[col_profile[x]] ((P, snum) interval
+    velocities), computed in float64 bit for bit (impdar_depth_convert_*).  `out` (default: the input dtype) may be
+    float64 for float32 input."""
+    import torch
+    if not (device.is_device_array(data_dev) and data_dev.dim() == 2
+            and data_dev.dtype in (torch.float32, torch.float64)):
+        raise ValueError('depth_convert_device needs a 2-D float32 or float64 CUDA tensor')
+    x = data_dev.contiguous()
+    S, T = x.shape
+    if S < 2:
+        raise ValueError('depth conversion needs at least two samples per trace')
+    tt = np.ascontiguousarray(device.host_f64(travel_time_us))
+    if tt.shape != (S,) or not np.all(np.isfinite(tt)) or not np.all(np.diff(tt / 1.0e6) > 0):
+        raise ValueError('travel_time must be %d finite, strictly ascending values' % S)
+    v, colp, zg = _depth_args(profiles, col_profile, S, T, zgrid)
+    nz = zg.size
+    if out is None:
+        out = torch.empty((nz, T), dtype=x.dtype, device=x.device)
+    if not (device.is_device_array(out) and tuple(out.shape) == (nz, T) and out.is_contiguous()):
+        raise ValueError('out must be a contiguous CUDA tensor of shape %s' % ((nz, T),))
+    name = _DEPTH_ENTRIES.get((str(x.dtype).split('.')[-1], str(out.dtype).split('.')[-1]))
+    if name is None:
+        raise ValueError('depth conversion runs float32 -> float32, float32 -> float64 or float64 -> float64, got %s -> %s'
+                         % (x.dtype, out.dtype))
+    lib = _lib.load()
+    ws = device.workspace(lib.impdar_depth_workspace_bytes(S, T, nz, v.shape[0]))
+    rc = getattr(lib, name)(device.ptr(x), device.ptr(out), S, T, nz, device.ptr(tt), device.ptr(v), v.shape[0],
+                            device.ptr(colp), device.ptr(zg), device.ptr(ws), ws.numel(), device.current_stream_ptr())
+    _lib.check(rc)
+    return out
+
+
+def _depth_field(dat, vel, vel_fn, field, genfromtxt_kwargs):
+    """(P, snum) interval profiles and the (tnum,) trace map of depthConvert's velocity argument."""
+    if field is not None:
+        if vel_fn is not None or not (np.ndim(vel) == 0 and vel == 1.69e8):
+            raise ValueError('give the velocity as vel / vel_fn or as field, not both')
+        try:
+            profiles, col_profile = field
+        except (TypeError, ValueError):
+            raise ValueError('field must be a pair (profiles, col_profile)')
+        return _kirch_lateral_args(profiles, col_profile, dat.snum, dat.tnum)
+    if vel_fn is not None:
+        try:
+            vel = np.genfromtxt(vel_fn, **genfromtxt_kwargs)
+            print('Velocities loaded from %s.' % vel_fn)
+        except Exception:
+            raise TypeError('File %s was given for input velocity array, but cannot be loaded. Please reformat to txt file.' % vel_fn)
+    if np.ndim(vel) == 0:
+        profiles = np.full((1, dat.snum), float(vel))
+    elif len(np.shape(vel)) == 2 and np.shape(vel)[1] == 3:
+        profiles, col_profile = lateral_velocity_profiles(dat, np.asarray(vel, dtype=np.float64))
+        return _kirch_lateral_args(profiles, col_profile, dat.snum, dat.tnum)
+    else:
+        profiles = np.asarray(getVelocityProfile(dat, np.asarray(vel, dtype=np.float64)), dtype=np.float64)[None, :]
+    return _kirch_lateral_args(profiles, np.zeros(dat.tnum, dtype=np.int32), dat.snum, dat.tnum)
+
+
+def depthConvert(dat, vel=1.69e8, vel_fn=None, field=None, dz=None, **genfromtxt_kwargs):
+    """Convert a (migrated) time section to depth with a velocity that may vary with depth and laterally.  The velocity
+    is a scalar, a (v, z) table (getVelocityProfile), a (v, z, x) table (lateral_velocity_profiles), a file `vel_fn`
+    loaded like migrationKirchhoffLateral loads one, or field=(profiles, col_profile) of interval velocities
+    (scan_interval_field).  Depth rows are zgrid = z0 + dz * arange(nz), z0 the shallowest first-sample depth of any
+    profile, and the last row the deepest last-sample depth of any profile does not pass; dz defaults to min(v) dt / 2, so no depth row is coarser than the
+    finest sample.  Each trace is resampled with np.interp on its own depth curve (NaN outside it; depth_convert_device).
+    dat.data becomes the (nz, tnum) section (float64 on the host lane, the tensor's dtype on the device lane, integer
+    input widened to float64), dat.snum = nz, dat.nmo_depth = zgrid, and dat.travel_time the two-way time of each depth
+    row in a trace of the most-used profile (the lowest index on ties), continued linearly beyond its first and last
+    samples with its first and last interval velocities."""
+    import torch
+    print('Depth conversion of %.0fx%.0f matrix' % (dat.snum, dat.tnum))
+    _check_data_shape(dat)
+    start = time.time()
+    profiles, col_profile = _depth_field(dat, vel, vel_fn, field, genfromtxt_kwargs)
+    z = depth_curves(dat.travel_time, profiles)
+    if dz is None:
+        dz = float(np.min(profiles)) * float(dat.dt) / 2.
+    dz = float(dz)
+    if not (np.isfinite(dz) and dz > 0):
+        raise ValueError('dz must be finite and positive, got %g' % dz)
+    z0, z1 = float(np.min(z[:, 0])), float(np.max(z[:, -1]))
+    nz = int(np.floor((z1 - z0) / dz)) + 1            # the last row no deeper than the deepest sample
+    while z0 + dz * nz <= z1:
+        nz += 1
+    while nz > 1 and z0 + dz * (nz - 1) > z1:
+        nz -= 1
+    zgrid = z0 + dz * np.arange(nz)
+    on_device = device.is_device_array(dat.data)
+    if on_device:
+        x = dat.data if dat.data.dtype in (torch.float32, torch.float64) else (
+            dat.data.to(torch.float32) if dat.data.is_floating_point() else dat.data.to(torch.float64))
+        out = depth_convert_device(x, dat.travel_time, profiles, col_profile, zgrid)
+        dat.data = out if out.dtype == dat.data.dtype or not dat.data.is_floating_point() else out.to(dat.data.dtype)
+    else:
+        device.require_cuda()
+        a = np.asarray(dat.data)
+        x = device.to_device(a, torch.float32 if a.dtype == np.float32 else torch.float64)
+        out = torch.empty((nz, dat.tnum), dtype=torch.float64, device=x.device)
+        dat.data = device.to_host(depth_convert_device(x, dat.travel_time, profiles, col_profile, zgrid, out=out),
+                                  np.float64)
+    p = int(np.argmax(np.bincount(col_profile, minlength=profiles.shape[0])))
+    tt = np.asarray(dat.travel_time, dtype=np.float64)
+    zp, vp = z[p], profiles[p]
+    newt = np.interp(zgrid, zp, tt)
+    below, above = zgrid > zp[-1], zgrid < zp[0]
+    newt[below] = tt[-1] + 2. * (zgrid[below] - zp[-1]) / vp[-1] * 1.0e6
+    newt[above] = tt[0] - 2. * (zp[0] - zgrid[above]) / vp[0] * 1.0e6
+    dat.travel_time = newt
+    dat.nmo_depth = zgrid
+    dat.snum = nz
+    print('Depth conversion of %.0fx%.0f matrix complete in %.2f seconds' % (nz, dat.tnum, time.time() - start))
+    return dat
 
 
 # -------------------------------------------------------------------------------------- phase shift

@@ -357,6 +357,31 @@ int impdar_interp_cols_f32_f64(const float *x, double *y, int snum, int tnum_in,
 int impdar_interp_cols_f64(const double *x, double *y, int snum, int tnum_in, int tnum_out, const void *nodes,
                            int mode, void *stream);
 
+/* --------------------------------------------------- time-to-depth conversion (depthConvert) --- */
+/* y (nz, tnum) = the (snum, tnum) time section x resampled per trace onto the depth grid zgrid: trace c uses profile
+ * col_profile[c] of `profiles` (nprof x snum interval velocities, m/s) and
+ *   y[k, c] = numpy.interp(zgrid[k], z, x[:, c], left=NaN, right=NaN)
+ * with z that profile's one-way depth curve: t = tt_us / 1e6, j0 = the first sample with t >= 0 (the last sample if none),
+ * z[j0] = v[j0] t[j0] / 2, then the trapezoid (v[i-1] + v[i]) / 2 (t[i] - t[i-1]) / 2 summed left to right above j0 and
+ * subtracted right to left below it (impdar_b200.migrationlib.depth_curves).  float64 throughout, numpy's operation
+ * order, no FMA contraction: bit for bit numpy's result (_f32 rounds it to float32 once).  Suffixes as
+ * impdar_interp_rows_*.  Deterministic.
+ *   tt_us (snum doubles), profiles (nprof x snum doubles), col_profile (tnum ints), zgrid (nz doubles): HOST memory,
+ *   uploaded on `stream` through page-locked staging.
+ * Status 1, before any CUDA call, for a null pointer, snum < 2, tnum < 1, nz < 1, nprof < 1, a velocity that is not
+ * finite and positive, a travel time that is not finite or not strictly ascending, a col_profile outside [0, nprof), a
+ * zgrid that is not finite or not strictly ascending, or a workspace smaller than impdar_depth_workspace_bytes.     */
+size_t impdar_depth_workspace_bytes(int snum, int tnum, int nz, int nprof);
+int impdar_depth_convert_f32(const float *x, float *y, int snum, int tnum, int nz, const double *tt_us,
+                             const double *profiles, int nprof, const int *col_profile, const double *zgrid,
+                             void *workspace, size_t workspace_bytes, void *stream);
+int impdar_depth_convert_f32_f64(const float *x, double *y, int snum, int tnum, int nz, const double *tt_us,
+                                 const double *profiles, int nprof, const int *col_profile, const double *zgrid,
+                                 void *workspace, size_t workspace_bytes, void *stream);
+int impdar_depth_convert_f64(const double *x, double *y, int snum, int tnum, int nz, const double *tt_us,
+                             const double *profiles, int nprof, const int *col_profile, const double *zgrid,
+                             void *workspace, size_t workspace_bytes, void *stream);
+
 /* ------------------------------------------------------- denoise (_RadarDataFiltering.py:552-587) --- */
 /* scipy.signal.wiener(x, mysize=(vert_win, hor_win), noise): float64 box statistics, float64 output y (snum, tnum).
  * estimate_noise != 0: noise = mean of the local variance (scipy's noise=None), `noise` is ignored.
